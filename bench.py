@@ -29,6 +29,12 @@ One bench "step" = MODEL_STEPS consecutive model timesteps of every column of th
   cpu_baseline / --impl reference: the CPU oracle (C port of the Fortran; no Fortran compiler exists in this image),
            one column per OS thread on all host cores, on a bounded sample of the same columns; the libm build (what
            the reference binary links) is the one that is timed, the deterministic-math build is reported beside it.
+
+--dump-outputs DIR (rank 0): after the timed steps, what the end-to-end path handed its caller in its last step --
+the five per-column diagnostics and the 18-number ensemble reduction -- plus N_active and status of every column and
+the layer profiles of a seeded sample of columns, as DIR/<name>.npy (float64; N_active and status float32), about
+55 MB at the default size.  Beyond 1,048,576 columns the per-column files hold a seeded sample, listed in
+columns.npy.  The inputs are seeded, so two builds run with the same arguments can be compared file for file.
 """
 from __future__ import annotations
 
@@ -45,6 +51,7 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True   # the bench writes nothing into the tree, which may be read-only
 
 TOTAL_COLUMNS = 1 << 20
 MODEL_STEPS = 64            # model timesteps per bench step (one launch)
@@ -68,6 +75,12 @@ YEAR_COLUMNS = 151552            # one full wave of the step kernel (148 SMs x 2
 YEAR_DRIFT_STEPS = 8640          # one model day
 YEAR_TIMED_STEPS = 640
 YEAR_REBIN_THRESHOLD = 0.03      # re-bin when more than 3 % of the lane-layers of a launch were idle
+# --dump-outputs: per-column outputs of every column up to DUMP_COLUMNS (a seeded sample beyond), layer profiles of a
+# seeded sample of DUMP_PROFILE_COLUMNS columns; together at most DUMP_MAX_BYTES
+DUMP_COLUMNS = 1 << 20
+DUMP_PROFILE_COLUMNS = 1024
+DUMP_PROFILES = ["m", "S_abs", "H_abs", "thick", "T"]
+DUMP_MAX_BYTES = 64 * 10**6
 
 
 def load_state(rec: int) -> dict:
@@ -278,6 +291,34 @@ def year_weighted(api, sites: np.ndarray, device: int) -> dict:
             "how": "harmonic mean of the regime rates weighted by the regime's share of the golden SHEBA records"}
 
 
+def column_sample(n: int, k: int, seed: int) -> np.ndarray:
+    """All n columns if n <= k, else a fixed seeded sample of k of them, in increasing order."""
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
+
+
+def dump_outputs(out_dir: str, eng, diag_names: list, diag: np.ndarray, red: dict) -> None:
+    """Write the outputs of the last timed step as out_dir/<name>.npy (see the module docstring)."""
+    cols = column_sample(eng.ncol, DUMP_COLUMNS, 0)
+    out = {name: diag[j, cols] for j, name in enumerate(diag_names)}
+    out["ensemble_reduction"] = np.array([[v["sum"], v["min"], v["max"]] for v in red.values()])  # rows in reduce_diag order
+    for name in ("N_active", "status"):
+        out[name] = eng.get_int(name)[cols].astype(np.float32)
+    if len(cols) < eng.ncol:
+        out["columns"] = cols.astype(np.float64)
+    pcols = column_sample(eng.ncol, DUMP_PROFILE_COLUMNS, 1)
+    out["profile_columns"] = pcols.astype(np.float64)
+    for name in DUMP_PROFILES:
+        out[f"profile_{name}"] = np.concatenate([eng.get_array(name, int(c), 1) for c in pcols])
+    nbytes = sum(a.nbytes for a in out.values())
+    assert nbytes <= DUMP_MAX_BYTES, nbytes
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in out.items():
+        np.save(d / f"{name}.npy", a)
+
+
 def main():
     global MODEL_STEPS
     ap = argparse.ArgumentParser()
@@ -292,7 +333,12 @@ def main():
     ap.add_argument("--no-year-weighted", action="store_true", help="skip the six-regime year-weighted block (N = 1 only)")
     ap.add_argument("--two-pass", action="store_true", help="kernel tuning: the two-pass step (samsim_step_kernel<true>) instead of the general path")
     ap.add_argument("--model-steps", type=int, default=MODEL_STEPS, help="model timesteps per bench step (one launch)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
 
     if args.impl == "reference":
         run_reference_arm(args)
@@ -390,6 +436,8 @@ def main():
     assert np.isfinite(diag_host).all() and red["N_active"]["max"] <= 100
     sampler.stop_flag.set()
     sampler.join(timeout=2)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, DIAG, diag_host, red)
 
     # ---- ensemble diagnostics: the only cross-GPU exchange of the model (NCCL all-reduce of 18 numbers) ----
     ensemble = D.reduce_ensemble(eng.reduce_diag(), per, device=torch.device("cuda", local_rank))

@@ -144,11 +144,28 @@ MODULE mo_samsim_b200
        TYPE(C_PTR), VALUE :: set_of_col
      END FUNCTION samsim_b200_set_lab_forcing
 
+     !> real length of each lab set when the sets are padded to one nrec (experiments of different durations)
+     INTEGER(C_INT) FUNCTION samsim_b200_set_lab_lengths(handle, nset, nrec_of_set) &
+          & BIND(C, NAME='samsim_b200_set_lab_lengths')
+       IMPORT :: C_INT, C_INT32_T, C_INT64_T, C_PTR
+       TYPE(C_PTR), VALUE :: handle
+       INTEGER(C_INT32_T), VALUE :: nset
+       INTEGER(C_INT64_T), INTENT(in) :: nrec_of_set(*)
+     END FUNCTION samsim_b200_set_lab_lengths
+
      INTEGER(C_INT) FUNCTION samsim_b200_step(handle, nsteps) BIND(C, NAME='samsim_b200_step')
        IMPORT :: C_INT, C_INT64_T, C_PTR
        TYPE(C_PTR), VALUE :: handle
        INTEGER(C_INT64_T), VALUE :: nsteps
      END FUNCTION samsim_b200_step
+
+     !> last loop index i of columns col0 .. col0+n-1 (0-based); HUGE(0_C_INT64_T) = no end
+     INTEGER(C_INT) FUNCTION samsim_b200_set_end_step(handle, end_i, col0, n) BIND(C, NAME='samsim_b200_set_end_step')
+       IMPORT :: C_INT, C_INT32_T, C_INT64_T, C_PTR
+       TYPE(C_PTR), VALUE :: handle
+       INTEGER(C_INT64_T), INTENT(in) :: end_i(*)
+       INTEGER(C_INT32_T), VALUE :: col0, n
+     END FUNCTION samsim_b200_set_end_step
 
      INTEGER(C_INT) FUNCTION samsim_b200_synchronize(handle) BIND(C, NAME='samsim_b200_synchronize')
        IMPORT :: C_INT, C_PTR

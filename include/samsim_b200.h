@@ -236,12 +236,25 @@ int samsim_b200_update_forcing(samsim_handle_t h, const double* series);
  * set_of_col NULL = set 0.  snow_precip_flag 0 zeroes the snowfall like the reference. */
 int samsim_b200_set_lab_forcing(samsim_handle_t h, int32_t nset, int64_t nrec, const double* series,
                                 const int32_t* set_of_col);
+/* Real length of each lab set when the sets of one table differ in length (experiments of different durations):
+ * the series stay padded to the nrec of samsim_b200_set_lab_forcing, and set s holds nrec_of_set[s] records
+ * (1..nrec).  nset must be that of the last samsim_b200_set_lab_forcing, which resets every length to nrec.
+ * samsim_b200_step checks each set whose columns have not all passed their end step against its own length. */
+int samsim_b200_set_lab_lengths(samsim_handle_t h, int32_t nset, const int64_t* nrec_of_set);
 
 /* ---- the hot path ------------------------------------------------------------------------- */
 /* Advance every column nsteps iterations of mo_grotz.f90:182-835 (S0-S24 except the file I/O of
  * S6/S8; S8's accumulator averaging and reset are done on the device at the reference's cadence).
- * Columns whose status is non-zero are frozen.  Asynchronous on the handle's stream. */
+ * Columns whose status is non-zero are frozen, and so are columns past their end step.  With lab forcing, a
+ * running column whose set would be read past its length makes the call return SAMSIM_ERR_STATE after the steps
+ * that fit.  Asynchronous on the handle's stream. */
 int samsim_b200_step(samsim_handle_t h, int64_t nsteps);
+/* Per-column end step: column col0+q runs loop index i only while i <= end_i[q], so one batch can hold runs of
+ * different lengths (time_total of each testcase, forcing records of each site).  A column past its end is frozen
+ * like a failed one but keeps status 0; it writes no more S8 records, so its snapshot keeps the last record it wrote
+ * (SAMSIM_SNAPSC_TIME says which).  Values must be >= 0 (else SAMSIM_ERR_ARG); INT64_MAX = no end, the default; an
+ * end at or below the current i freezes the column from now on.  Caller's column numbering, like every setter. */
+int samsim_b200_set_end_step(samsim_handle_t h, const int64_t* end_i, int32_t col0, int32_t n);
 int samsim_b200_synchronize(samsim_handle_t h);
 /* Steps from now until (and including) the next step that writes an output record. */
 int64_t samsim_b200_steps_to_next_output(samsim_handle_t h);
@@ -299,8 +312,8 @@ int samsim_b200_get_slot_map(samsim_handle_t h, int32_t* slot_of_col);
 /* ---- checkpoint / restart (SURVEY 8f-4) ------------------------------------------------------
  * The reference can only start from init(testcase) (mo_init.f90:62); a year of 1 M columns wants restarts.
  * save: every state array, scalar and int of every column plus the clock, in the caller's column order.
- * load: into a handle created with the same config and column count (else SAMSIM_ERR_CONFIG); forcing tables are
- * inputs and must be set again.  A restarted run continues bit-identically. */
+ * load: into a handle created with the same config and column count (else SAMSIM_ERR_CONFIG); forcing tables, end
+ * steps and lab lengths are run inputs and must be set again.  A restarted run continues bit-identically. */
 int samsim_b200_save_checkpoint(samsim_handle_t h, const char* path);
 int samsim_b200_load_checkpoint(samsim_handle_t h, const char* path);
 

@@ -59,6 +59,24 @@ typedef struct {
  * formats for column 0.  Returns 0, a negative samsim_b200_err, or the positive reference STOP code of column 0. */
 int samsim_grotz(int32_t testcase, const char* description, const samsim_grotz_options_t* opt);
 
+/* one member of samsim_grotz_batch: a testcase run of its own length with its own dat_*.dat files */
+typedef struct {
+  int32_t testcase;
+  const char* description;
+  const char* output_dir;    /* must exist */
+  int64_t max_steps;         /* 0 = i_time of the testcase */
+} samsim_grotz_member_t;
+
+/* grotz(testcase, description) for n members at once, one column each, e.g. the five lab experiments 101-105 of
+ * different durations.  Every member's testcase must give the same samsim_config_t, except that testcases 101-105
+ * may be mixed (else SAMSIM_ERR_CONFIG, before any device call).  opt supplies device, forcing_dir, lab_input_dir and
+ * quiet; its ncol, output_dir, max_steps and perturbation pointers must be 0 / NULL (else SAMSIM_ERR_ARG).  Member q
+ * reads its own series (101-105: length_input_lab records) and runs min(i_time, max_steps) steps; it writes the
+ * records samsim_grotz(testcase, description) with that max_steps writes, byte for byte except the ncol line of
+ * dat_settings.dat, and stops writing when its status turns non-zero while the others go on.  codes[q] = 0, a
+ * negative samsim_b200_err or the member's STOP code.  Returns 0 or a negative samsim_b200_err. */
+int samsim_grotz_batch(const samsim_grotz_member_t* m, int32_t n, const samsim_grotz_options_t* opt, int32_t* codes);
+
 #ifdef __cplusplus
 }
 #endif

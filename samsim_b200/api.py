@@ -166,7 +166,9 @@ def load_library() -> C.CDLL:
         "samsim_b200_set_forcing": (C.c_int, [H, C.c_int32, C.c_int32, dp, ip, dp, dp]),
         "samsim_b200_update_forcing": (C.c_int, [H, dp]),
         "samsim_b200_set_lab_forcing": (C.c_int, [H, C.c_int32, C.c_int64, dp, ip]),
+        "samsim_b200_set_lab_lengths": (C.c_int, [H, C.c_int32, C.POINTER(C.c_int64)]),
         "samsim_b200_step": (C.c_int, [H, C.c_int64]),
+        "samsim_b200_set_end_step": (C.c_int, [H, C.POINTER(C.c_int64), C.c_int32, C.c_int32]),
         "samsim_b200_synchronize": (C.c_int, [H]),
         "samsim_b200_steps_to_next_output": (C.c_int64, [H]),
         "samsim_b200_set_snapshot_mode": (C.c_int, [H, C.c_int32]),
@@ -203,7 +205,7 @@ EXPORTED_SYMBOLS = [
     "samsim_b200_array_extent", "samsim_b200_set_array", "samsim_b200_get_array", "samsim_b200_set_scalar",
     "samsim_b200_get_scalar", "samsim_b200_set_int", "samsim_b200_get_int", "samsim_b200_broadcast_column",
     "samsim_b200_set_clock", "samsim_b200_get_clock", "samsim_b200_set_forcing", "samsim_b200_update_forcing",
-    "samsim_b200_set_lab_forcing",
+    "samsim_b200_set_lab_forcing", "samsim_b200_set_lab_lengths", "samsim_b200_set_end_step",
     "samsim_b200_step", "samsim_b200_synchronize", "samsim_b200_steps_to_next_output",
     "samsim_b200_set_snapshot_mode", "samsim_b200_get_snapshot", "samsim_b200_get_status",
     "samsim_b200_count_failed", "samsim_b200_reduce_diag", "samsim_b200_launch_count", "samsim_b200_last_step_ms",
@@ -218,6 +220,10 @@ def _dp(a):
 
 def _ip(a):
     return a.ctypes.data_as(C.POINTER(C.c_int32)) if a is not None else None
+
+
+def _lp(a):
+    return a.ctypes.data_as(C.POINTER(C.c_int64)) if a is not None else None
 
 
 def _check(L, rc):
@@ -352,8 +358,9 @@ class Engine:
             else np.ascontiguousarray(series, dtype=np.float64)
         _check(self.L, self.L.samsim_b200_update_forcing(self.h, _dp(s)))
 
-    def set_lab_forcing(self, series, set_of_col=None):
-        """series[nset, 4, nrec] in kind order Tice, snowfall, heat, styropor."""
+    def set_lab_forcing(self, series, set_of_col=None, nrec_of_set=None):
+        """series[nset, 4, nrec] in kind order Tice, snowfall, heat, styropor.  nrec_of_set[nset]: the real length of
+        each set when the sets are padded to a common nrec (None = every set holds nrec records)."""
         s = np.ascontiguousarray(series, dtype=np.float64)
         if s.ndim == 2:
             s = s[None]
@@ -361,6 +368,16 @@ class Engine:
         assert four == 4
         soc = None if set_of_col is None else np.ascontiguousarray(set_of_col, dtype=np.int32)
         _check(self.L, self.L.samsim_b200_set_lab_forcing(self.h, nset, nrec, _dp(s), _ip(soc)))
+        if nrec_of_set is not None:
+            ln = np.ascontiguousarray(nrec_of_set, dtype=np.int64)
+            assert ln.shape == (nset,)
+            _check(self.L, self.L.samsim_b200_set_lab_lengths(self.h, nset, _lp(ln)))
+
+    def set_end_step(self, values, col0: int = 0):
+        """Last loop index i each of the columns col0, col0+1, ... runs; past it the column is frozen with status 0
+        (INT64_MAX = no end, the default)."""
+        v = np.ascontiguousarray(np.atleast_1d(values), dtype=np.int64)
+        _check(self.L, self.L.samsim_b200_set_end_step(self.h, _lp(v), col0, v.shape[0]))
 
     # ---- stepping ---------------------------------------------------------------------------
     def step(self, nsteps: int = 1, sync: bool = True):

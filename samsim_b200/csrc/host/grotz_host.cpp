@@ -8,6 +8,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <string>
 #include <vector>
 
@@ -63,11 +64,134 @@ void row_ES(FILE* f, const double* a, int n) {
   fputc('\n', f);
 }
 
+FILE* open_out(const std::string& dir, const char* name) { return fopen((dir + "/" + name).c_str(), "w"); }
+
+// The dat_*.dat files of one run (output_begin / output_begin_bgc, mo_output.f90:276-339, :354-384) and the record
+// output() writes at S8 (mo_output.f90:116-146, output_bgc :156-188).
 struct OutFiles {
-  FILE *T, *psi_s, *thick, *S_bu, *ray, *psi_l, *freeboard, *snow, *vital, *grav, *T2m, *perm, *flush_v, *flush_h, *psi_g, *melt;
+  FILE *T = nullptr, *psi_s = nullptr, *thick = nullptr, *S_bu = nullptr, *ray = nullptr, *psi_l = nullptr, *freeboard = nullptr,
+       *snow = nullptr, *vital = nullptr, *grav = nullptr, *T2m = nullptr, *perm = nullptr, *flush_v = nullptr, *flush_h = nullptr,
+       *psi_g = nullptr, *melt = nullptr;
+  FILE* bgc[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};
+  int N = 0, N_bgc = 0;
+
+  std::vector<FILE**> all() {
+    return {&T, &psi_s, &thick, &S_bu, &ray, &psi_l, &freeboard, &snow, &vital, &grav, &T2m, &perm, &flush_v, &flush_h, &psi_g, &melt,
+            &bgc[0][0], &bgc[0][1], &bgc[1][0], &bgc[1][1]};
+  }
+  void close() {
+    for (FILE** f : all())
+      if (*f) { fclose(*f); *f = nullptr; }
+  }
+  // the 16 standard files must all open (the reference aborts in OPEN); then dat_settings.dat; then the tracer files
+  int open(const std::string& out, const char* description, int32_t testcase, const samsim_host_case_t& cs, int32_t ncol) {
+    const samsim_config_t& g = cs.cfg;
+    N = g.Nlayer; N_bgc = g.N_bgc;
+    T = open_out(out, "dat_T.dat"); psi_s = open_out(out, "dat_psi_s.dat"); thick = open_out(out, "dat_thick.dat");
+    S_bu = open_out(out, "dat_S_bu.dat"); ray = open_out(out, "dat_ray.dat"); psi_l = open_out(out, "dat_psi_l.dat");
+    freeboard = open_out(out, "dat_freeboard.dat"); snow = open_out(out, "dat_snow.dat");
+    vital = open_out(out, "dat_vital_signs.dat"); grav = open_out(out, "dat_grav_drain.dat");
+    T2m = open_out(out, "dat_T2m_T_top.dat"); perm = open_out(out, "dat_perm.dat"); flush_v = open_out(out, "dat_flush_v.dat");
+    flush_h = open_out(out, "dat_flush_h.dat"); psi_g = open_out(out, "dat_psi_g.dat"); melt = open_out(out, "dat_melt.dat");
+    for (FILE** f : all())
+      if (f < &bgc[0][0] && !*f) return SAMSIM_ERR_STATE;
+    FILE* s = open_out(out, "dat_settings.dat");
+    if (s) {
+      fprintf(s, " ################  Description  ###############\n %s\n #################  Testcase  #################\ntestcase         %8d\n", description ? description : "", testcase);
+      fprintf(s, " ##############  Basic settings  ##############\ndt               %14.3f\nthick_0          %14.3f\ntime_out         %14.3f\ntime_total       %14.3f\n", g.dt, g.thick_0, g.time_out, cs.time_total);
+      fprintf(s, "fl_q_bottom      %14.3f\nT_bottom         %14.3f\nS_bu_bottom      %14.3f\nN_top            %8d\nN_middle         %8d\nN_bottom         %8d\nNlayer           %8d\n",
+              cs.scalars[SAMSIM_SC_FL_Q_BOTTOM], cs.scalars[SAMSIM_SC_T_BOTTOM], cs.scalars[SAMSIM_SC_S_BU_BOTTOM], g.N_top, g.N_middle, g.N_bottom, g.Nlayer);
+      fprintf(s, " ##################  Flags  ###################\nboundflux_flag   %8d\natmoflux_flag    %8d\nalbedo_flag      %8d\ngrav_flag        %8d\nflush_flag       %8d\nflood_flag       %8d\ngrav_heat_flag   %8d\nflush_heat_flag  %8d\nharmonic_flag    %8d\nk_snow_flush     %14.3f\nprescribe_flag   %8d\nsalt_flag        %8d\nturb_flag        %8d\nbottom_flag      %8d\ntank_flag        %8d\nprecip_flag      %8d\n",
+              g.boundflux_flag, g.atmoflux_flag, g.albedo_flag, g.grav_flag, g.flush_flag, g.flood_flag, g.grav_heat_flag, g.flush_heat_flag, g.harmonic_flag, g.k_snow_flush, g.prescribe_flag, g.salt_flag, g.turb_flag, g.bottom_flag, g.tank_flag, g.precip_flag);
+      fprintf(s, " engine           %s\n ncol             %d\n", samsim_b200_version(), ncol);
+      fclose(s);
+    }
+    for (int q = 0; q < N_bgc; q++) {  // dat_bgc0<k>.bu.dat / .br.dat per tracer
+      char name[32];
+      snprintf(name, sizeof name, "dat_bgc0%d.bu.dat", q + 1); bgc[q][0] = open_out(out, name);
+      snprintf(name, sizeof name, "dat_bgc0%d.br.dat", q + 1); bgc[q][1] = open_out(out, name);
+      if (!bgc[q][0] || !bgc[q][1]) return SAMSIM_ERR_STATE;
+    }
+    return SAMSIM_OK;
+  }
+  // one output record from a snapshot: ssc[SAMSIM_SNAPSC_COUNT], A[SAMSIM_SNAPARR_COUNT][N]
+  void write(const double* ssc, const double* A) {
+    row_F(T, A + (size_t)SAMSIM_SNAPARR_T * N, N, 9, 3);
+    row_F(psi_s, A + (size_t)SAMSIM_SNAPARR_PSI_S * N, N, 9, 3);
+    row_F(thick, A + (size_t)SAMSIM_SNAPARR_THICK * N, N, 9, 5);
+    row_F(S_bu, A + (size_t)SAMSIM_SNAPARR_S_BU * N, N, 9, 3);
+    row_F(ray, A + (size_t)SAMSIM_SNAPARR_RAY * N, N - 1, 9, 3);
+    row_F(psi_l, A + (size_t)SAMSIM_SNAPARR_PSI_L * N, N, 9, 3);
+    put_F(freeboard, ssc[SAMSIM_SNAPSC_FREEBOARD], 9, 3); fputc('\n', freeboard);
+    put_F(snow, ssc[SAMSIM_SNAPSC_THICK_SNOW], 9, 3); fputs("  ", snow); put_F(snow, ssc[SAMSIM_SNAPSC_T_SNOW], 9, 3); fputs("  ", snow);
+    put_F(snow, ssc[SAMSIM_SNAPSC_PSI_L_SNOW], 9, 3); fputs("  ", snow); put_F(snow, ssc[SAMSIM_SNAPSC_PSI_S_SNOW], 9, 3); fputc('\n', snow);
+    put_F(vital, ssc[SAMSIM_SNAPSC_ENERGY_STORED], 15, 1);
+    for (int q : {SAMSIM_SNAPSC_FRESHWATER, SAMSIM_SNAPSC_TOTAL_RESIST, SAMSIM_SNAPSC_THICKNESS, SAMSIM_SNAPSC_BULK_SALIN}) { fputs("  ", vital); put_F(vital, ssc[q], 10, 5); }
+    fputc('\n', vital);
+    put_F(grav, ssc[SAMSIM_SNAPSC_GRAV_DRAIN], 9, 6); fputs("  ", grav); put_F(grav, ssc[SAMSIM_SNAPSC_GRAV_SALT], 9, 5); fputs("  ", grav);
+    put_F(grav, ssc[SAMSIM_SNAPSC_GRAV_TEMP], 7, 3); fputc('\n', grav);
+    fprintf(T2m, "  %24.16E  %24.16E\n", ssc[SAMSIM_SNAPSC_T2M], ssc[SAMSIM_SNAPSC_T_TOP]);  // WRITE(45,*): list-directed, 17 digits
+    row_ES(perm, A + (size_t)SAMSIM_SNAPARR_PERM * N, N);
+    row_ES(flush_v, A + (size_t)SAMSIM_SNAPARR_FLUSH_V * N, N);
+    row_ES(flush_h, A + (size_t)SAMSIM_SNAPARR_FLUSH_H * N, N);
+    row_F(psi_g, A + (size_t)SAMSIM_SNAPARR_PSI_G * N, N, 9, 3);
+    for (int q = 0; q < N_bgc; q++) {  // output_bgc, format_bgc = Nlayer x (F16.8,2x)
+      if (bgc[q][0]) row_F(bgc[q][0], A + (size_t)(SAMSIM_SNAPARR_BGC1_BU + 2 * q) * N, N, 16, 8);
+      if (bgc[q][1]) row_F(bgc[q][1], A + (size_t)(SAMSIM_SNAPARR_BGC1_BR + 2 * q) * N, N, 16, 8);
+    }
+    put_ES(melt, ssc[SAMSIM_SNAPSC_MELT_THICK_OUTPUT1]); fputs("  ", melt); put_ES(melt, ssc[SAMSIM_SNAPSC_MELT_THICK_OUTPUT2]); fputs("  ", melt);
+    put_ES(melt, ssc[SAMSIM_SNAPSC_MELT_THICK_OUTPUT3]); fputc('\n', melt);
+  }
 };
 
-FILE* open_out(const std::string& dir, const char* name) { return fopen((dir + "/" + name).c_str(), "w"); }
+// the initial column of one testcase into column `col` of the handle
+int load_case(samsim_handle_t h, const samsim_host_case_t& cs, int32_t col) {
+  int rc = 0;
+  for (int a = 0; a < SAMSIM_ARR_COUNT && !rc; a++)
+    if (samsim_b200_array_extent(h, a) > 0) rc = samsim_b200_set_array(h, a, cs.arrays[a], col, 1);
+  for (int q = 0; q < SAMSIM_SC_COUNT && !rc; q++) rc = samsim_b200_set_scalar(h, q, &cs.scalars[q], col, 1);
+  if (!rc) rc = samsim_b200_set_int(h, SAMSIM_INT_N_ACTIVE, &cs.N_active, col, 1);
+  return rc;
+}
+
+// forcing of atmoflux_flag 2 (mo_grotz.f90:131-135): the four *.txt.input files, 13148 records
+int set_reanalysis_forcing(samsim_handle_t h, const samsim_grotz_options_t* opt) {
+  const int nrec = 13148;
+  std::vector<double> series((size_t)4 * nrec);
+  int rc = samsim_host_read_forcing(opt->forcing_dir, nrec, series.data());
+  if (!rc) rc = samsim_b200_set_forcing(h, 1, nrec, series.data(), nullptr, opt->forcing_scale, opt->forcing_offset);
+  return rc;
+}
+
+// The series a testcase reads in the prologue, in the kind order of samsim_b200_set_lab_forcing ([4][nrec]):
+// 101-105 the four per-second lab series (mo_grotz.f90:138-169), length_input_lab records each; 8 Tinput.txt
+// (mo_grotz.f90:138-143, one value per minute) and 111 Ts_<int(dt)>s.txt (mo_grotz.f90:171-176, one value per step)
+// as Tice, as many records as the file holds.  nrec = 0: the testcase reads no series.
+int read_case_series(const samsim_host_case_t& cs, int32_t testcase, const samsim_grotz_options_t* opt, std::vector<double>& lab,
+                     int64_t& nrec) {
+  nrec = 0;
+  lab.clear();
+  if (testcase == 8 || testcase == 111) {
+    std::vector<double> T;
+    char ts_name[64];
+    snprintf(ts_name, sizeof ts_name, "/Ts_%ds.txt", (int)cs.cfg.dt);
+    const std::string path = std::string(opt->lab_input_dir ? opt->lab_input_dir : "2017_input") + (testcase == 8 ? "/Tinput.txt" : ts_name);
+    FILE* f = fopen(path.c_str(), "r");
+    if (!f) return SAMSIM_ERR_STATE;
+    double x;
+    while (fscanf(f, " %lf", &x) == 1) T.push_back(x);
+    fclose(f);
+    if (T.empty()) return SAMSIM_ERR_STATE;
+    nrec = (int64_t)T.size();
+    lab.assign(4 * T.size(), 0.0);
+    for (size_t r = 0; r < T.size(); r++) lab[r] = T[r];
+  } else if (testcase >= 101 && testcase <= 105) {
+    nrec = cs.length_input_lab;
+    lab.resize((size_t)4 * (size_t)nrec);
+    return samsim_host_read_lab_series(opt->lab_input_dir, testcase, nrec, lab.data());
+  }
+  return SAMSIM_OK;
+}
 
 }  // namespace
 
@@ -348,99 +472,34 @@ int samsim_grotz(int32_t testcase, const char* description, const samsim_grotz_o
   if (rc) return rc;
   const samsim_config_t& g = cs.cfg;
   const int N = g.Nlayer;
-  const std::string out = opt->output_dir;
 
   // ---- output_begin / output_settings (mo_output.f90:276-339, :41-106) ----
   OutFiles F;
-  F.T = open_out(out, "dat_T.dat"); F.psi_s = open_out(out, "dat_psi_s.dat"); F.thick = open_out(out, "dat_thick.dat");
-  F.S_bu = open_out(out, "dat_S_bu.dat"); F.ray = open_out(out, "dat_ray.dat"); F.psi_l = open_out(out, "dat_psi_l.dat");
-  F.freeboard = open_out(out, "dat_freeboard.dat"); F.snow = open_out(out, "dat_snow.dat");
-  F.vital = open_out(out, "dat_vital_signs.dat"); F.grav = open_out(out, "dat_grav_drain.dat");
-  F.T2m = open_out(out, "dat_T2m_T_top.dat"); F.perm = open_out(out, "dat_perm.dat"); F.flush_v = open_out(out, "dat_flush_v.dat");
-  F.flush_h = open_out(out, "dat_flush_h.dat"); F.psi_g = open_out(out, "dat_psi_g.dat"); F.melt = open_out(out, "dat_melt.dat");
-  FILE* Fbgc[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};
   samsim_handle_t h = nullptr;
-  auto all_files = [&]() {
-    return std::vector<FILE**>{&F.T, &F.psi_s, &F.thick, &F.S_bu, &F.ray, &F.psi_l, &F.freeboard, &F.snow, &F.vital, &F.grav, &F.T2m,
-                               &F.perm, &F.flush_v, &F.flush_h, &F.psi_g, &F.melt, &Fbgc[0][0], &Fbgc[0][1], &Fbgc[1][0], &Fbgc[1][1]};
-  };
   auto finish = [&](int code) {  // every exit path: close the files, release the device and the host case
-    for (FILE** f : all_files())
-      if (*f) { fclose(*f); *f = nullptr; }
+    F.close();
     if (h) samsim_b200_destroy(h);
     samsim_host_case_free(&cs);
     return code;
   };
-  for (FILE** f : all_files())
-    if (f < &Fbgc[0][0] || f > &Fbgc[1][1])  // the 16 standard files must all be open (the reference aborts in OPEN)
-      if (!*f) return finish(SAMSIM_ERR_STATE);
-  {
-    FILE* s = open_out(out, "dat_settings.dat");
-    if (s) {
-      fprintf(s, " ################  Description  ###############\n %s\n #################  Testcase  #################\ntestcase         %8d\n", description ? description : "", testcase);
-      fprintf(s, " ##############  Basic settings  ##############\ndt               %14.3f\nthick_0          %14.3f\ntime_out         %14.3f\ntime_total       %14.3f\n", g.dt, g.thick_0, g.time_out, cs.time_total);
-      fprintf(s, "fl_q_bottom      %14.3f\nT_bottom         %14.3f\nS_bu_bottom      %14.3f\nN_top            %8d\nN_middle         %8d\nN_bottom         %8d\nNlayer           %8d\n",
-              cs.scalars[SAMSIM_SC_FL_Q_BOTTOM], cs.scalars[SAMSIM_SC_T_BOTTOM], cs.scalars[SAMSIM_SC_S_BU_BOTTOM], g.N_top, g.N_middle, g.N_bottom, g.Nlayer);
-      fprintf(s, " ##################  Flags  ###################\nboundflux_flag   %8d\natmoflux_flag    %8d\nalbedo_flag      %8d\ngrav_flag        %8d\nflush_flag       %8d\nflood_flag       %8d\ngrav_heat_flag   %8d\nflush_heat_flag  %8d\nharmonic_flag    %8d\nk_snow_flush     %14.3f\nprescribe_flag   %8d\nsalt_flag        %8d\nturb_flag        %8d\nbottom_flag      %8d\ntank_flag        %8d\nprecip_flag      %8d\n",
-              g.boundflux_flag, g.atmoflux_flag, g.albedo_flag, g.grav_flag, g.flush_flag, g.flood_flag, g.grav_heat_flag, g.flush_heat_flag, g.harmonic_flag, g.k_snow_flush, g.prescribe_flag, g.salt_flag, g.turb_flag, g.bottom_flag, g.tank_flag, g.precip_flag);
-      fprintf(s, " engine           %s\n ncol             %d\n", samsim_b200_version(), opt->ncol);
-      fclose(s);
-    }
-  }
-
-  // output_begin_bgc (mo_output.f90:354-384): dat_bgc0<k>.bu.dat / .br.dat per tracer
-  for (int q = 0; q < g.N_bgc; q++) {
-    char name[32];
-    snprintf(name, sizeof name, "dat_bgc0%d.bu.dat", q + 1); Fbgc[q][0] = open_out(out, name);
-    snprintf(name, sizeof name, "dat_bgc0%d.br.dat", q + 1); Fbgc[q][1] = open_out(out, name);
-    if (!Fbgc[q][0] || !Fbgc[q][1]) return finish(SAMSIM_ERR_STATE);
-  }
+  if ((rc = F.open(opt->output_dir, description, testcase, cs, opt->ncol))) return finish(rc);
 
   // ---- device ----
   rc = samsim_b200_create(&g, opt->ncol, opt->device, &h);
   if (rc) return finish(rc);
-  for (int a = 0; a < SAMSIM_ARR_COUNT && !rc; a++)
-    if (samsim_b200_array_extent(h, a) > 0) rc = samsim_b200_set_array(h, a, cs.arrays[a], 0, 1);
-  for (int q = 0; q < SAMSIM_SC_COUNT && !rc; q++) rc = samsim_b200_set_scalar(h, q, &cs.scalars[q], 0, 1);
-  if (!rc) rc = samsim_b200_set_int(h, SAMSIM_INT_N_ACTIVE, &cs.N_active, 0, 1);
+  rc = load_case(h, cs, 0);
   if (!rc) rc = samsim_b200_set_clock(h, 0.0, 0, 0, 1);
   if (!rc && opt->ncol > 1) rc = samsim_b200_broadcast_column(h, 0, 0, opt->ncol);
   if (!rc && opt->ttop_warm) rc = samsim_b200_set_scalar(h, SAMSIM_SC_TTOP_WARM, opt->ttop_warm, 0, opt->ncol);
   if (!rc && opt->ttop_warm) rc = samsim_b200_set_scalar(h, SAMSIM_SC_T_TOP, opt->ttop_warm, 0, opt->ncol);  // T_top starts at the warm level (mo_init.f90:894)
   if (!rc && opt->ttop_cold) rc = samsim_b200_set_scalar(h, SAMSIM_SC_TTOP_COLD, opt->ttop_cold, 0, opt->ncol);
   if (!rc && opt->oflux_amp) rc = samsim_b200_set_scalar(h, SAMSIM_SC_OFLUX_AMP, opt->oflux_amp, 0, opt->ncol);
-  if (!rc && g.atmoflux_flag == 2) {  // mo_grotz.f90:131-135
-    const int nrec = 13148;
-    std::vector<double> series((size_t)4 * nrec);
-    rc = samsim_host_read_forcing(opt->forcing_dir, nrec, series.data());
-    if (!rc) rc = samsim_b200_set_forcing(h, 1, nrec, series.data(), nullptr, opt->forcing_scale, opt->forcing_offset);
-  }
-  if (!rc && (testcase == 8 || testcase == 111)) {
-    // 8: mo_grotz.f90:138-143 reads Tinput; the field series is Tinput.txt, one value per minute.
-    // 111: mo_grotz.f90:171-176 reads Ts_<int(dt)>s.txt, one value per time step.
-    std::vector<double> T;
-    char ts_name[64];
-    snprintf(ts_name, sizeof ts_name, "/Ts_%ds.txt", (int)g.dt);
-    const std::string path = std::string(opt->lab_input_dir ? opt->lab_input_dir : "2017_input") + (testcase == 8 ? "/Tinput.txt" : ts_name);
-    FILE* f = fopen(path.c_str(), "r");
-    if (!f) rc = SAMSIM_ERR_STATE;
-    else {
-      double x;
-      while (fscanf(f, " %lf", &x) == 1) T.push_back(x);
-      fclose(f);
-      if (T.empty()) rc = SAMSIM_ERR_STATE;
-    }
-    if (!rc) {
-      std::vector<double> lab(4 * T.size(), 0.0);
-      for (size_t r = 0; r < T.size(); r++) lab[r] = T[r];
-      rc = samsim_b200_set_lab_forcing(h, 1, (int64_t)T.size(), lab.data(), nullptr);
-    }
-  }
-  if (!rc && testcase >= 101 && testcase <= 105) {  // mo_grotz.f90:138-169: the four per-second lab series
-    const int64_t nrec = cs.length_input_lab;
-    std::vector<double> lab((size_t)4 * (size_t)nrec);
-    rc = samsim_host_read_lab_series(opt->lab_input_dir, testcase, nrec, lab.data());
-    if (!rc) rc = samsim_b200_set_lab_forcing(h, 1, nrec, lab.data(), nullptr);
+  if (!rc && g.atmoflux_flag == 2) rc = set_reanalysis_forcing(h, opt);
+  {
+    std::vector<double> lab;
+    int64_t nrec = 0;
+    if (!rc) rc = read_case_series(cs, testcase, opt, lab, nrec);
+    if (!rc && nrec > 0) rc = samsim_b200_set_lab_forcing(h, 1, nrec, lab.data(), nullptr);
   }
   if (!rc) rc = samsim_b200_set_snapshot_mode(h, SAMSIM_SNAP_FULL);
 
@@ -462,38 +521,112 @@ int samsim_grotz(int32_t testcase, const char* description, const samsim_grotz_o
     if (wrote) {  // S8: CALL output(...) (mo_output.f90:116-146) with the values the device captured there
       rc = samsim_b200_get_snapshot(h, ssc.data(), sar.data(), 0, 1);
       if (rc) break;
-      const double* A = sar.data();
-      row_F(F.T, A + (size_t)SAMSIM_SNAPARR_T * N, N, 9, 3);
-      row_F(F.psi_s, A + (size_t)SAMSIM_SNAPARR_PSI_S * N, N, 9, 3);
-      row_F(F.thick, A + (size_t)SAMSIM_SNAPARR_THICK * N, N, 9, 5);
-      row_F(F.S_bu, A + (size_t)SAMSIM_SNAPARR_S_BU * N, N, 9, 3);
-      row_F(F.ray, A + (size_t)SAMSIM_SNAPARR_RAY * N, N - 1, 9, 3);
-      row_F(F.psi_l, A + (size_t)SAMSIM_SNAPARR_PSI_L * N, N, 9, 3);
-      put_F(F.freeboard, ssc[SAMSIM_SNAPSC_FREEBOARD], 9, 3); fputc('\n', F.freeboard);
-      put_F(F.snow, ssc[SAMSIM_SNAPSC_THICK_SNOW], 9, 3); fputs("  ", F.snow); put_F(F.snow, ssc[SAMSIM_SNAPSC_T_SNOW], 9, 3); fputs("  ", F.snow);
-      put_F(F.snow, ssc[SAMSIM_SNAPSC_PSI_L_SNOW], 9, 3); fputs("  ", F.snow); put_F(F.snow, ssc[SAMSIM_SNAPSC_PSI_S_SNOW], 9, 3); fputc('\n', F.snow);
-      put_F(F.vital, ssc[SAMSIM_SNAPSC_ENERGY_STORED], 15, 1);
-      for (int q : {SAMSIM_SNAPSC_FRESHWATER, SAMSIM_SNAPSC_TOTAL_RESIST, SAMSIM_SNAPSC_THICKNESS, SAMSIM_SNAPSC_BULK_SALIN}) { fputs("  ", F.vital); put_F(F.vital, ssc[q], 10, 5); }
-      fputc('\n', F.vital);
-      put_F(F.grav, ssc[SAMSIM_SNAPSC_GRAV_DRAIN], 9, 6); fputs("  ", F.grav); put_F(F.grav, ssc[SAMSIM_SNAPSC_GRAV_SALT], 9, 5); fputs("  ", F.grav);
-      put_F(F.grav, ssc[SAMSIM_SNAPSC_GRAV_TEMP], 7, 3); fputc('\n', F.grav);
-      fprintf(F.T2m, "  %24.16E  %24.16E\n", ssc[SAMSIM_SNAPSC_T2M], ssc[SAMSIM_SNAPSC_T_TOP]);  // WRITE(45,*): list-directed, 17 digits
-      row_ES(F.perm, A + (size_t)SAMSIM_SNAPARR_PERM * N, N);
-      row_ES(F.flush_v, A + (size_t)SAMSIM_SNAPARR_FLUSH_V * N, N);
-      row_ES(F.flush_h, A + (size_t)SAMSIM_SNAPARR_FLUSH_H * N, N);
-      row_F(F.psi_g, A + (size_t)SAMSIM_SNAPARR_PSI_G * N, N, 9, 3);
-      for (int q = 0; q < g.N_bgc; q++) {  // output_bgc, format_bgc = Nlayer x (F16.8,2x)
-        if (Fbgc[q][0]) row_F(Fbgc[q][0], A + (size_t)(SAMSIM_SNAPARR_BGC1_BU + 2 * q) * N, N, 16, 8);
-        if (Fbgc[q][1]) row_F(Fbgc[q][1], A + (size_t)(SAMSIM_SNAPARR_BGC1_BR + 2 * q) * N, N, 16, 8);
-      }
-      put_ES(F.melt, ssc[SAMSIM_SNAPSC_MELT_THICK_OUTPUT1]); fputs("  ", F.melt); put_ES(F.melt, ssc[SAMSIM_SNAPSC_MELT_THICK_OUTPUT2]); fputs("  ", F.melt);
-      put_ES(F.melt, ssc[SAMSIM_SNAPSC_MELT_THICK_OUTPUT3]); fputc('\n', F.melt);
+      F.write(ssc.data(), sar.data());
       if (!opt->quiet)
         printf("progress: %3d%%,  thickness: %6.3f m,  surface T: %7.3f C,  T2m: %7.3f\n", (int)(100.0 * ssc[SAMSIM_SNAPSC_TIME] / cs.time_total),
                ssc[SAMSIM_SNAPSC_THICKNESS], ssc[SAMSIM_SNAPSC_T_TOP], ssc[SAMSIM_SNAPSC_T2M]);
     }
   }
   return finish(rc ? rc : status);  // 0, a negative samsim_b200_err, or the reference STOP code of column 0
+}
+
+int samsim_grotz_batch(const samsim_grotz_member_t* m, int32_t n, const samsim_grotz_options_t* opt, int32_t* codes) {
+  if (!m || n < 1 || !opt || !codes) return SAMSIM_ERR_ARG;
+  if (opt->ncol != 0 || opt->output_dir || opt->max_steps != 0 || opt->forcing_scale || opt->forcing_offset || opt->ttop_warm ||
+      opt->ttop_cold || opt->oflux_amp)
+    return SAMSIM_ERR_ARG;  // these belong to a member or to samsim_grotz's identical columns
+  for (int32_t q = 0; q < n; q++)
+    if (!m[q].output_dir || m[q].max_steps < 0) return SAMSIM_ERR_ARG;
+  std::vector<samsim_host_case_t> cs((size_t)n);
+  std::vector<OutFiles> F((size_t)n);
+  int32_t ninit = 0;
+  samsim_handle_t h = nullptr;
+  auto finish = [&](int code) {  // every exit path: close the files, release the device and the host cases
+    for (OutFiles& f : F) f.close();
+    if (h) samsim_b200_destroy(h);
+    for (int32_t q = 0; q < ninit; q++) samsim_host_case_free(&cs[q]);
+    return code;
+  };
+  // ---- init(testcase) of every member; one run-wide configuration, checked before any device call ----
+  int rc = 0;
+  for (; ninit < n; ninit++)
+    if ((rc = samsim_host_init_testcase(m[ninit].testcase, &cs[ninit]))) return finish(rc);
+  const samsim_config_t& g = cs[0].cfg;
+  auto lab = [](int32_t tc) { return tc >= 101 && tc <= 105; };
+  for (int32_t q = 1; q < n; q++) {
+    samsim_config_t c = cs[q].cfg;
+    if (lab(c.testcase) && lab(g.testcase)) c.testcase = g.testcase;  // the five lab experiments take one device path
+    if (memcmp(&c, &g, sizeof c) != 0) return finish(SAMSIM_ERR_CONFIG);
+  }
+  const int N = g.Nlayer;
+  for (int32_t q = 0; q < n && !rc; q++) rc = F[q].open(m[q].output_dir, m[q].description, m[q].testcase, cs[q], n);
+  if (rc) return finish(rc);
+
+  // ---- device: member q is column q and reads lab set q ----
+  if ((rc = samsim_b200_create(&g, n, opt->device, &h))) return finish(rc);
+  for (int32_t q = 0; q < n && !rc; q++) rc = load_case(h, cs[q], q);
+  if (!rc) rc = samsim_b200_set_clock(h, 0.0, 0, 0, 1);
+  if (!rc && g.atmoflux_flag == 2) rc = set_reanalysis_forcing(h, opt);
+  {
+    std::vector<std::vector<double>> series((size_t)n);
+    std::vector<int64_t> len((size_t)n, 0);
+    int64_t nrec = 0;
+    for (int32_t q = 0; q < n && !rc; q++) {
+      rc = read_case_series(cs[q], m[q].testcase, opt, series[q], len[q]);
+      nrec = std::max(nrec, len[q]);
+    }
+    if (!rc && nrec > 0) {  // one table padded to the longest series; each set keeps its own length
+      std::vector<double> table((size_t)n * 4 * (size_t)nrec, 0.0);
+      std::vector<int32_t> set_of_col((size_t)n);
+      for (int32_t q = 0; q < n; q++) {
+        set_of_col[q] = q;
+        for (int kind = 0; kind < 4; kind++)
+          std::copy(series[q].begin() + (size_t)kind * len[q], series[q].begin() + (size_t)(kind + 1) * len[q],
+                    table.begin() + ((size_t)q * 4 + kind) * (size_t)nrec);
+      }
+      rc = samsim_b200_set_lab_forcing(h, n, nrec, table.data(), set_of_col.data());
+      if (!rc) rc = samsim_b200_set_lab_lengths(h, n, len.data());
+    }
+  }
+  std::vector<int64_t> end((size_t)n);
+  int64_t total = 0;
+  for (int32_t q = 0; q < n; q++) {
+    end[q] = (m[q].max_steps > 0 && m[q].max_steps < cs[q].i_time) ? m[q].max_steps : cs[q].i_time;
+    total = std::max(total, end[q]);
+  }
+  if (!rc) rc = samsim_b200_set_end_step(h, end.data(), 0, n);
+  if (!rc) rc = samsim_b200_set_snapshot_mode(h, SAMSIM_SNAP_FULL);
+
+  // ---- the time loop of samsim_grotz up to the latest end; a member writes while it runs and its status is 0 ----
+  int64_t done = 0;
+  std::vector<double> ssc((size_t)n * SAMSIM_SNAPSC_COUNT), sar((size_t)n * SAMSIM_SNAPARR_COUNT * N);
+  std::vector<int32_t> status((size_t)n, 0);
+  while (!rc && done < total) {
+    int64_t k = samsim_b200_steps_to_next_output(h);
+    if (k <= 0) { rc = SAMSIM_ERR_STATE; break; }
+    const bool wrote = (done + k <= total);
+    if (k > total - done) k = total - done;
+    if ((rc = samsim_b200_step(h, k))) break;
+    done += k;
+    if ((rc = samsim_b200_get_status(h, status.data(), 0, n))) break;
+    bool running = false;
+    for (int32_t q = 0; q < n; q++) running = running || (status[q] == 0 && done < end[q]);
+    if (wrote) {
+      if ((rc = samsim_b200_get_snapshot(h, ssc.data(), sar.data(), 0, n))) break;
+      for (int32_t q = 0; q < n; q++) {
+        if (status[q] != 0 || done > end[q]) continue;
+        const double* sc = ssc.data() + (size_t)q * SAMSIM_SNAPSC_COUNT;
+        F[q].write(sc, sar.data() + (size_t)q * SAMSIM_SNAPARR_COUNT * N);
+        if (!opt->quiet)
+          printf("member %d progress: %3d%%,  thickness: %6.3f m,  surface T: %7.3f C,  T2m: %7.3f\n", q,
+                 (int)(100.0 * sc[SAMSIM_SNAPSC_TIME] / cs[q].time_total), sc[SAMSIM_SNAPSC_THICKNESS], sc[SAMSIM_SNAPSC_T_TOP],
+                 sc[SAMSIM_SNAPSC_T2M]);
+      }
+    }
+    if (!running) break;  // every member has failed or reached its end
+  }
+  for (int32_t q = 0; q < n; q++) codes[q] = rc ? rc : status[q];
+  return finish(rc);
 }
 
 }  // extern "C"

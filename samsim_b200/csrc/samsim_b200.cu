@@ -8,6 +8,7 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <algorithm>
 #include <string>
 #include <vector>
 
@@ -61,6 +62,8 @@ struct KParams {
   const double* lab;      // [nset][4][lab_nrec]
   long long lab_nrec;
   const int* set_of_col;
+  // last loop index each column runs (samsim_b200_set_end_step), [ncol_pad] in slot order; nullptr = no column ends
+  const int64_t* end_of_col;
   // snapshot
   double* snap_sc;
   double* snap_arr;
@@ -68,6 +71,10 @@ struct KParams {
   // lanes disagree on the snow class or the status, [3] warps
   unsigned long long* divergence;
 };
+
+// status of a column that has passed its end step, inside the step kernel only (padding columns hold -1, failed
+// ones the reference's positive STOP code); never written back
+#define STATUS_FINISHED (-2)
 
 __device__ __forceinline__ void cp_async8(void* smem_dst, const void* gmem_src) {
   unsigned s = (unsigned)__cvta_generic_to_shared(smem_dst);
@@ -127,8 +134,20 @@ __global__ void __launch_bounds__(SAMSIM_BLOCK, SAMSIM_MINBLOCKS) samsim_step_ke
   SnapOut snap;
   snap.scalars = p.snap_sc; snap.arrays = p.snap_arr; snap.ncol_pad = ls; snap.col = (int)col;
 
-  // every thread runs every step: a failed column only skips the phase bodies (column_step checks c.status)
-  for (int s = 0; s < p.nsteps; s++) column_step<TWO_PASS>(c, f, s == p.nsteps - 1, snap);
+  // A column runs loop index i only while i <= its end step.  From then on it is frozen like a failed column: its
+  // status holds STATUS_FINISHED for the rest of the launch and 0 again on write-back.
+  int my_steps = p.nsteps;
+  if (p.end_of_col) {
+    const long long left = p.end_of_col[col] - p.i;
+    my_steps = (left <= 0) ? 0 : (left < p.nsteps) ? (int)left : p.nsteps;
+  }
+  // every thread runs every step: a failed or finished column only skips the phase bodies (column_step checks
+  // c.status).  A column's last step materialises what a launch otherwise only writes at its end (S_bu, ray, fl_Q, the
+  // S0 diagnostics); want_diag at any step leaves the results unchanged, as launches of arbitrary lengths show.
+  for (int s = 0; s < p.nsteps; s++) {
+    if (s == my_steps && c.status == 0) c.status = STATUS_FINISHED;
+    column_step<TWO_PASS>(c, f, s == p.nsteps - 1 || s == my_steps - 1, snap);
+  }
 
   // ---- lane divergence of this launch's end state, measured where it arises: in the warp --------------------------
   // A warp runs every layer sweep to the deepest of its 32 columns and every branch that one of its lanes takes.
@@ -162,7 +181,7 @@ __global__ void __launch_bounds__(SAMSIM_BLOCK, SAMSIM_MINBLOCKS) samsim_step_ke
   if (padding) return;
   for (int q = 0; q < SC_COUNT; q++) p.sc[(size_t)q * ls + col] = c.sc[q];
   p.in[(size_t)IN_N_ACTIVE * ls + col] = c.N_active;
-  p.in[(size_t)IN_STATUS * ls + col] = c.status;
+  p.in[(size_t)IN_STATUS * ls + col] = (c.status == STATUS_FINISHED) ? 0 : c.status;
   p.in[(size_t)IN_STYROPOR * ls + col] = c.styropor_flag;
   p.in[(size_t)IN_EVENTS0 * ls + col] = (int)c.ev0;
   p.in[(size_t)IN_EVENTS1 * ls + col] = (int)c.ev1;
@@ -249,14 +268,16 @@ __global__ void samsim_vec_set_kernel(T* row, const T* src, int col0, int n, con
 }
 
 // ---- re-binning (SURVEY 8e: columns are re-binned by regime for warp coherence; local permutation only) ----
-// key: failed columns last; then N_active descending (loop trip counts), snow class (the snow branches) and melting
+// key: failed and finished columns last; then N_active descending (loop trip counts), snow class (the snow branches) and melting
 // surface (flushing, full S4 sweep), forcing site, surface temperature
-__global__ void samsim_rebin_key_kernel(const double* sc, const int* in, const int* site_of_col, long long ncol,
-                                        long long ncol_pad, double thick_min, unsigned* keys, int* vals) {
+__global__ void samsim_rebin_key_kernel(const double* sc, const int* in, const int* site_of_col, const int64_t* end_of_col,
+                                        long long i, long long ncol, long long ncol_pad, double thick_min, unsigned* keys,
+                                        int* vals) {
   const long long s = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (s >= ncol) return;
   const int na = in[(size_t)IN_N_ACTIVE * ncol_pad + s];
-  const int st = in[(size_t)IN_STATUS * ncol_pad + s];
+  // a finished column idles like a failed one: their warps should hold no running column
+  const bool idle = in[(size_t)IN_STATUS * ncol_pad + s] != 0 || (end_of_col && end_of_col[s] <= i);
   const double snow = sc[(size_t)SC_THICK_SNOW * ncol_pad + s];
   const unsigned cls = ((snow <= 0.0) ? 0u : (snow < thick_min / 100.0) ? 1u : (snow < thick_min) ? 2u : 3u) |
                        ((sc[(size_t)SC_MELT_THICK * ncol_pad + s] > 0.0) ? 4u : 0u);  // melting surface: the flushing / full-S4 path
@@ -266,7 +287,7 @@ __global__ void samsim_rebin_key_kernel(const double* sc, const int* in, const i
   // their Newton sweeps take the same number of iterations and their drainage candidates span the same layers
   const double tt = sc[(size_t)SC_T_TOP * ncol_pad + s];
   const unsigned tb = (tt > -80.0) ? ((tt < 22.3) ? (unsigned)((tt + 80.0) * 10.0) : 1023u) : 0u;  // NaN -> 0
-  keys[s] = ((st != 0) ? 0x80000000u : 0u) | ((0xFFFu - ((unsigned)na & 0xFFFu)) << 19) | (cls << 15) | ((site & 0x1Fu) << 10) | tb;
+  keys[s] = (idle ? 0x80000000u : 0u) | ((0xFFFu - ((unsigned)na & 0xFFFu)) << 19) | (cls << 15) | ((site & 0x1Fu) << 10) | tb;
   vals[s] = (int)s;
 }
 __global__ void samsim_rebin_unsorted_kernel(const unsigned* keys, long long ncol, int* out) {
@@ -413,6 +434,14 @@ struct samsim_b200_handle_s {
   double* lab = nullptr;
   long long lab_nrec = 0;
   int* set_of_col = nullptr;
+  // lab sets: the real length of each set (samsim_b200_set_lab_lengths, else lab_nrec), the set of every column in
+  // caller order (empty = all in set 0) and the latest end step of each set's columns (INT64_MIN: the set has none)
+  std::vector<int64_t> lab_len, lab_end;
+  std::vector<int32_t> set_host;
+  // per-column end steps (samsim_b200_set_end_step): device row in slot order (nullptr until the first call) and the
+  // host copy in caller order
+  int64_t* end_of_col = nullptr;
+  std::vector<int64_t> end_host;
   // snapshot
   int snap_mode = SAMSIM_SNAP_NONE;
   double *snap_sc = nullptr, *snap_arr = nullptr;
@@ -620,7 +649,7 @@ void samsim_b200_destroy(samsim_handle_t h) {
   if (h->divergence_host) cudaFreeHost(h->divergence_host);
   cudaFree(h->arr); cudaFree(h->sc); cudaFree(h->in); cudaFree(h->series); cudaFree(h->site_of_col);
   cudaFree(h->fscale); cudaFree(h->foffset); cudaFree(h->lab); cudaFree(h->set_of_col); cudaFree(h->snap_sc);
-  cudaFree(h->snap_arr); cudaFree(h->stage); cudaFree(h->slot_of_col); cudaFree(h->col_of_slot);
+  cudaFree(h->snap_arr); cudaFree(h->stage); cudaFree(h->slot_of_col); cudaFree(h->col_of_slot); cudaFree(h->end_of_col);
   if (h->ev0) cudaEventDestroy(h->ev0);
   if (h->ev1) cudaEventDestroy(h->ev1);
   if (h->stream) cudaStreamDestroy(h->stream);
@@ -778,6 +807,16 @@ int samsim_b200_update_forcing(samsim_handle_t h, const double* series) {
   return 0;
 }
 
+// latest end step of the columns of each lab set: only the sets of running columns bound a launch (samsim_b200_step)
+static void update_lab_end(samsim_handle_t h) {
+  h->lab_end.assign(h->lab_len.size(), INT64_MIN);
+  if (h->lab_end.empty()) return;
+  for (long long c = 0; c < h->ncol; c++) {
+    int64_t& e = h->lab_end[h->set_host.empty() ? 0 : h->set_host[c]];
+    e = std::max(e, h->end_host.empty() ? INT64_MAX : h->end_host[c]);
+  }
+}
+
 int samsim_b200_set_lab_forcing(samsim_handle_t h, int32_t nset, int64_t nrec, const double* series, const int32_t* set_of_col) {
   if (!h || !series || nset < 1 || nrec < 1) return fail(SAMSIM_ERR_ARG, "set_lab_forcing: bad argument");
   if (set_of_col)
@@ -794,6 +833,10 @@ int samsim_b200_set_lab_forcing(samsim_handle_t h, int32_t nset, int64_t nrec, c
     for (int s = 0; s < nset; s++) CU(cudaMemset(h->lab + ((size_t)s * 4 + 1) * nrec, 0, (size_t)nrec * sizeof(double)));
   }
   h->lab_nrec = nrec;
+  h->lab_len.assign((size_t)nset, nrec);
+  if (set_of_col) h->set_host.assign(set_of_col, set_of_col + h->ncol);
+  else h->set_host.clear();
+  update_lab_end(h);
   if (set_of_col) {
     CU(cudaMalloc(&h->set_of_col, (size_t)h->ncol_pad * sizeof(int)));
     CU(cudaMemset(h->set_of_col, 0, (size_t)h->ncol_pad * sizeof(int)));
@@ -801,6 +844,36 @@ int samsim_b200_set_lab_forcing(samsim_handle_t h, int32_t nset, int64_t nrec, c
     int rc = to_slot_order<int>(h, h->set_of_col, 1);
     if (rc) return rc;
   }
+  return 0;
+}
+
+int samsim_b200_set_lab_lengths(samsim_handle_t h, int32_t nset, const int64_t* nrec_of_set) {
+  if (!h || !nrec_of_set) return fail(SAMSIM_ERR_ARG, "set_lab_lengths: bad argument");
+  if (!h->lab) return fail(SAMSIM_ERR_STATE, "set_lab_lengths: call samsim_b200_set_lab_forcing first");
+  if (nset != (int32_t)h->lab_len.size()) return fail(SAMSIM_ERR_ARG, "set_lab_lengths: nset differs from the last samsim_b200_set_lab_forcing");
+  for (int32_t s = 0; s < nset; s++)
+    if (nrec_of_set[s] < 1 || nrec_of_set[s] > h->lab_nrec) return fail(SAMSIM_ERR_ARG, "set_lab_lengths: every length must be in 1..nrec");
+  h->lab_len.assign(nrec_of_set, nrec_of_set + nset);
+  return 0;
+}
+
+int samsim_b200_set_end_step(samsim_handle_t h, const int64_t* end_i, int32_t col0, int32_t n) {
+  int rc = check_cols(h, col0, n);
+  if (rc) return rc;
+  if (n > 0 && !end_i) return fail(SAMSIM_ERR_ARG, "set_end_step: null pointer");
+  for (int32_t q = 0; q < n; q++)
+    if (end_i[q] < 0) return fail(SAMSIM_ERR_ARG, "set_end_step: end steps must be >= 0 (INT64_MAX = no end)");
+  if (n == 0) return 0;
+  CU(cudaSetDevice(h->device));
+  if (!h->end_of_col) {  // every column starts without an end, whatever the slot order
+    const std::vector<int64_t> none((size_t)h->ncol_pad, INT64_MAX);
+    CU(cudaMalloc(&h->end_of_col, none.size() * sizeof(int64_t)));
+    CU(cudaMemcpyAsync(h->end_of_col, none.data(), none.size() * sizeof(int64_t), cudaMemcpyHostToDevice, h->stream));
+    h->end_host.assign((size_t)h->ncol, INT64_MAX);
+  }
+  if ((rc = vec_set<int64_t>(h, h->end_of_col, end_i, col0, n))) return rc;
+  std::copy(end_i, end_i + n, h->end_host.begin() + col0);
+  update_lab_end(h);
   return 0;
 }
 
@@ -905,27 +978,34 @@ int samsim_b200_step(samsim_handle_t h, int64_t nsteps) {
       p.site_of_col = h->site_of_col; p.fscale = h->fscale; p.foffset = h->foffset;
     }
     if (need_lab) {
-      // Records FLOOR(1 + time/dt) of every step of the chunk must exist.  The device accumulates time by repeated
-      // `+ dt`, which for a dt that is not exactly representable can sit an ulp above k*dt: the bound is found by
-      // replaying the same additions, never by a multiplication.  Only the tail of the series needs the replay.
+      // Records FLOOR(1 + time/dt) of every step a column runs in the chunk must exist in its set.  The device
+      // accumulates time by repeated `+ dt`, which for a dt that is not exactly representable can sit an ulp above
+      // k*dt: the bound is found by replaying the same additions, never by a multiplication.  Only the tail of a
+      // series needs the replay.  A set whose columns have all passed their end step is not read any more.
       const double per_rec = tc8 ? 60.0 : h->cfg.dt;       // seconds per record
       const double t_last = tc8 ? 475200.0 : 1e300;          // the series is not read from this time on
       auto rec_at = [&](double t) { return (t < t_last) ? (long long)floor(1 + t / per_rec) : 1LL; };
       const long long first_rec = rec_at(h->time);
-      if (first_rec < 1 || first_rec > h->lab_nrec) return fail(SAMSIM_ERR_STATE, "step: lab series exhausted");
-      if (first_rec + (long long)((double)chunk * h->cfg.dt / per_rec) + 2 > h->lab_nrec) {
-        double t = h->time;
-        int64_t ok = 0;
-        for (; ok < chunk; ok++) {
-          const long long rec = rec_at(t);
-          if (rec < 1 || rec > h->lab_nrec) break;
-          t = t + h->cfg.dt;
+      for (size_t s = 0; s < h->lab_len.size(); s++) {
+        if (h->lab_end[s] <= h->i) continue;
+        const long long len = h->lab_len[s];
+        const int64_t need = std::min<int64_t>(chunk, h->lab_end[s] - h->i);  // steps the set's columns run
+        if (first_rec < 1 || first_rec > len) return fail(SAMSIM_ERR_STATE, "step: lab series exhausted");
+        if (first_rec + (long long)((double)need * h->cfg.dt / per_rec) + 2 > len) {
+          double t = h->time;
+          int64_t ok = 0;
+          for (; ok < need; ok++) {
+            const long long rec = rec_at(t);
+            if (rec < 1 || rec > len) break;
+            t = t + h->cfg.dt;
+          }
+          if (ok < 1) return fail(SAMSIM_ERR_STATE, "step: lab series exhausted");
+          if (ok < need) chunk = ok;
         }
-        if (ok < 1) return fail(SAMSIM_ERR_STATE, "step: lab series exhausted");
-        chunk = ok;
       }
       p.lab = h->lab; p.lab_nrec = h->lab_nrec; p.set_of_col = h->set_of_col;
     }
+    p.end_of_col = h->end_of_col;
     p.nsteps = (int)chunk;
     p.divergence = h->divergence;
     p.snap_sc = (h->snap_mode >= SAMSIM_SNAP_SCALARS) ? h->snap_sc : nullptr;
@@ -963,7 +1043,7 @@ int samsim_b200_step(samsim_handle_t h, int64_t nsteps) {
 // Re-bin the columns by regime (SURVEY 8e).  A warp costs as much as its deepest column and pays for every branch
 // any of its lanes takes, so an ensemble whose columns have drifted apart (freeze-up at different dates, different
 // snow states) runs faster once equal columns sit next to each other.  Columns are independent, so the order is
-// free: a stable radix sort on (failed, N_active, snow class, forcing site) gives the new order, every per-column
+// free: a stable radix sort on (failed or finished, N_active, snow class, forcing site) gives the new order, every per-column
 // row is permuted on the device, and slot_of_col / col_of_slot keep the caller's column numbering intact.
 int samsim_b200_rebin(samsim_handle_t h, int32_t* changed) {
   if (!h) return fail(SAMSIM_ERR_ARG, "null handle");
@@ -989,7 +1069,8 @@ int samsim_b200_rebin(samsim_handle_t h, int32_t* changed) {
   RB(cudaMalloc(&order, (size_t)n * sizeof(int)));
   RB(cudaMalloc(&flag, sizeof(int)));
   RB(cudaMemsetAsync(flag, 0, sizeof(int), h->stream));
-  samsim_rebin_key_kernel<<<nb, 256, 0, h->stream>>>(h->sc, h->in, h->site_of_col, n, h->ncol_pad, h->cfg.thick_min, keys, vals);
+  samsim_rebin_key_kernel<<<nb, 256, 0, h->stream>>>(h->sc, h->in, h->site_of_col, h->end_of_col, h->i, n, h->ncol_pad, h->cfg.thick_min,
+                                                      keys, vals);
   samsim_rebin_unsorted_kernel<<<nb, 256, 0, h->stream>>>(keys, n, flag);
   RB(cudaGetLastError());
   int unsorted = 0;
@@ -1019,6 +1100,7 @@ int samsim_b200_rebin(samsim_handle_t h, int32_t* changed) {
   if (!rc) rc = permute_rows<int>(h, h->in, IN_COUNT, order, tmp);
   if (!rc) rc = permute_rows<int>(h, h->site_of_col, 1, order, tmp);
   if (!rc) rc = permute_rows<int>(h, h->set_of_col, 1, order, tmp);
+  if (!rc) rc = permute_rows<int64_t>(h, h->end_of_col, 1, order, tmp);
   if (!rc) rc = permute_rows<double>(h, h->fscale, 4, order, tmp);
   if (!rc) rc = permute_rows<double>(h, h->foffset, 4, order, tmp);
   if (!rc) rc = permute_rows<double>(h, h->snap_sc, SAMSIM_SNAPSC_COUNT, order, tmp);
@@ -1072,7 +1154,8 @@ int samsim_b200_get_slot_map(samsim_handle_t h, int32_t* slot_of_col) {
 
 // ---- binary checkpoint / restart (SURVEY 8f-4; the reference can only start from init) ----------------------
 // File: "SAMB2CK1", sizeof(samsim_config_t), the config, ncol, the clock, then in the caller's column order
-// arrays[id][col][extent], scalars[id][col], ints[id][col].  Forcing tables are inputs, not state: set them again.
+// arrays[id][col][extent], scalars[id][col], ints[id][col].  Forcing tables, end steps and lab lengths are run inputs,
+// not state: set them again.
 static const char CK_MAGIC[8] = {'S', 'A', 'M', 'B', '2', 'C', 'K', '2'};
 
 int samsim_b200_save_checkpoint(samsim_handle_t h, const char* path) {

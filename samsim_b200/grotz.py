@@ -26,6 +26,10 @@ class _GrotzOptions(C.Structure):
                 ("quiet", C.c_int32), ("lab_input_dir", C.c_char_p)]
 
 
+class _GrotzMember(C.Structure):
+    _fields_ = [("testcase", C.c_int32), ("description", C.c_char_p), ("output_dir", C.c_char_p), ("max_steps", C.c_int64)]
+
+
 def _lib():
     L = api.load_library()
     L.samsim_host_init_testcase.restype = C.c_int
@@ -37,6 +41,8 @@ def _lib():
     L.samsim_host_read_lab_series.argtypes = [C.c_char_p, C.c_int32, C.c_int64, C.POINTER(C.c_double)]
     L.samsim_grotz.restype = C.c_int
     L.samsim_grotz.argtypes = [C.c_int32, C.c_char_p, C.POINTER(_GrotzOptions)]
+    L.samsim_grotz_batch.restype = C.c_int
+    L.samsim_grotz_batch.argtypes = [C.POINTER(_GrotzMember), C.c_int32, C.POINTER(_GrotzOptions), C.POINTER(C.c_int32)]
     return L
 
 
@@ -103,3 +109,29 @@ def grotz(testcase: int, description: str = "", *, output_dir, forcing_dir=".", 
     if rc < 0:
         raise api.SamsimError(rc, L.samsim_b200_last_error().decode())
     return rc
+
+
+def grotz_batch(members, *, device: int = 0, forcing_dir=None, lab_input_dir=None, quiet: bool = True) -> list[int]:
+    """Run several grotz(testcase, description) at once, one GPU column each, every member to its own end.
+
+    `members`: dicts with `testcase`, `output_dir` and optionally `description` and `max_steps` (0 = i_time).  The
+    testcases must share one configuration; 101-105 may be mixed.  Each member writes the dat_*.dat files grotz()
+    writes for it alone.  Returns each member's code: 0 or its reference STOP code.  forcing_dir / lab_input_dir
+    None = the reference's defaults ("." and "2017_input").
+    """
+    L = _lib()
+    ms = (_GrotzMember * len(members))() if members else None
+    for q, m in enumerate(members):
+        Path(m["output_dir"]).mkdir(parents=True, exist_ok=True)
+        ms[q] = _GrotzMember(testcase=int(m["testcase"]), description=str(m.get("description", "")).encode(),
+                             output_dir=str(m["output_dir"]).encode(), max_steps=int(m.get("max_steps", 0)))
+    o = _GrotzOptions(ncol=0, device=device, forcing_dir=None if forcing_dir is None else str(forcing_dir).encode(),
+                      output_dir=None, max_steps=0, quiet=int(quiet),
+                      lab_input_dir=None if lab_input_dir is None else str(lab_input_dir).encode())
+    codes = (C.c_int32 * max(len(members), 1))()
+    rc = L.samsim_grotz_batch(ms, len(members), C.byref(o), codes)
+    if rc < 0:
+        why = {-1: "bad argument (members, or an option that belongs to samsim_grotz)",
+               -4: "the members' testcases do not share one configuration"}
+        raise api.SamsimError(rc, why.get(rc) or L.samsim_b200_last_error().decode())
+    return [int(c) for c in codes[:len(members)]]

@@ -134,6 +134,15 @@ MODULE mo_samsim_b200
        TYPE(C_PTR), VALUE :: site_of_col, scale, offset   !< C_NULL_PTR = site 0 / identity
      END FUNCTION samsim_b200_set_forcing
 
+     !> refresh records rec0 .. rec0+n-1 (1-based) of every site and kind from series((site*4 + kind)*n + r)
+     INTEGER(C_INT) FUNCTION samsim_b200_update_forcing_records(handle, rec0, n, series) &
+          & BIND(C, NAME='samsim_b200_update_forcing_records')
+       IMPORT :: C_INT, C_INT32_T, C_PTR, C_DOUBLE
+       TYPE(C_PTR), VALUE :: handle
+       INTEGER(C_INT32_T), VALUE :: rec0, n
+       REAL(C_DOUBLE), INTENT(in) :: series(*)
+     END FUNCTION samsim_b200_update_forcing_records
+
      INTEGER(C_INT) FUNCTION samsim_b200_set_lab_forcing(handle, nset, nrec, series, set_of_col) &
           & BIND(C, NAME='samsim_b200_set_lab_forcing')
        IMPORT :: C_INT, C_INT32_T, C_INT64_T, C_PTR, C_DOUBLE

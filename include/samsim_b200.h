@@ -224,13 +224,25 @@ int samsim_b200_get_clock(samsim_handle_t h, double* time, int64_t* i, int32_t* 
  * each, series[(site*4 + kind)*nrec + r]; time_input(k) = (k-1)*10800 s.  Column c reads site
  * site_of_col[c] through value*scale + offset with scale/offset[kind*ncol + c]; NULL = site 0 /
  * identity.  One multiply and one add in double, so the CPU oracle fed series*scale+offset
- * matches bit for bit. */
+ * matches bit for bit.  Any nsite >= 1 is accepted, up to one site per column or more (a reanalysis grid cell per
+ * column, or a series shifted in time per ensemble member for its own start date); only device memory limits the
+ * table (nsite*4*nrec doubles).  Up to 16 sites are staged in shared memory per launch, larger tables are read in
+ * place; both give the same results.  site_of_col is checked before anything is replaced (SAMSIM_ERR_ARG leaves the
+ * previous forcing in place).  If a device allocation or copy fails (SAMSIM_ERR_CUDA), the handle holds no forcing
+ * at all afterwards, as if set_forcing had never been called: steps with atmoflux_flag 2 return SAMSIM_ERR_STATE
+ * until a set_forcing succeeds. */
 int samsim_b200_set_forcing(samsim_handle_t h, int32_t nsite, int32_t nrec, const double* series,
                             const int32_t* site_of_col, const double* scale, const double* offset);
 /* Refresh the base series of an existing forcing table in place (same nsite/nrec; per-column vectors are kept):
  * the streaming path when new reanalysis records arrive while the run is in progress.  Asynchronous on the handle's
  * stream when `series` is pinned host memory. */
 int samsim_b200_update_forcing(samsim_handle_t h, const double* series);
+/* Refresh records rec0 .. rec0+n-1 (1-based) of every site and kind of the table of the last set_forcing from
+ * series[(site*4 + kind)*n + r], r = 0..n-1; all other records are kept.  The streaming path of large tables: a day
+ * of new records for every site, without sending the whole table again.  One 2-D copy on the handle's stream,
+ * ordered with launches like samsim_b200_update_forcing (asynchronous when `series` is pinned host memory).
+ * SAMSIM_ERR_STATE before set_forcing; SAMSIM_ERR_ARG for a NULL pointer, n < 1 or records outside 1..nrec. */
+int samsim_b200_update_forcing_records(samsim_handle_t h, int32_t rec0, int32_t n, const double* series);
 /* lab series (mo_grotz.f90:138-169): nset record sets of nrec per-dt values, kinds
  * 0 Tice->T2m, 1 snowfall->solid_precip, 2 heat->fl_q_bottom, 3 styropor; series[(set*4+kind)*nrec + r];
  * set_of_col NULL = set 0.  snow_precip_flag 0 zeroes the snowfall like the reference. */

@@ -165,6 +165,7 @@ def load_library() -> C.CDLL:
         "samsim_b200_get_clock": (C.c_int, [H, dp, C.POINTER(C.c_int64), ip, ip]),
         "samsim_b200_set_forcing": (C.c_int, [H, C.c_int32, C.c_int32, dp, ip, dp, dp]),
         "samsim_b200_update_forcing": (C.c_int, [H, dp]),
+        "samsim_b200_update_forcing_records": (C.c_int, [H, C.c_int32, C.c_int32, dp]),
         "samsim_b200_set_lab_forcing": (C.c_int, [H, C.c_int32, C.c_int64, dp, ip]),
         "samsim_b200_set_lab_lengths": (C.c_int, [H, C.c_int32, C.POINTER(C.c_int64)]),
         "samsim_b200_step": (C.c_int, [H, C.c_int64]),
@@ -205,6 +206,7 @@ EXPORTED_SYMBOLS = [
     "samsim_b200_array_extent", "samsim_b200_set_array", "samsim_b200_get_array", "samsim_b200_set_scalar",
     "samsim_b200_get_scalar", "samsim_b200_set_int", "samsim_b200_get_int", "samsim_b200_broadcast_column",
     "samsim_b200_set_clock", "samsim_b200_get_clock", "samsim_b200_set_forcing", "samsim_b200_update_forcing",
+    "samsim_b200_update_forcing_records",
     "samsim_b200_set_lab_forcing", "samsim_b200_set_lab_lengths", "samsim_b200_set_end_step",
     "samsim_b200_step", "samsim_b200_synchronize", "samsim_b200_steps_to_next_output",
     "samsim_b200_set_snapshot_mode", "samsim_b200_get_snapshot", "samsim_b200_get_status",
@@ -341,7 +343,9 @@ class Engine:
 
     # ---- forcing ----------------------------------------------------------------------------
     def set_forcing(self, series, site_of_col=None, scale=None, offset=None):
-        """series[nsite, 4, nrec] in kind order fl_sw, fl_lw, T2m, precip; scale/offset[4, ncol]."""
+        """series[nsite, 4, nrec] in kind order fl_sw, fl_lw, T2m, precip; site_of_col[ncol]; scale/offset[4, ncol].
+        Any nsite is accepted, up to one series per column or more (a grid cell per column, a time-shifted series
+        per ensemble member); only device memory limits the table."""
         s = np.ascontiguousarray(series, dtype=np.float64)
         if s.ndim == 2:
             s = s[None]
@@ -357,6 +361,15 @@ class Engine:
         s = series if isinstance(series, np.ndarray) and series.flags.c_contiguous and series.dtype == np.float64 \
             else np.ascontiguousarray(series, dtype=np.float64)
         _check(self.L, self.L.samsim_b200_update_forcing(self.h, _dp(s)))
+
+    def update_forcing_records(self, rec0: int, series):
+        """Refresh records rec0 .. rec0+n-1 (1-based) of every site and kind from series[nsite, 4, n]; the other
+        records of the table are kept."""
+        s = np.ascontiguousarray(series, dtype=np.float64)
+        if s.ndim == 2:
+            s = s[None]
+        assert s.ndim == 3 and s.shape[1] == 4
+        _check(self.L, self.L.samsim_b200_update_forcing_records(self.h, int(rec0), s.shape[2], _dp(s)))
 
     def set_lab_forcing(self, series, set_of_col=None, nrec_of_set=None):
         """series[nset, 4, nrec] in kind order Tice, snowfall, heat, styropor.  nrec_of_set[nset]: the real length of

@@ -36,7 +36,11 @@ static_assert((int)SAMSIM_SNAPSC_COUNT == 20 && (int)SAMSIM_SNAPARR_COUNT == 14,
 #define SAMSIM_MINBLOCKS 2
 #endif
 #define SAMSIM_MAXWIN 24   // forcing records staged per launch (3-hourly): 22 * 10800 s of model time per launch
+// Tables of up to SAMSIM_MAXSITE sites are staged in shared memory per launch; larger ones are read in place from
+// global memory (samsim_b200_set_forcing)
+#ifndef SAMSIM_MAXSITE
 #define SAMSIM_MAXSITE 16
+#endif
 
 // ------------------------------------------------------------------------------------------
 // kernel parameters
@@ -54,7 +58,7 @@ struct KParams {
   int n_time_out, time_counter;
   int nsteps;
   // forcing
-  const double* series;   // [nsite][4][nrec] global
+  const double* series;   // [nsite][4][nrec] global; staged when nsite <= SAMSIM_MAXSITE
   int nsite, nrec, win_first, win_len;
   const int* site_of_col; // [ncol_pad] or nullptr
   const double* fscale;   // [4][ncol_pad] or nullptr
@@ -84,8 +88,9 @@ __device__ __forceinline__ void cp_async8(void* smem_dst, const void* gmem_src) 
 template <bool TWO_PASS>
 __global__ void __launch_bounds__(SAMSIM_BLOCK, SAMSIM_MINBLOCKS) samsim_step_kernel(const __grid_constant__ KParams p) {
   __shared__ double s_win[SAMSIM_MAXSITE * 4 * SAMSIM_MAXWIN];
+  const bool staged = (p.nsite <= SAMSIM_MAXSITE);
   // stage the forcing window: records win_first .. win_first+win_len-1 of every site/kind (cp.async)
-  if (p.series != nullptr) {
+  if (p.series != nullptr && staged) {
     const int n = p.nsite * 4 * p.win_len;
     for (int e = threadIdx.x; e < n; e += blockDim.x) {
       const int sk = e / p.win_len, r = e - sk * p.win_len;
@@ -122,7 +127,11 @@ __global__ void __launch_bounds__(SAMSIM_BLOCK, SAMSIM_MINBLOCKS) samsim_step_ke
   c.fb_x = 0.0;
 
   Forcing f;
-  f.win = s_win; f.win_len = p.win_len; f.win_first = p.win_first;
+  if (staged) {
+    f.win = s_win; f.win_len = p.win_len; f.win_first = p.win_first;
+  } else {  // the table as samsim_b200_set_forcing stored it
+    f.win = p.series; f.win_len = p.nrec; f.win_first = 1; f.global = true;
+  }
   f.site = p.site_of_col ? p.site_of_col[col] : 0;
   for (int k = 0; k < 4; k++) {
     f.scale[k] = p.fscale ? p.fscale[(size_t)k * ls + col] : 1.0;
@@ -269,10 +278,11 @@ __global__ void samsim_vec_set_kernel(T* row, const T* src, int col0, int n, con
 
 // ---- re-binning (SURVEY 8e: columns are re-binned by regime for warp coherence; local permutation only) ----
 // key: failed and finished columns last; then N_active descending (loop trip counts), snow class (the snow branches) and melting
-// surface (flushing, full S4 sweep), forcing site, surface temperature
+// surface (flushing, full S4 sweep), forcing site, surface temperature.  Bits from the top: idle (1), 0xFFF - N_active (12),
+// class (3), site (site_bits, the whole site index), T_top bucket (10).
 __global__ void samsim_rebin_key_kernel(const double* sc, const int* in, const int* site_of_col, const int64_t* end_of_col,
-                                        long long i, long long ncol, long long ncol_pad, double thick_min, unsigned* keys,
-                                        int* vals) {
+                                        long long i, long long ncol, long long ncol_pad, double thick_min, int site_bits,
+                                        unsigned long long* keys, int* vals) {
   const long long s = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (s >= ncol) return;
   const int na = in[(size_t)IN_N_ACTIVE * ncol_pad + s];
@@ -281,16 +291,18 @@ __global__ void samsim_rebin_key_kernel(const double* sc, const int* in, const i
   const double snow = sc[(size_t)SC_THICK_SNOW * ncol_pad + s];
   const unsigned cls = ((snow <= 0.0) ? 0u : (snow < thick_min / 100.0) ? 1u : (snow < thick_min) ? 2u : 3u) |
                        ((sc[(size_t)SC_MELT_THICK * ncol_pad + s] > 0.0) ? 4u : 0u);  // melting surface: the flushing / full-S4 path
-  const unsigned site = site_of_col ? (unsigned)site_of_col[s] : 0u;
+  const unsigned long long site = site_of_col ? (unsigned)site_of_col[s] : 0u;
   // deepest columns first: blocks are dispatched in index order, so the cheap ones fill the tail of the launch
   // within a site, columns with a similar surface temperature (0.1 K buckets over -80..+22 degC) sit next to each other:
   // their Newton sweeps take the same number of iterations and their drainage candidates span the same layers
   const double tt = sc[(size_t)SC_T_TOP * ncol_pad + s];
   const unsigned tb = (tt > -80.0) ? ((tt < 22.3) ? (unsigned)((tt + 80.0) * 10.0) : 1023u) : 0u;  // NaN -> 0
-  keys[s] = (idle ? 0x80000000u : 0u) | ((0xFFFu - ((unsigned)na & 0xFFFu)) << 19) | (cls << 15) | ((site & 0x1Fu) << 10) | tb;
+  const int b = 10 + site_bits;
+  keys[s] = ((idle ? 1ull : 0ull) << (b + 15)) | ((unsigned long long)(0xFFFu - ((unsigned)na & 0xFFFu)) << (b + 3)) |
+            ((unsigned long long)cls << b) | (site << 10) | tb;
   vals[s] = (int)s;
 }
-__global__ void samsim_rebin_unsorted_kernel(const unsigned* keys, long long ncol, int* out) {
+__global__ void samsim_rebin_unsorted_kernel(const unsigned long long* keys, long long ncol, int* out) {
   const long long s = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (s + 1 < ncol && keys[s] > keys[s + 1]) atomicAdd(out, 1);
 }
@@ -765,17 +777,15 @@ int samsim_b200_get_clock(samsim_handle_t h, double* time, int64_t* i, int32_t* 
   return 0;
 }
 
-int samsim_b200_set_forcing(samsim_handle_t h, int32_t nsite, int32_t nrec, const double* series, const int32_t* site_of_col,
-                            const double* scale, const double* offset) {
-  if (!h || !series || nsite < 1 || nsite > SAMSIM_MAXSITE || nrec < 2) return fail(SAMSIM_ERR_ARG, "set_forcing: bad argument (nsite <= 16)");
-  if (site_of_col)  // validate everything before the tables of the previous call are replaced
-    for (long long c = 0; c < h->ncol; c++)
-      if (site_of_col[c] < 0 || site_of_col[c] >= nsite) return fail(SAMSIM_ERR_ARG, "set_forcing: site index out of range");
-  CU(cudaSetDevice(h->device));
-  CU(cudaStreamSynchronize(h->stream));  // a launch in flight may still read the old tables
+static void drop_forcing(samsim_handle_t h) {
   cudaFree(h->series); cudaFree(h->site_of_col); cudaFree(h->fscale); cudaFree(h->foffset);
   h->series = nullptr; h->site_of_col = nullptr; h->fscale = nullptr; h->foffset = nullptr;
-  const size_t nb = (size_t)nsite * 4 * nrec * sizeof(double);
+  h->nsite = h->nrec = 0;
+}
+
+static int upload_forcing(samsim_handle_t h, int32_t nsite, int32_t nrec, const double* series, const int32_t* site_of_col,
+                          const double* scale, const double* offset) {
+  const size_t nb = (size_t)nsite * 4 * (size_t)nrec * sizeof(double);
   CU(cudaMalloc(&h->series, nb));
   CU(cudaMemcpy(h->series, series, nb, cudaMemcpyHostToDevice));
   h->nsite = nsite; h->nrec = nrec;
@@ -799,11 +809,40 @@ int samsim_b200_set_forcing(samsim_handle_t h, int32_t nsite, int32_t nrec, cons
   return 0;
 }
 
+int samsim_b200_set_forcing(samsim_handle_t h, int32_t nsite, int32_t nrec, const double* series, const int32_t* site_of_col,
+                            const double* scale, const double* offset) {
+  if (!h || !series || nsite < 1 || nrec < 2) return fail(SAMSIM_ERR_ARG, "set_forcing: bad argument");
+  if (site_of_col)  // validate everything before the tables of the previous call are replaced
+    for (long long c = 0; c < h->ncol; c++)
+      if (site_of_col[c] < 0 || site_of_col[c] >= nsite) return fail(SAMSIM_ERR_ARG, "set_forcing: site index out of range");
+  CU(cudaSetDevice(h->device));
+  CU(cudaStreamSynchronize(h->stream));  // a launch in flight may still read the old tables
+  drop_forcing(h);
+  const int rc = upload_forcing(h, nsite, nrec, series, site_of_col, scale, offset);
+  if (rc) {  // e.g. a table larger than the free device memory: the handle is left without forcing
+    drop_forcing(h);
+    cudaGetLastError();  // an allocation failure is not sticky; keep it from surfacing at the next launch check
+  }
+  return rc;
+}
+
 int samsim_b200_update_forcing(samsim_handle_t h, const double* series) {
   if (!h || !series) return fail(SAMSIM_ERR_ARG, "update_forcing: bad argument");
   if (!h->series) return fail(SAMSIM_ERR_STATE, "update_forcing: call samsim_b200_set_forcing first");
   CU(cudaSetDevice(h->device));
   CU(cudaMemcpyAsync(h->series, series, (size_t)h->nsite * 4 * h->nrec * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+  return 0;
+}
+
+int samsim_b200_update_forcing_records(samsim_handle_t h, int32_t rec0, int32_t n, const double* series) {
+  if (!h || !series) return fail(SAMSIM_ERR_ARG, "update_forcing_records: bad argument");
+  if (!h->series) return fail(SAMSIM_ERR_STATE, "update_forcing_records: call samsim_b200_set_forcing first");
+  if (n < 1 || rec0 < 1 || (int64_t)rec0 + n - 1 > h->nrec)
+    return fail(SAMSIM_ERR_ARG, "update_forcing_records: records rec0 .. rec0+n-1 must lie in 1..nrec");
+  CU(cudaSetDevice(h->device));
+  // one row of n records per (site, kind): source rows are n apart, table rows nrec apart
+  CU(cudaMemcpy2DAsync(h->series + (rec0 - 1), (size_t)h->nrec * sizeof(double), series, (size_t)n * sizeof(double),
+                       (size_t)n * sizeof(double), (size_t)h->nsite * 4, cudaMemcpyHostToDevice, h->stream));
   return 0;
 }
 
@@ -1051,7 +1090,7 @@ int samsim_b200_rebin(samsim_handle_t h, int32_t* changed) {
   CU(cudaSetDevice(h->device));
   const long long n = h->ncol;
   const unsigned nb = (unsigned)((n + 255) / 256);
-  unsigned *keys = nullptr, *keys_out = nullptr;
+  unsigned long long *keys = nullptr, *keys_out = nullptr;
   int *vals = nullptr, *order = nullptr, *flag = nullptr;
   void *cub_tmp = nullptr, *tmp = nullptr;
   int rc = 0;
@@ -1063,14 +1102,17 @@ int samsim_b200_rebin(samsim_handle_t h, int32_t* changed) {
     cudaError_t e_ = (call);                                                                  \
     if (e_ != cudaSuccess) { cleanup(); return fail(SAMSIM_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_)); } \
   } while (0)
-  RB(cudaMalloc(&keys, (size_t)n * sizeof(unsigned)));
-  RB(cudaMalloc(&keys_out, (size_t)n * sizeof(unsigned)));
+  RB(cudaMalloc(&keys, (size_t)n * sizeof(unsigned long long)));
+  RB(cudaMalloc(&keys_out, (size_t)n * sizeof(unsigned long long)));
   RB(cudaMalloc(&vals, (size_t)n * sizeof(int)));
   RB(cudaMalloc(&order, (size_t)n * sizeof(int)));
   RB(cudaMalloc(&flag, sizeof(int)));
   RB(cudaMemsetAsync(flag, 0, sizeof(int), h->stream));
+  int site_bits = 0;  // bits of the largest site index
+  while (h->site_of_col && (1ll << site_bits) < h->nsite) site_bits++;
+  const int end_bit = 26 + site_bits;
   samsim_rebin_key_kernel<<<nb, 256, 0, h->stream>>>(h->sc, h->in, h->site_of_col, h->end_of_col, h->i, n, h->ncol_pad, h->cfg.thick_min,
-                                                      keys, vals);
+                                                      site_bits, keys, vals);
   samsim_rebin_unsorted_kernel<<<nb, 256, 0, h->stream>>>(keys, n, flag);
   RB(cudaGetLastError());
   int unsorted = 0;
@@ -1079,9 +1121,9 @@ int samsim_b200_rebin(samsim_handle_t h, int32_t* changed) {
   if (unsorted == 0) { cleanup(); return 0; }  // already in regime order
 
   size_t cub_bytes = 0;
-  RB(cub::DeviceRadixSort::SortPairs(nullptr, cub_bytes, keys, keys_out, vals, order, (int)n, 0, 32, h->stream));
+  RB(cub::DeviceRadixSort::SortPairs(nullptr, cub_bytes, keys, keys_out, vals, order, (int)n, 0, end_bit, h->stream));
   RB(cudaMalloc(&cub_tmp, cub_bytes));
-  RB(cub::DeviceRadixSort::SortPairs(cub_tmp, cub_bytes, keys, keys_out, vals, order, (int)n, 0, 32, h->stream));
+  RB(cub::DeviceRadixSort::SortPairs(cub_tmp, cub_bytes, keys, keys_out, vals, order, (int)n, 0, end_bit, h->stream));
   RB(cudaMalloc(&tmp, permute_tmp_bytes(h)));
 
   const size_t astr = (size_t)h->LS * h->ncol_pad;  // one array of the (row-major) snapshot buffer

@@ -9,8 +9,9 @@ namespace samsim {
 
 // forcing tables visible to a thread
 struct Forcing {
-  // atmoflux_flag 2: window of records staged in shared memory, [(site*4 + kind)*win + r]
-  const double* win;      // shared memory
+  // atmoflux_flag 2: window of records, [(site*4 + kind)*win_len + r]: staged in shared memory, or (global) the
+  // whole table in global memory with win_len = nrec and win_first = 1
+  const double* win;
   int win_len;            // records in the window
   int win_first;          // 1-based record number of window element 0
   int site;               // this column's site
@@ -19,10 +20,17 @@ struct Forcing {
   const double* lab;
   long long lab_nrec;
   int lab_set;
+  bool global = false;    // win is the device table in global memory: read-only loads, 64-bit index
 };
 
 __device__ __forceinline__ double forcing_rec(const Forcing& f, int kind, int rec /*1-based*/) {
-  const double base = f.win[(f.site * 4 + kind) * f.win_len + (rec - f.win_first)];
+#ifdef __CUDA_ARCH__
+  // (site*4 + kind)*nrec passes 2^31 at about 183,000 sites of a year of 3-hourly records
+  const double base = f.global ? __ldg(f.win + (((long long)f.site * 4 + kind) * f.win_len + (rec - f.win_first)))
+                               : f.win[(f.site * 4 + kind) * f.win_len + (rec - f.win_first)];
+#else
+  const double base = f.win[((long long)f.site * 4 + kind) * f.win_len + (rec - f.win_first)];
+#endif
   return base * f.scale[kind] + f.offset[kind];
 }
 // time_input(k) = (REAL(k)-1._wp)*3600._wp*3._wp, mo_functions.f90:323-325

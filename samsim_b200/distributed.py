@@ -19,6 +19,16 @@ def shard(total: int, rank: int, world: int) -> tuple[int, int]:
     return col0, n
 
 
+def local_sites(site_of_col, col0: int, n: int) -> tuple[np.ndarray, np.ndarray]:
+    """The forcing sites of the block [col0, col0 + n) of a rank: (sites, local_site_of_col).  `sites` are the
+    sorted distinct sites the block reads and local_site_of_col[c] indexes into them, so the rank uploads
+    table[sites] with local_site_of_col instead of the whole grid: table[sites][local_site_of_col] equals
+    table[site_of_col[col0:col0 + n]]."""
+    block = np.asarray(site_of_col)[col0:col0 + n]
+    sites, local = np.unique(block, return_inverse=True)
+    return sites, local.astype(np.int32).reshape(-1)
+
+
 def reduce_ensemble(local: dict, ncol_local: int, group=None, device=None) -> dict:
     """local = Engine.reduce_diag() of this rank; returns the ensemble-wide mean/min/max per diagnostic."""
     import torch

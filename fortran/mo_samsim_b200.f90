@@ -199,6 +199,33 @@ MODULE mo_samsim_b200
        INTEGER(C_INT32_T), VALUE :: col0, n
      END FUNCTION samsim_b200_get_snapshot
 
+     !> ensemble statistics per column group at every output record (ngroup = 0: off); group_of_col, depth: C_LOC of
+     !> the arrays or C_NULL_PTR; profile_mask: bits of samsim_snapshot_array_id (uint32_t in C, masks < 2**14)
+     INTEGER(C_INT) FUNCTION samsim_b200_set_group_stats(handle, ngroup, group_of_col, nz, depth, profile_mask, &
+          & max_records) BIND(C, NAME='samsim_b200_set_group_stats')
+       IMPORT :: C_INT, C_INT32_T, C_PTR
+       TYPE(C_PTR), VALUE :: handle, group_of_col, depth
+       INTEGER(C_INT32_T), VALUE :: ngroup, nz, profile_mask, max_records
+     END FUNCTION samsim_b200_set_group_stats
+
+     INTEGER(C_INT32_T) FUNCTION samsim_b200_group_stats_held(handle) BIND(C, NAME='samsim_b200_group_stats_held')
+       IMPORT :: C_INT32_T, C_PTR
+       TYPE(C_PTR), VALUE :: handle
+     END FUNCTION samsim_b200_group_stats_held
+
+     !> records rec0 .. rec0+nrec-1 (0-based): stats(5, Q, ngroup, nrec), rec_time(nrec), rec_i(nrec); C_NULL_PTR skips one
+     INTEGER(C_INT) FUNCTION samsim_b200_get_group_stats(handle, stats, rec_time, rec_i, rec0, nrec) &
+          & BIND(C, NAME='samsim_b200_get_group_stats')
+       IMPORT :: C_INT, C_INT32_T, C_PTR
+       TYPE(C_PTR), VALUE :: handle, stats, rec_time, rec_i
+       INTEGER(C_INT32_T), VALUE :: rec0, nrec
+     END FUNCTION samsim_b200_get_group_stats
+
+     INTEGER(C_INT) FUNCTION samsim_b200_clear_group_stats(handle) BIND(C, NAME='samsim_b200_clear_group_stats')
+       IMPORT :: C_INT, C_PTR
+       TYPE(C_PTR), VALUE :: handle
+     END FUNCTION samsim_b200_clear_group_stats
+
      INTEGER(C_INT) FUNCTION samsim_b200_get_status(handle, status, col0, n) BIND(C, NAME='samsim_b200_get_status')
        IMPORT :: C_INT, C_INT32_T, C_PTR
        TYPE(C_PTR), VALUE :: handle

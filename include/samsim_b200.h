@@ -277,6 +277,37 @@ int samsim_b200_set_snapshot_mode(samsim_handle_t h, int32_t mode);
  * arrays[(c*SAMSIM_SNAPARR_COUNT + id)*Nlayer + (k-1)] (arrays may be NULL) */
 int samsim_b200_get_snapshot(samsim_handle_t h, double* scalars, double* arrays, int32_t col0, int32_t n);
 
+/* ---- ensemble statistics per column group at every S8 record ------------------------------------
+ * Computed and kept on the device, so that one samsim_b200_step call may span any number of records.  ngroup = 0
+ * switches them off (the default).  group_of_col[c] in [-1, ngroup) in the caller's column order, -1 = in no group,
+ * NULL = every column in group 0.  depth[0..nz): metres below the ice surface (the top of layer 1), finite, > 0 and
+ * strictly increasing; nz = 0 = scalars only.  profile_mask: bits of samsim_snapshot_array_id (not RAY; tracer rows only
+ * with N_bgc tracers; non-zero needs nz > 0).  A bad argument is SAMSIM_ERR_ARG and keeps the previous setting; a
+ * snapshot mode below SCALARS (FULL with profiles) is SAMSIM_ERR_STATE.  A new setting drops the held records.
+ *
+ * Quantities q: the SAMSIM_SNAPSC_COUNT scalars, then nz depths of each selected profile in samsim_snapshot_array_id
+ * order.  stats[((r*ngroup + g)*Q + q)*5 + s], s = count, mean, variance, min, max; rec_time[r] = SAMSIM_SNAPSC_TIME
+ * and rec_i[r] = loop index of record r; any output pointer may be NULL.
+ *
+ * Bitwise contract.  A member contributes to the record of step i when its status is 0 at the end of step i and its
+ * end step is >= i.  Profile p at depth z: p(k) of the smallest k <= N_active with z <= D_k, D_k = (((thick(1) +
+ * thick(2)) + ...) + thick(k)) over the snapshot; a member with z > D_{N_active} does not contribute there.  Sums are
+ * the pairwise tree over ALL members of the group in ascending caller column order (non-contributing ones +0.0),
+ * padded with +0.0 to a power of two, a = a[0::2] + a[1::2] repeated; mean = S / count; M2 = the same tree over
+ * (x - mean)^2 (+0.0 for the others); variance = M2 / (count - 1), 0 for count 1; min / max = fmin / fmax over the
+ * contributors; count 0 gives NaN for mean, variance, min and max.  Results do not depend on re-binning or launch
+ * lengths.
+ *
+ * samsim_b200_step with statistics on: no launch runs past an output step, and after each launch that ends on one the
+ * statistics kernels are queued on the handle's stream (no host synchronisation).  A call that would write more
+ * records than max_records - held returns SAMSIM_ERR_STATE before anything runs.  Not saved in checkpoints. */
+int samsim_b200_set_group_stats(samsim_handle_t h, int32_t ngroup, const int32_t* group_of_col, int32_t nz,
+                                const double* depth, uint32_t profile_mask, int32_t max_records);
+int32_t samsim_b200_group_stats_held(samsim_handle_t h); /* records held, -1 for a null handle */
+int samsim_b200_get_group_stats(samsim_handle_t h, double* stats, double* rec_time, int64_t* rec_i, int32_t rec0,
+                                int32_t nrec);
+int samsim_b200_clear_group_stats(samsim_handle_t h); /* drop the held records */
+
 /* ---- diagnostics -------------------------------------------------------------------------- */
 int samsim_b200_get_status(samsim_handle_t h, int32_t* status, int32_t col0, int32_t n);
 /* number of columns with non-zero status */

@@ -174,6 +174,10 @@ def load_library() -> C.CDLL:
         "samsim_b200_steps_to_next_output": (C.c_int64, [H]),
         "samsim_b200_set_snapshot_mode": (C.c_int, [H, C.c_int32]),
         "samsim_b200_get_snapshot": (C.c_int, [H, dp, dp, C.c_int32, C.c_int32]),
+        "samsim_b200_set_group_stats": (C.c_int, [H, C.c_int32, ip, C.c_int32, dp, C.c_uint32, C.c_int32]),
+        "samsim_b200_group_stats_held": (C.c_int32, [H]),
+        "samsim_b200_get_group_stats": (C.c_int, [H, dp, dp, C.POINTER(C.c_int64), C.c_int32, C.c_int32]),
+        "samsim_b200_clear_group_stats": (C.c_int, [H]),
         "samsim_b200_get_status": (C.c_int, [H, ip, C.c_int32, C.c_int32]),
         "samsim_b200_count_failed": (C.c_int, [H, ip]),
         "samsim_b200_reduce_diag": (C.c_int, [H, dp]),
@@ -209,7 +213,9 @@ EXPORTED_SYMBOLS = [
     "samsim_b200_update_forcing_records",
     "samsim_b200_set_lab_forcing", "samsim_b200_set_lab_lengths", "samsim_b200_set_end_step",
     "samsim_b200_step", "samsim_b200_synchronize", "samsim_b200_steps_to_next_output",
-    "samsim_b200_set_snapshot_mode", "samsim_b200_get_snapshot", "samsim_b200_get_status",
+    "samsim_b200_set_snapshot_mode", "samsim_b200_get_snapshot", "samsim_b200_set_group_stats",
+    "samsim_b200_group_stats_held", "samsim_b200_get_group_stats", "samsim_b200_clear_group_stats",
+    "samsim_b200_get_status",
     "samsim_b200_count_failed", "samsim_b200_reduce_diag", "samsim_b200_launch_count", "samsim_b200_last_step_ms",
     "samsim_b200_device_layout", "samsim_b200_save_checkpoint", "samsim_b200_load_checkpoint", "samsim_b200_rebin", "samsim_b200_set_tuning", "samsim_b200_set_rebin_interval", "samsim_b200_set_rebin_auto", "samsim_b200_get_divergence", "samsim_b200_get_slot_map",
     "samsim_b200_kat_getT", "samsim_b200_kat_scalar", "samsim_b200_fp64_peak",
@@ -420,6 +426,49 @@ class Engine:
             for j, name in enumerate(SNAP_ARRAYS):
                 out[name] = ar[:, j, : (self.cfg.Nlayer - 1 if name == "ray" else self.cfg.Nlayer)]
         return out
+
+    # ---- group statistics at S8 records -------------------------------------------------------
+    def set_group_stats(self, group_of_col=None, depths=(), profiles=(), max_records: int = 64, ngroup: int | None = None):
+        """Ensemble statistics per column group at every output record, kept on the device (include/samsim_b200.h).
+        group_of_col[ncol] in [-1, ngroup), -1 = in no group, None = one group of every column; ngroup defaults to
+        max(group_of_col) + 1, and 0 switches the statistics off.  depths: metres below the ice surface; profiles:
+        names of SNAP_ARRAYS.  Needs snapshot mode SCALARS, FULL with profiles."""
+        goc = None if group_of_col is None else np.ascontiguousarray(group_of_col, dtype=np.int32)
+        if ngroup is None:
+            ngroup = 1 if goc is None else int(goc.max()) + 1
+        assert goc is None or goc.shape == (self.ncol,)
+        z = np.ascontiguousarray(depths, dtype=np.float64).reshape(-1)
+        mask = 0
+        for name in profiles:
+            mask |= 1 << SNAP_ARRAYS.index(name)
+        _check(self.L, self.L.samsim_b200_set_group_stats(self.h, int(ngroup), _ip(goc), len(z), _dp(z) if len(z) else None,
+                                                          mask, int(max_records)))
+        self._gs = {"ngroup": int(ngroup), "depths": z.copy(),
+                    "profiles": [n for j, n in enumerate(SNAP_ARRAYS) if mask >> j & 1]} if ngroup else None
+
+    def group_stats_held(self) -> int:
+        return int(self.L.samsim_b200_group_stats_held(self.h))
+
+    def group_stats(self, clear: bool = True, rec0: int = 0, nrec: int | None = None) -> dict:
+        """The held records: time[R], i[R], quantities [(name, depth or None)] and count / mean / var / min / max of
+        shape [R, G, Q].  clear=True drops the held records afterwards."""
+        g = getattr(self, "_gs", None)
+        assert g is not None, "group statistics are off"
+        nrec = self.group_stats_held() - rec0 if nrec is None else nrec
+        qn = [(n, None) for n in SNAP_SCALARS] + [(p, float(d)) for p in g["profiles"] for d in g["depths"]]
+        st = np.empty((nrec, g["ngroup"], len(qn), 5), dtype=np.float64)
+        t = np.empty(nrec, dtype=np.float64)
+        i = np.empty(nrec, dtype=np.int64)
+        _check(self.L, self.L.samsim_b200_get_group_stats(self.h, _dp(st), _dp(t), _lp(i), int(rec0), int(nrec)))
+        if clear:
+            _check(self.L, self.L.samsim_b200_clear_group_stats(self.h))
+        out = {"time": t, "i": i, "quantities": qn}
+        for k, name in enumerate(("count", "mean", "var", "min", "max")):
+            out[name] = st[..., k]
+        return out
+
+    def clear_group_stats(self):
+        _check(self.L, self.L.samsim_b200_clear_group_stats(self.h))
 
     # ---- diagnostics ------------------------------------------------------------------------
     def status(self) -> np.ndarray:

@@ -15,6 +15,7 @@
 #include <cub/device/device_radix_sort.cuh>
 
 #include "../../include/samsim_b200.h"
+#include "group_stats.cuh"
 #include "step.cuh"
 
 using namespace samsim;
@@ -350,6 +351,177 @@ __global__ void samsim_reduce_kernel(const double* sc, const int* in, long long 
       for (int q = 0; q < 3; q++) out[((size_t)blockIdx.x * 6 + j) * 3 + q] = sh[j][q][0];
 }
 
+// ---- group statistics at S8 records (group_stats.cuh; samsim_b200_set_group_stats) --------------------------------
+struct GsParams {
+  // snapshot, status and end steps, all in slot order
+  const double* snap_sc;   // [SNAPSC_COUNT][ncol_pad]
+  const double* snap_arr;  // [SNAPARR_COUNT][LS][ncol_pad]
+  const int* in;
+  const int64_t* end_of_col;
+  const int* map;          // slot_of_col, nullptr = identity
+  long long ncol_pad;
+  int LS;
+  long long i;             // loop index of the record
+  // padded member layout (GsLayout)
+  const int* col;
+  const int* info;
+  long long npad;
+  const double* z;
+  int nz, nprof, Q;
+  int prof[SAMSIM_SNAPARR_COUNT];  // selected snapshot arrays, ascending
+  double* vals;            // [Q][npad]
+  double* reach;           // [npad]: -inf = not contributing, else D_{N_active} of the member's snapshot
+  double *pS, *pN, *pMn, *pMx;  // [Q][npad / SAMSIM_GS_TILE] chunk sums of groups larger than a tile
+  const int* big_group;    // groups larger than a tile
+  double* out;             // this record: [ngroup][Q][5] = count, mean, variance, min, max
+};
+
+// one thread per padded entry: the member's quantities in [q][entry] order (coalesced writes)
+__global__ void samsim_gs_gather_kernel(const GsParams p) {
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= p.npad) return;
+  const int c = p.col[t];
+  double reach = -INFINITY;
+  if (c >= 0) {
+    const long long s = slot_of(p.map, c);
+    const size_t ls = (size_t)p.ncol_pad;
+    // failed and finished columns hold stale snapshots
+    if (p.in[(size_t)IN_STATUS * ls + s] == 0 && (!p.end_of_col || p.end_of_col[s] >= p.i)) {
+      const size_t np = (size_t)p.npad;
+      for (int q = 0; q < SAMSIM_GS_NSC; q++) p.vals[q * np + t] = p.snap_sc[q * ls + s];
+      reach = 0.0;
+      if (p.nprof > 0) {
+        const double* A = p.snap_arr;
+        const int LS = p.LS;
+        const int na = (int)p.snap_sc[(size_t)SAMSIM_SNAPSC_N_ACTIVE * ls + s];
+        auto thick = [&](int k) { return A[((size_t)SAMSIM_SNAPARR_THICK * LS + k) * ls + s]; };
+        reach = gs_regrid(thick, na, p.z, p.nz, [&](int j, int k) {
+          for (int a = 0; a < p.nprof; a++)
+            p.vals[(size_t)(SAMSIM_GS_NSC + a * p.nz + j) * np + t] = A[((size_t)p.prof[a] * LS + k) * ls + s];
+        });
+      }
+    }
+  }
+  p.reach[t] = reach;
+}
+
+template <bool S_ONLY>
+__device__ __forceinline__ GsAcc gs_shfl(const GsAcc& a, int o) {
+  const unsigned full = 0xffffffffu;
+  GsAcc b;
+  b.s = __shfl_xor_sync(full, a.s, o);
+  if (S_ONLY) return b;
+  b.n = __shfl_xor_sync(full, a.n, o);
+  b.mn = __shfl_xor_sync(full, a.mn, o);
+  b.mx = __shfl_xor_sync(full, a.mx, o);
+  return b;
+}
+template <bool S_ONLY>
+__device__ __forceinline__ GsAcc gs_add(const GsAcc& a, const GsAcc& b) {
+  if (S_ONLY) return GsAcc{a.s + b.s, a.n, a.mn, a.mx};
+  return gs_combine(a, b);
+}
+
+// Pairwise tree over aligned blocks of 2^lgw (<= SAMSIM_GS_TILE) threads: each thread holds one leaf and the lgw of
+// its block (uniform over the block).  emit(first thread of the block, g, result) is called once per block.  All
+// threads of the block of SAMSIM_GS_TILE must call it.
+template <bool S_ONLY, class Emit>
+__device__ __forceinline__ void gs_block_tree(GsAcc a, int lgw, int g, Emit emit) {
+  __shared__ double sh[4][32];
+  __shared__ int shl[32], shg[32];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  for (int o = 1; o < 32; o <<= 1) {
+    const GsAcc b = gs_shfl<S_ONLY>(a, o);
+    if (o < (1 << lgw)) a = gs_add<S_ONLY>(a, b);
+  }
+  if (lgw <= 5 && (lane & ((1 << lgw) - 1)) == 0) emit((int)threadIdx.x, g, a);
+  if (lane == 0) { sh[0][warp] = a.s; sh[1][warp] = a.n; sh[2][warp] = a.mn; sh[3][warp] = a.mx; shl[warp] = lgw; shg[warp] = g; }
+  __syncthreads();
+  if (warp == 0) {
+    GsAcc x{sh[0][lane], sh[1][lane], sh[2][lane], sh[3][lane]};
+    const int l2 = shl[lane] - 5;  // levels above the warp
+    for (int o = 1; o < 32; o <<= 1) {
+      const GsAcc b = gs_shfl<S_ONLY>(x, o);
+      if (l2 > 0 && o < (1 << l2)) x = gs_add<S_ONLY>(x, b);
+    }
+    if (l2 > 0 && (lane & ((1 << l2) - 1)) == 0) emit(lane * 32, shg[lane], x);
+  }
+  __syncthreads();
+}
+
+// One tile of SAMSIM_GS_TILE padded entries per block, every quantity.  Pass 1 (SECOND = false): count, sum, min,
+// max; pass 2: the sum of squared deviations from the mean of pass 1.  Groups inside the tile are finished here;
+// a group larger than the tile leaves its chunk sum in pS.. for samsim_gs_final_kernel.
+template <bool SECOND>
+__global__ void __launch_bounds__(SAMSIM_GS_TILE) samsim_gs_tile_kernel(const GsParams p) {
+  const long long tile = blockIdx.x, t = tile * SAMSIM_GS_TILE + threadIdx.x;
+  const long long ntile = p.npad / SAMSIM_GS_TILE;
+  const size_t np = (size_t)p.npad;
+  const int info = p.info[t];
+  const int g = (info < 0) ? -1 : (info >> 5);
+  const int lg = (info < 0) ? 0 : (info & 31);
+  const int lgw = (lg < 10) ? lg : 10;
+  const double reach = p.reach[t];
+  const int Q = p.Q;
+  for (int q = 0; q < Q; q++) {
+    const double v = p.vals[q * np + t];
+    const bool in = (q < SAMSIM_GS_NSC) ? (reach != -INFINITY) : (p.z[(q - SAMSIM_GS_NSC) % p.nz] <= reach);
+    GsAcc a;
+    if (!SECOND) {
+      a = in ? GsAcc{v, 1.0, v, v} : GsAcc{0.0, 0.0, nan(""), nan("")};
+    } else {
+      const double d = (in && g >= 0) ? v - p.out[((size_t)g * Q + q) * 5 + 1] : 0.0;
+      a = GsAcc{d * d, 0.0, 0.0, 0.0};
+    }
+    gs_block_tree<SECOND>(a, lgw, g, [&](int, int gg, const GsAcc& r) {
+      if (gg < 0) return;
+      if (lg > 10) {
+        const size_t k = (size_t)q * ntile + tile;
+        p.pS[k] = r.s;
+        if (!SECOND) { p.pN[k] = r.n; p.pMn[k] = r.mn; p.pMx[k] = r.mx; }
+        return;
+      }
+      double* o = p.out + ((size_t)gg * Q + q) * 5;
+      if (!SECOND) { o[0] = r.n; o[1] = gs_mean(r.n, r.s); o[3] = r.mn; o[4] = r.mx; }
+      else o[2] = gs_variance(o[0], r.s);
+    });
+  }
+}
+
+// Groups larger than a tile: the same tree over their chunk sums, one block per (group, quantity).  Chunk sums are
+// reduced in place, SAMSIM_GS_TILE at a time, until one is left.
+template <bool SECOND>
+__global__ void __launch_bounds__(SAMSIM_GS_TILE) samsim_gs_final_kernel(const GsParams p, const int* start_tile,
+                                                                         const int* lg_of) {
+  const int b = blockIdx.x, q = blockIdx.y, Q = p.Q;
+  const int g = p.big_group[b];
+  const long long ntile = p.npad / SAMSIM_GS_TILE;
+  const size_t base = (size_t)q * ntile + start_tile[b];
+  long long n = 1ll << (lg_of[b] - 10);
+  while (n > 1) {
+    const int lgw = (n >= SAMSIM_GS_TILE) ? 10 : gs_log2_ceil(n);
+    const long long w = 1ll << lgw;
+    for (long long c = 0; c < n / w; c++) {
+      const size_t k = base + c * w + threadIdx.x;
+      GsAcc a{0.0, 0.0, nan(""), nan("")};
+      if (threadIdx.x < w) {
+        a.s = p.pS[k];
+        if (!SECOND) { a.n = p.pN[k]; a.mn = p.pMn[k]; a.mx = p.pMx[k]; }
+      }
+      gs_block_tree<SECOND>(a, lgw, g, [&](int pos, int, const GsAcc& r) {
+        if (pos != 0) return;
+        p.pS[base + c] = r.s;
+        if (!SECOND) { p.pN[base + c] = r.n; p.pMn[base + c] = r.mn; p.pMx[base + c] = r.mx; }
+      });
+    }
+    n /= w;
+  }
+  if (threadIdx.x != 0) return;
+  double* o = p.out + ((size_t)g * Q + q) * 5;
+  if (!SECOND) { o[0] = p.pN[base]; o[1] = gs_mean(p.pN[base], p.pS[base]); o[3] = p.pMn[base]; o[4] = p.pMx[base]; }
+  else o[2] = gs_variance(o[0], p.pS[base]);
+}
+
 __global__ void samsim_count_failed_kernel(const int* in, long long ncol, long long ncol_pad, int* out) {
   const long long col = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (col < ncol && in[(size_t)IN_STATUS * ncol_pad + col] != 0) atomicAdd(out, 1);
@@ -473,6 +645,16 @@ struct samsim_b200_handle_s {
   bool div_pending = false;
   double rebin_auto_threshold = 0.0;              // 0 = off
   double last_idle_share = 0.0, last_class_split_share = 0.0;
+  // group statistics (samsim_b200_set_group_stats): off while gs_ngroup == 0
+  int gs_ngroup = 0, gs_Q = 0, gs_nz = 0, gs_nprof = 0, gs_max = 0, gs_held = 0;
+  int gs_prof[SAMSIM_SNAPARR_COUNT] = {0};
+  uint32_t gs_mask = 0;
+  long long gs_npad = 0;
+  int gs_nbig = 0;
+  int *gs_col = nullptr, *gs_info = nullptr, *gs_big = nullptr;  // gs_big: [3][nbig] group, first tile, log2 size
+  double *gs_z = nullptr, *gs_vals = nullptr, *gs_reach = nullptr, *gs_part = nullptr, *gs_hist = nullptr;
+  std::vector<double> gs_time;
+  std::vector<int64_t> gs_i;
 };
 
 // The step kernel reads its configuration from constant memory (samsim_dev_cfg, physics.cuh), one copy per device.
@@ -570,6 +752,53 @@ static int to_slot_order(samsim_handle_t h, T* rows, int nrows) {
   return rc;
 }
 
+static void gs_free(samsim_handle_t h) {
+  cudaFree(h->gs_col); cudaFree(h->gs_info); cudaFree(h->gs_big); cudaFree(h->gs_z); cudaFree(h->gs_vals);
+  cudaFree(h->gs_reach); cudaFree(h->gs_part); cudaFree(h->gs_hist);
+  h->gs_col = h->gs_info = h->gs_big = nullptr;
+  h->gs_z = h->gs_vals = h->gs_reach = h->gs_part = h->gs_hist = nullptr;
+  h->gs_ngroup = h->gs_Q = h->gs_nz = h->gs_nprof = h->gs_max = h->gs_held = h->gs_nbig = 0;
+  h->gs_mask = 0;
+  h->gs_npad = 0;
+  h->gs_time.clear();
+  h->gs_i.clear();
+}
+
+// Queue the statistics of the record just written by the last step kernel (loop index h->i, model time `time`) into
+// history slot gs_held.  Five kernels on the handle's stream, no host synchronisation.
+static int gs_record(samsim_handle_t h, double time) {
+  GsParams p;
+  memset(&p, 0, sizeof p);
+  p.snap_sc = h->snap_sc; p.snap_arr = h->snap_arr; p.in = h->in; p.end_of_col = h->end_of_col; p.map = h->slot_of_col;
+  p.ncol_pad = h->ncol_pad; p.LS = h->LS; p.i = h->i;
+  p.col = h->gs_col; p.info = h->gs_info; p.npad = h->gs_npad;
+  p.z = h->gs_z; p.nz = h->gs_nz; p.nprof = h->gs_nprof; p.Q = h->gs_Q;
+  for (int a = 0; a < h->gs_nprof; a++) p.prof[a] = h->gs_prof[a];
+  p.vals = h->gs_vals; p.reach = h->gs_reach;
+  const size_t npart = (size_t)h->gs_Q * (h->gs_npad / SAMSIM_GS_TILE);
+  p.pS = h->gs_part; p.pN = p.pS + npart; p.pMn = p.pN + npart; p.pMx = p.pMn + npart;
+  p.big_group = h->gs_big;
+  p.out = h->gs_hist + (size_t)h->gs_held * h->gs_ngroup * h->gs_Q * 5;
+  const unsigned ntile = (unsigned)(h->gs_npad / SAMSIM_GS_TILE);
+  samsim_gs_gather_kernel<<<(unsigned)((h->gs_npad + 255) / 256), 256, 0, h->stream>>>(p);
+  const dim3 big((unsigned)h->gs_nbig, (unsigned)h->gs_Q);
+  samsim_gs_tile_kernel<false><<<ntile, SAMSIM_GS_TILE, 0, h->stream>>>(p);
+  if (h->gs_nbig) samsim_gs_final_kernel<false><<<big, SAMSIM_GS_TILE, 0, h->stream>>>(p, h->gs_big + h->gs_nbig, h->gs_big + 2 * h->gs_nbig);
+  samsim_gs_tile_kernel<true><<<ntile, SAMSIM_GS_TILE, 0, h->stream>>>(p);
+  if (h->gs_nbig) samsim_gs_final_kernel<true><<<big, SAMSIM_GS_TILE, 0, h->stream>>>(p, h->gs_big + h->gs_nbig, h->gs_big + 2 * h->gs_nbig);
+  CU(cudaGetLastError());
+  h->gs_time[(size_t)h->gs_held] = time;
+  h->gs_i[(size_t)h->gs_held] = h->i;
+  h->gs_held++;
+  return 0;
+}
+
+// records that `nsteps` steps from the current clock write (output steps: i == 1 and every i_time_out+1 steps)
+static int64_t records_in(samsim_handle_t h, int64_t nsteps) {
+  const int64_t first = (h->i == 0) ? 1 : (int64_t)(h->cfg.i_time_out - h->n_time_out) + 1;
+  return (nsteps < first) ? 0 : 1 + (nsteps - first) / ((int64_t)h->cfg.i_time_out + 1);
+}
+
 extern "C" {
 
 const char* samsim_b200_last_error(void) { return g_err.c_str(); }
@@ -662,6 +891,7 @@ void samsim_b200_destroy(samsim_handle_t h) {
   cudaFree(h->arr); cudaFree(h->sc); cudaFree(h->in); cudaFree(h->series); cudaFree(h->site_of_col);
   cudaFree(h->fscale); cudaFree(h->foffset); cudaFree(h->lab); cudaFree(h->set_of_col); cudaFree(h->snap_sc);
   cudaFree(h->snap_arr); cudaFree(h->stage); cudaFree(h->slot_of_col); cudaFree(h->col_of_slot); cudaFree(h->end_of_col);
+  gs_free(h);
   if (h->ev0) cudaEventDestroy(h->ev0);
   if (h->ev1) cudaEventDestroy(h->ev1);
   if (h->stream) cudaStreamDestroy(h->stream);
@@ -917,12 +1147,14 @@ int samsim_b200_set_end_step(samsim_handle_t h, const int64_t* end_i, int32_t co
 }
 
 // advance the host copy of the clock by one step exactly like the device does
-static inline void clock_tick(samsim_handle_t h) {
+// (true: the step wrote an output record)
+static inline bool clock_tick(samsim_handle_t h) {
   h->i += 1;
   const bool out = (h->n_time_out == h->cfg.i_time_out || h->i == 1);
   if (h->cfg.atmoflux_flag == 2 && h->time > host_time_input(h->time_counter)) h->time_counter += 1;
   h->n_time_out = out ? 0 : h->n_time_out + 1;
   h->time = h->time + h->cfg.dt;
+  return out;
 }
 
 // Divergence of the last launch (measured in the kernel with warp reductions / ballots): fold the counters into the
@@ -972,6 +1204,9 @@ int samsim_b200_step(samsim_handle_t h, int64_t nsteps) {
                         (h->cfg.boundflux_flag == 3 && h->cfg.lab_snow_flag == 1);  // 111: T_top = Ttop_input(FLOOR(1 + time/dt))
   if (need_forcing && !h->series) return fail(SAMSIM_ERR_STATE, "step: atmoflux_flag 2 needs samsim_b200_set_forcing first");
   if (need_lab && !h->lab) return fail(SAMSIM_ERR_STATE, "step: lab testcases need samsim_b200_set_lab_forcing first");
+  if (h->gs_ngroup > 0 && (int64_t)h->gs_held + records_in(h, nsteps) > h->gs_max)
+    return fail(SAMSIM_ERR_STATE, "step: the call writes more output records than the group statistics history can hold "
+                                  "(samsim_b200_get_group_stats / _clear_group_stats, or a larger max_records)");
   CU(cudaSetDevice(h->device));
   {
     int rc = collect_divergence(h, /*may_rebin=*/true);  // the previous call's measurement decides about re-binning now
@@ -990,6 +1225,8 @@ int samsim_b200_step(samsim_handle_t h, int64_t nsteps) {
     int64_t chunk = left;
     if (chunk > 1000000) chunk = 1000000;
     if (h->rebin_every > 0 && chunk > h->rebin_every - h->since_rebin) chunk = h->rebin_every - h->since_rebin;
+    // group statistics read the snapshot, status and end steps of each record: no launch runs past an output step
+    if (h->gs_ngroup > 0 && chunk > samsim_b200_steps_to_next_output(h)) chunk = samsim_b200_steps_to_next_output(h);
     if (need_forcing) {
       // simulate the clock to find the records the launch touches
       const int tc0 = h->time_counter;
@@ -1062,7 +1299,16 @@ int samsim_b200_step(samsim_handle_t h, int64_t nsteps) {
     CU(cudaGetLastError());
     CU(cudaEventRecord(h->ev_launch, h->stream));
     h->launches++;
-    for (int64_t s = 0; s < chunk; s++) clock_tick(h);
+    bool out = false;
+    double out_time = 0.0;
+    for (int64_t s = 0; s < chunk; s++) {
+      out_time = h->time;
+      out = clock_tick(h);
+    }
+    if (out && h->gs_ngroup > 0) {
+      int rc = gs_record(h, out_time);
+      if (rc) return rc;
+    }
     left -= chunk;
     if (h->rebin_every > 0 && (h->since_rebin += chunk) >= h->rebin_every) {
       h->since_rebin = 0;
@@ -1292,6 +1538,8 @@ int samsim_b200_synchronize(samsim_handle_t h) {
 
 int samsim_b200_set_snapshot_mode(samsim_handle_t h, int32_t mode) {
   if (!h || mode < 0 || mode > 2) return fail(SAMSIM_ERR_ARG, "set_snapshot_mode: bad argument");
+  if (h->gs_ngroup > 0 && mode < (h->gs_mask ? SAMSIM_SNAP_FULL : SAMSIM_SNAP_SCALARS))
+    return fail(SAMSIM_ERR_STATE, "set_snapshot_mode: the group statistics read this snapshot (switch them off first)");
   CU(cudaSetDevice(h->device));
   if (mode >= SAMSIM_SNAP_SCALARS && !h->snap_sc) {
     CU(cudaMalloc(&h->snap_sc, (size_t)SAMSIM_SNAPSC_COUNT * h->ncol_pad * sizeof(double)));
@@ -1333,6 +1581,103 @@ int samsim_b200_get_snapshot(samsim_handle_t h, double* scalars, double* arrays,
     CU(cudaMemcpyAsync(arrays, h->stage, bytes, cudaMemcpyDeviceToHost, h->stream));
     CU(cudaStreamSynchronize(h->stream));
   }
+  return 0;
+}
+
+int samsim_b200_set_group_stats(samsim_handle_t h, int32_t ngroup, const int32_t* group_of_col, int32_t nz,
+                                const double* depth, uint32_t profile_mask, int32_t max_records) {
+  if (!h) return fail(SAMSIM_ERR_ARG, "null handle");
+  if (ngroup == 0) {  // off
+    CU(cudaSetDevice(h->device));
+    CU(cudaStreamSynchronize(h->stream));
+    gs_free(h);
+    return 0;
+  }
+  // every argument is checked before the previous setting is dropped
+  if (ngroup < 0 || ngroup >= (1 << 26)) return fail(SAMSIM_ERR_ARG, "set_group_stats: ngroup must be in 0 .. 2^26-1");
+  if (max_records < 1) return fail(SAMSIM_ERR_ARG, "set_group_stats: max_records must be >= 1");
+  if (group_of_col)
+    for (long long c = 0; c < h->ncol; c++)
+      if (group_of_col[c] < -1 || group_of_col[c] >= ngroup) return fail(SAMSIM_ERR_ARG, "set_group_stats: group index out of [-1, ngroup)");
+  if (nz < 0 || (nz > 0 && !depth)) return fail(SAMSIM_ERR_ARG, "set_group_stats: bad depth grid");
+  for (int32_t j = 0; j < nz; j++)
+    if (!isfinite(depth[j]) || !(depth[j] > 0.0) || (j > 0 && !(depth[j] > depth[j - 1])))
+      return fail(SAMSIM_ERR_ARG, "set_group_stats: depths must be finite, > 0 and strictly increasing");
+  if (profile_mask >> SAMSIM_SNAPARR_COUNT) return fail(SAMSIM_ERR_ARG, "set_group_stats: unknown snapshot array in profile_mask");
+  if (profile_mask & (1u << SAMSIM_SNAPARR_RAY))
+    return fail(SAMSIM_ERR_ARG, "set_group_stats: ray is an interface quantity (extent Nlayer-1), not a layer profile");
+  for (int a = SAMSIM_SNAPARR_BGC1_BU; a < SAMSIM_SNAPARR_COUNT; a++)
+    if ((profile_mask >> a & 1u) && (a - SAMSIM_SNAPARR_BGC1_BU) / 2 >= h->cfg.N_bgc)
+      return fail(SAMSIM_ERR_ARG, "set_group_stats: tracer rows need N_bgc tracers");
+  if (profile_mask && nz == 0) return fail(SAMSIM_ERR_ARG, "set_group_stats: profiles need a depth grid (nz > 0)");
+  if (h->snap_mode < (profile_mask ? SAMSIM_SNAP_FULL : SAMSIM_SNAP_SCALARS))
+    return fail(SAMSIM_ERR_STATE, "set_group_stats: needs snapshot mode SCALARS, or FULL for profiles");
+  int nprof = 0;
+  int prof[SAMSIM_SNAPARR_COUNT];
+  for (int a = 0; a < SAMSIM_SNAPARR_COUNT; a++)
+    if (profile_mask >> a & 1u) prof[nprof++] = a;
+  const int Q = SAMSIM_GS_NSC + nprof * nz;
+  const GsLayout L = gs_layout(h->ncol, ngroup, group_of_col);
+  std::vector<int32_t> big;  // [3][nbig]: group, first tile, log2 size
+  for (int32_t g = 0; g < ngroup; g++)
+    if (L.lg[(size_t)g] > 10) big.push_back(g);
+  const int nbig = (int)big.size();
+  big.resize(3 * (size_t)nbig);
+  for (int b = 0; b < nbig; b++) {
+    big[(size_t)nbig + b] = (int32_t)(L.start[(size_t)big[b]] / SAMSIM_GS_TILE);
+    big[2 * (size_t)nbig + b] = L.lg[(size_t)big[b]];
+  }
+
+  CU(cudaSetDevice(h->device));
+  CU(cudaStreamSynchronize(h->stream));
+  gs_free(h);
+  const size_t np = (size_t)L.npad, npart = (size_t)Q * (np / SAMSIM_GS_TILE);
+  const size_t nhist = (size_t)max_records * ngroup * Q * 5;
+  cudaError_t e;
+  if ((e = cudaMalloc(&h->gs_col, np * sizeof(int))) != cudaSuccess || (e = cudaMalloc(&h->gs_info, np * sizeof(int))) != cudaSuccess ||
+      (e = cudaMalloc(&h->gs_big, (big.size() + 1) * sizeof(int))) != cudaSuccess ||
+      (e = cudaMalloc(&h->gs_z, ((size_t)nz + 1) * sizeof(double))) != cudaSuccess ||
+      (e = cudaMalloc(&h->gs_vals, (size_t)Q * np * sizeof(double))) != cudaSuccess ||
+      (e = cudaMalloc(&h->gs_reach, np * sizeof(double))) != cudaSuccess ||
+      (e = cudaMalloc(&h->gs_part, 4 * npart * sizeof(double))) != cudaSuccess ||
+      (e = cudaMalloc(&h->gs_hist, nhist * sizeof(double))) != cudaSuccess ||
+      (e = cudaMemcpy(h->gs_col, L.col.data(), np * sizeof(int), cudaMemcpyHostToDevice)) != cudaSuccess ||
+      (e = cudaMemcpy(h->gs_info, L.info.data(), np * sizeof(int), cudaMemcpyHostToDevice)) != cudaSuccess ||
+      (nbig && (e = cudaMemcpy(h->gs_big, big.data(), big.size() * sizeof(int), cudaMemcpyHostToDevice)) != cudaSuccess) ||
+      (nz && (e = cudaMemcpy(h->gs_z, depth, (size_t)nz * sizeof(double), cudaMemcpyHostToDevice)) != cudaSuccess)) {
+    gs_free(h);
+    cudaGetLastError();
+    return fail(SAMSIM_ERR_CUDA, std::string("set_group_stats: ") + cudaGetErrorString(e));
+  }
+  h->gs_ngroup = ngroup; h->gs_Q = Q; h->gs_nz = nz; h->gs_nprof = nprof; h->gs_max = max_records; h->gs_held = 0;
+  for (int a = 0; a < nprof; a++) h->gs_prof[a] = prof[a];
+  h->gs_mask = profile_mask; h->gs_npad = L.npad; h->gs_nbig = nbig;
+  h->gs_time.assign((size_t)max_records, 0.0);
+  h->gs_i.assign((size_t)max_records, 0);
+  return 0;
+}
+
+int32_t samsim_b200_group_stats_held(samsim_handle_t h) { return h ? h->gs_held : -1; }
+
+int samsim_b200_get_group_stats(samsim_handle_t h, double* stats, double* rec_time, int64_t* rec_i, int32_t rec0, int32_t nrec) {
+  if (!h) return fail(SAMSIM_ERR_ARG, "null handle");
+  if (rec0 < 0 || nrec < 0 || (int64_t)rec0 + nrec > h->gs_held)
+    return fail(SAMSIM_ERR_ARG, "get_group_stats: records rec0 .. rec0+nrec-1 must be held");
+  if (nrec == 0) return 0;
+  if (rec_time) std::copy(h->gs_time.begin() + rec0, h->gs_time.begin() + rec0 + nrec, rec_time);
+  if (rec_i) std::copy(h->gs_i.begin() + rec0, h->gs_i.begin() + rec0 + nrec, rec_i);
+  if (stats) {
+    CU(cudaSetDevice(h->device));
+    const size_t per = (size_t)h->gs_ngroup * h->gs_Q * 5;
+    CU(cudaMemcpyAsync(stats, h->gs_hist + (size_t)rec0 * per, (size_t)nrec * per * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+  }
+  return 0;
+}
+
+int samsim_b200_clear_group_stats(samsim_handle_t h) {
+  if (!h) return fail(SAMSIM_ERR_ARG, "null handle");
+  h->gs_held = 0;
   return 0;
 }
 

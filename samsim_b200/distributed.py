@@ -2,7 +2,8 @@
 
 The only exchange SAMSIM-style ensembles need is the optional reduction / gather of diagnostics at output cadence
 (SURVEY section 8e): 18 numbers per rank (sum/min/max of ice thickness, bulk salinity, freeboard, snow depth,
-surface temperature, N_active) -> one all-reduce each for SUM / MIN / MAX over NCCL (gloo on CPU in the tests).
+surface temperature, N_active) -> one all-reduce each for SUM / MIN / MAX over NCCL (gloo on CPU in the tests), and
+the per-group statistics of the output records (reduce_group_stats) -> four all-reduces of [records, groups, quantities].
 """
 from __future__ import annotations
 
@@ -42,6 +43,41 @@ def reduce_ensemble(local: dict, ncol_local: int, group=None, device=None) -> di
         dist.all_reduce(mx, op=dist.ReduceOp.MAX, group=group)
     total = float(s[-1].item())
     return {n: {"mean": float(s[j].item()) / total, "min": float(mn[j].item()), "max": float(mx[j].item())} for j, n in enumerate(NAMES)} | {"columns": int(total)}
+
+
+def reduce_group_stats(local: dict, group=None, device=None) -> dict:
+    """Combine Engine.group_stats() of ranks whose shards share column groups (same groups, depths, profiles and
+    records on every rank; a group may be empty on some ranks).  All-reduces only: count and count*mean with SUM, then
+    M2_r + n_r*(mean_r - mean)^2 with SUM, min / max with MIN / MAX.  Returns the same dict for the whole ensemble."""
+    import torch
+    import torch.distributed as dist
+    multi = dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1
+    f64 = dict(dtype=torch.float64, device=device)
+    n = torch.as_tensor(np.asarray(local["count"]), **f64)
+    has = n > 0
+    mean_r = torch.where(has, torch.as_tensor(np.asarray(local["mean"]), **f64), 0.0)
+    sums = torch.stack([n, n * mean_r])
+    if multi:
+        dist.all_reduce(sums, op=dist.ReduceOp.SUM, group=group)
+    N = sums[0]
+    mean = sums[1] / N                                 # NaN where no rank has a contributor
+    var_r = torch.as_tensor(np.asarray(local["var"]), **f64)
+    m2 = torch.where(has, torch.where(n >= 2, var_r * (n - 1), 0.0) + n * (mean_r - mean) ** 2, 0.0)
+    if multi:
+        dist.all_reduce(m2, op=dist.ReduceOp.SUM, group=group)
+    var = torch.where(N >= 2, m2 / (N - 1), torch.where(N == 1, 0.0, float("nan")))
+    inf = float("inf")
+    mn = torch.as_tensor(np.asarray(local["min"]), **f64)
+    mx = torch.as_tensor(np.asarray(local["max"]), **f64)
+    mn, mx = torch.where(mn.isnan(), inf, mn), torch.where(mx.isnan(), -inf, mx)
+    if multi:
+        dist.all_reduce(mn, op=dist.ReduceOp.MIN, group=group)
+        dist.all_reduce(mx, op=dist.ReduceOp.MAX, group=group)
+    nan = torch.full_like(N, float("nan"))
+    out = {k: local[k] for k in ("time", "i", "quantities")}
+    out.update(count=N.cpu().numpy(), mean=mean.cpu().numpy(), var=var.cpu().numpy(),
+               min=torch.where(N > 0, mn, nan).cpu().numpy(), max=torch.where(N > 0, mx, nan).cpu().numpy())
+    return out
 
 
 def gather_columns(values, group=None, dst: int = 0):

@@ -226,6 +226,40 @@ MODULE mo_samsim_b200
        TYPE(C_PTR), VALUE :: handle
      END FUNCTION samsim_b200_clear_group_stats
 
+     !> per-column time statistics over windows of output records (both masks 0: off); depth: C_LOC of the array or
+     !> C_NULL_PTR; scalar_mask: bits of samsim_snapshot_scalar_id, profile_mask: bits of samsim_snapshot_array_id
+     !> (uint32_t in C, masks < 2**20)
+     INTEGER(C_INT) FUNCTION samsim_b200_set_time_stats(handle, records_per_window, scalar_mask, nz, depth, &
+          & profile_mask, max_windows) BIND(C, NAME='samsim_b200_set_time_stats')
+       IMPORT :: C_INT, C_INT32_T, C_PTR
+       TYPE(C_PTR), VALUE :: handle, depth
+       INTEGER(C_INT32_T), VALUE :: records_per_window, scalar_mask, nz, profile_mask, max_windows
+     END FUNCTION samsim_b200_set_time_stats
+
+     INTEGER(C_INT32_T) FUNCTION samsim_b200_time_stats_held(handle) BIND(C, NAME='samsim_b200_time_stats_held')
+       IMPORT :: C_INT32_T, C_PTR
+       TYPE(C_PTR), VALUE :: handle
+     END FUNCTION samsim_b200_time_stats_held
+
+     !> windows win0 .. win0+nwin-1 and columns col0 .. col0+n-1 (0-based): stats(5, Q, n, nwin), win_nrec(nwin),
+     !> win_time(2, nwin), win_i(2, nwin); C_NULL_PTR skips one
+     INTEGER(C_INT) FUNCTION samsim_b200_get_time_stats(handle, stats, win_nrec, win_time, win_i, win0, nwin, col0, n) &
+          & BIND(C, NAME='samsim_b200_get_time_stats')
+       IMPORT :: C_INT, C_INT32_T, C_PTR
+       TYPE(C_PTR), VALUE :: handle, stats, win_nrec, win_time, win_i
+       INTEGER(C_INT32_T), VALUE :: win0, nwin, col0, n
+     END FUNCTION samsim_b200_get_time_stats
+
+     INTEGER(C_INT) FUNCTION samsim_b200_close_time_window(handle) BIND(C, NAME='samsim_b200_close_time_window')
+       IMPORT :: C_INT, C_PTR
+       TYPE(C_PTR), VALUE :: handle
+     END FUNCTION samsim_b200_close_time_window
+
+     INTEGER(C_INT) FUNCTION samsim_b200_clear_time_stats(handle) BIND(C, NAME='samsim_b200_clear_time_stats')
+       IMPORT :: C_INT, C_PTR
+       TYPE(C_PTR), VALUE :: handle
+     END FUNCTION samsim_b200_clear_time_stats
+
      INTEGER(C_INT) FUNCTION samsim_b200_get_status(handle, status, col0, n) BIND(C, NAME='samsim_b200_get_status')
        IMPORT :: C_INT, C_INT32_T, C_PTR
        TYPE(C_PTR), VALUE :: handle

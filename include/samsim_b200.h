@@ -308,6 +308,46 @@ int samsim_b200_get_group_stats(samsim_handle_t h, double* stats, double* rec_ti
                                 int32_t nrec);
 int samsim_b200_clear_group_stats(samsim_handle_t h); /* drop the held records */
 
+/* ---- per-column time statistics over windows of S8 records ----------------------------------------
+ * Accumulated and kept on the device, so that one samsim_b200_step call may span any number of records and windows.
+ * Quantities q: the SAMSIM_SNAPSC_* scalars whose bits are set in scalar_mask (bits 0..19), in id order, then nz
+ * depths of each profile selected by profile_mask in samsim_snapshot_array_id order; Q = their number.  depth and
+ * profile_mask follow the rules of samsim_b200_set_group_stats (finite, > 0, strictly increasing; not RAY; tracer
+ * rows only with N_bgc tracers; non-zero needs nz > 0).  Q = 0 (both masks 0) switches them off (the default).  A bad
+ * argument is SAMSIM_ERR_ARG and keeps the previous setting; a snapshot mode below SCALARS (FULL with profiles) is
+ * SAMSIM_ERR_STATE.  A new setting drops the held windows and the window in progress.  Device memory:
+ * (1 + max_windows) * 5 * Q * ncol_pad doubles; a failed allocation is SAMSIM_ERR_CUDA and leaves them off.
+ *
+ * Windows: a window collects records_per_window (>= 0) consecutive records, counted from the set call or the last
+ * close; its last record finalises it into history slot `held` and a new window starts.  records_per_window = 0: a
+ * window closes only through samsim_b200_close_time_window (calendar windows such as months).  Closing an empty
+ * window, or closing with a full history, is SAMSIM_ERR_STATE.
+ *
+ * Output for windows win0..win0+nwin-1 and caller columns col0..col0+n-1: stats[((w*n + c)*Q + q)*5 + s], s = count,
+ * mean, variance, min, max; win_nrec[w] = records in window w; win_time[2w], [2w+1] = SAMSIM_SNAPSC_TIME and win_i[2w],
+ * [2w+1] = loop index of its first and last record; any output pointer may be NULL.
+ *
+ * Bitwise contract.  A column contributes the record of step i when its status is 0 at the end of step i and its end
+ * step is >= i.  Profile p at depth z takes the layer of samsim_b200_set_group_stats' regrid; depths below D_{N_active}
+ * do not contribute, so every quantity has its own count.  Records are accumulated in record order, starting from
+ * n = 0, mean = 0, M2 = 0, min = max = NaN, with exactly
+ *     n = n + 1;  d = x - mean;  mean = mean + d / n;  M2 = M2 + d * (x - mean);  min = fmin(min, x);  max = fmax(max, x)
+ * (no contraction; of two equal values, +0.0 and -0.0, fmin / fmax keep min / max).  Finalising: mean NaN for count 0;
+ * variance = M2 / (n - 1), 0 for n = 1, NaN for n = 0; min and max NaN for count 0.  Results do not depend on
+ * re-binning, launch lengths, block size, the two-pass step or whether group statistics are on.
+ *
+ * samsim_b200_step with time statistics on: no launch runs past an output step, and after each launch that ends on one
+ * the time-statistics kernel is queued on the handle's stream (no host synchronisation).  A call that would complete
+ * more windows than max_windows - held returns SAMSIM_ERR_STATE before anything runs.  Time statistics are run outputs:
+ * not saved in checkpoints; samsim_b200_load_checkpoint and samsim_b200_set_clock leave the accumulators alone. */
+int samsim_b200_set_time_stats(samsim_handle_t h, int32_t records_per_window, uint32_t scalar_mask, int32_t nz,
+                               const double* depth, uint32_t profile_mask, int32_t max_windows);
+int32_t samsim_b200_time_stats_held(samsim_handle_t h); /* completed windows held, -1 for a null handle */
+int samsim_b200_get_time_stats(samsim_handle_t h, double* stats, int32_t* win_nrec, double* win_time, int64_t* win_i,
+                               int32_t win0, int32_t nwin, int32_t col0, int32_t n);
+int samsim_b200_close_time_window(samsim_handle_t h); /* close the window in progress now */
+int samsim_b200_clear_time_stats(samsim_handle_t h);  /* drop the held windows */
+
 /* ---- diagnostics -------------------------------------------------------------------------- */
 int samsim_b200_get_status(samsim_handle_t h, int32_t* status, int32_t col0, int32_t n);
 /* number of columns with non-zero status */

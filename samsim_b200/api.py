@@ -178,6 +178,12 @@ def load_library() -> C.CDLL:
         "samsim_b200_group_stats_held": (C.c_int32, [H]),
         "samsim_b200_get_group_stats": (C.c_int, [H, dp, dp, C.POINTER(C.c_int64), C.c_int32, C.c_int32]),
         "samsim_b200_clear_group_stats": (C.c_int, [H]),
+        "samsim_b200_set_time_stats": (C.c_int, [H, C.c_int32, C.c_uint32, C.c_int32, dp, C.c_uint32, C.c_int32]),
+        "samsim_b200_time_stats_held": (C.c_int32, [H]),
+        "samsim_b200_get_time_stats": (C.c_int, [H, dp, ip, dp, C.POINTER(C.c_int64), C.c_int32, C.c_int32, C.c_int32,
+                                                 C.c_int32]),
+        "samsim_b200_close_time_window": (C.c_int, [H]),
+        "samsim_b200_clear_time_stats": (C.c_int, [H]),
         "samsim_b200_get_status": (C.c_int, [H, ip, C.c_int32, C.c_int32]),
         "samsim_b200_count_failed": (C.c_int, [H, ip]),
         "samsim_b200_reduce_diag": (C.c_int, [H, dp]),
@@ -215,6 +221,8 @@ EXPORTED_SYMBOLS = [
     "samsim_b200_step", "samsim_b200_synchronize", "samsim_b200_steps_to_next_output",
     "samsim_b200_set_snapshot_mode", "samsim_b200_get_snapshot", "samsim_b200_set_group_stats",
     "samsim_b200_group_stats_held", "samsim_b200_get_group_stats", "samsim_b200_clear_group_stats",
+    "samsim_b200_set_time_stats", "samsim_b200_time_stats_held", "samsim_b200_get_time_stats",
+    "samsim_b200_close_time_window", "samsim_b200_clear_time_stats",
     "samsim_b200_get_status",
     "samsim_b200_count_failed", "samsim_b200_reduce_diag", "samsim_b200_launch_count", "samsim_b200_last_step_ms",
     "samsim_b200_device_layout", "samsim_b200_save_checkpoint", "samsim_b200_load_checkpoint", "samsim_b200_rebin", "samsim_b200_set_tuning", "samsim_b200_set_rebin_interval", "samsim_b200_set_rebin_auto", "samsim_b200_get_divergence", "samsim_b200_get_slot_map",
@@ -469,6 +477,57 @@ class Engine:
 
     def clear_group_stats(self):
         _check(self.L, self.L.samsim_b200_clear_group_stats(self.h))
+
+    # ---- time statistics over windows of S8 records -------------------------------------------
+    def set_time_stats(self, records_per_window: int, scalars=None, depths=(), profiles=(), max_windows: int = 64):
+        """Per-column count, mean, variance, min and max over windows of output records, accumulated on the device
+        (include/samsim_b200.h).  A window collects records_per_window records; 0 = windows end only at
+        close_time_window().  scalars: names of SNAP_SCALARS (None = all 20); depths: metres below the ice surface;
+        profiles: names of SNAP_ARRAYS.  No scalars and no profiles switch the statistics off.  Needs snapshot mode
+        SCALARS, FULL with profiles.  A new setting drops the held windows and the window in progress."""
+        sc = list(SNAP_SCALARS) if scalars is None else list(scalars)
+        scmask = 0
+        for name in sc:
+            scmask |= 1 << SNAP_SCALARS.index(name)
+        z = np.ascontiguousarray(depths, dtype=np.float64).reshape(-1)
+        mask = 0
+        for name in profiles:
+            mask |= 1 << SNAP_ARRAYS.index(name)
+        _check(self.L, self.L.samsim_b200_set_time_stats(self.h, int(records_per_window), scmask, len(z),
+                                                         _dp(z) if len(z) else None, mask, int(max_windows)))
+        qn = [(n, None) for j, n in enumerate(SNAP_SCALARS) if scmask >> j & 1]
+        qn += [(p, float(d)) for j, p in enumerate(SNAP_ARRAYS) if mask >> j & 1 for d in z]
+        self._ts = {"quantities": qn} if qn else None
+
+    def time_stats_held(self) -> int:
+        return int(self.L.samsim_b200_time_stats_held(self.h))
+
+    def time_stats(self, col0: int = 0, n: int | None = None, clear: bool = False) -> dict:
+        """The held windows for caller columns col0..col0+n-1: nrec, time_first, time_last, i_first, i_last of shape
+        [W]; quantities [(name, depth or None)]; count / mean / var / min / max of shape [W, n, Q].  clear=True drops
+        the held windows afterwards."""
+        t = getattr(self, "_ts", None)
+        assert t is not None, "time statistics are off"
+        n = self.ncol - col0 if n is None else n
+        W, qn = self.time_stats_held(), t["quantities"]
+        st = np.empty((W, n, len(qn), 5), dtype=np.float64)
+        nrec = np.empty(W, dtype=np.int32)
+        tm = np.empty((W, 2), dtype=np.float64)
+        i = np.empty((W, 2), dtype=np.int64)
+        _check(self.L, self.L.samsim_b200_get_time_stats(self.h, _dp(st), _ip(nrec), _dp(tm), _lp(i), 0, W, int(col0), int(n)))
+        if clear:
+            self.clear_time_stats()
+        out = {"nrec": nrec, "time_first": tm[:, 0], "time_last": tm[:, 1], "i_first": i[:, 0], "i_last": i[:, 1],
+               "quantities": qn}
+        for k, name in enumerate(("count", "mean", "var", "min", "max")):
+            out[name] = st[..., k]
+        return out
+
+    def close_time_window(self):
+        _check(self.L, self.L.samsim_b200_close_time_window(self.h))
+
+    def clear_time_stats(self):
+        _check(self.L, self.L.samsim_b200_clear_time_stats(self.h))
 
     # ---- diagnostics ------------------------------------------------------------------------
     def status(self) -> np.ndarray:

@@ -17,6 +17,7 @@
 #include "../../include/samsim_b200.h"
 #include "group_stats.cuh"
 #include "step.cuh"
+#include "time_stats.cuh"
 
 using namespace samsim;
 
@@ -522,6 +523,91 @@ __global__ void __launch_bounds__(SAMSIM_GS_TILE) samsim_gs_final_kernel(const G
   else o[2] = gs_variance(o[0], p.pS[base]);
 }
 
+// ---- time statistics over windows of S8 records (time_stats.cuh; samsim_b200_set_time_stats) --------------------
+struct TsParams {
+  // snapshot, status and end steps, all in slot order
+  const double* snap_sc;   // [SNAPSC_COUNT][ncol_pad]
+  const double* snap_arr;  // [SNAPARR_COUNT][LS][ncol_pad]
+  const int* in;
+  const int64_t* end_of_col;
+  const int* map;          // slot_of_col, nullptr = identity
+  long long ncol, ncol_pad;
+  int LS;
+  long long i;             // loop index of the record
+  const double* z;
+  int nz, nsc, nprof;
+  int sc[SAMSIM_SNAPSC_COUNT];     // selected snapshot scalars, ascending
+  int prof[SAMSIM_SNAPARR_COUNT];  // selected snapshot arrays, ascending
+  double* acc;             // window in progress: [Q][5][ncol_pad] = n, mean, M2, min, max in caller column order
+  double* out;             // history slot [Q][5][ncol_pad] when this record closes the window, else nullptr
+  bool first;              // the record opens a window: the accumulators are not read
+};
+
+// One record of quantity q for caller column c: the Welford update where the column contributes, and on the window's
+// closing record the finalised statistics into the history slot instead of the accumulators.
+__device__ __forceinline__ void ts_one(const TsParams& p, long long c, int q, bool contributes, double x) {
+  const size_t ls = (size_t)p.ncol_pad, base = (size_t)q * SAMSIM_TS_NSTAT * ls + c;
+  if (!contributes && !p.first && !p.out) return;  // nothing changes
+  TsAcc a = ts_init();
+  if (!p.first) a = TsAcc{p.acc[base], p.acc[base + ls], p.acc[base + 2 * ls], p.acc[base + 3 * ls], p.acc[base + 4 * ls]};
+  if (contributes) ts_update(a, x);
+  if (p.out) {
+    double r[SAMSIM_TS_NSTAT];
+    ts_finish(a, r);
+    for (int s = 0; s < SAMSIM_TS_NSTAT; s++) p.out[base + s * ls] = r[s];
+  } else {
+    p.acc[base] = a.n; p.acc[base + ls] = a.mean; p.acc[base + 2 * ls] = a.m2; p.acc[base + 3 * ls] = a.mn;
+    p.acc[base + 4 * ls] = a.mx;
+  }
+}
+
+// one thread per caller column: reads its snapshot through slot_of_col (re-binning permutes nothing here)
+__global__ void samsim_ts_record_kernel(const TsParams p) {
+  const long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= p.ncol) return;
+  const long long s = slot_of(p.map, c);
+  const size_t ls = (size_t)p.ncol_pad;
+  // failed and finished columns hold stale snapshots
+  const bool live = p.in[(size_t)IN_STATUS * ls + s] == 0 && (!p.end_of_col || p.end_of_col[s] >= p.i);
+  for (int q = 0; q < p.nsc; q++) ts_one(p, c, q, live, live ? p.snap_sc[(size_t)p.sc[q] * ls + s] : 0.0);
+  if (p.nprof == 0) return;
+  int reached = 0;  // depths above the column's ice bottom
+  if (live) {
+    const double* A = p.snap_arr;
+    const int LS = p.LS;
+    const int na = (int)p.snap_sc[(size_t)SAMSIM_SNAPSC_N_ACTIVE * ls + s];
+    auto thick = [&](int k) { return A[((size_t)SAMSIM_SNAPARR_THICK * LS + k) * ls + s]; };
+    gs_regrid(thick, na, p.z, p.nz, [&](int j, int k) {
+      for (int a = 0; a < p.nprof; a++) ts_one(p, c, p.nsc + a * p.nz + j, true, A[((size_t)p.prof[a] * LS + k) * ls + s]);
+      reached = j + 1;
+    });
+  }
+  for (int j = reached; j < p.nz; j++)
+    for (int a = 0; a < p.nprof; a++) ts_one(p, c, p.nsc + a * p.nz + j, false, 0.0);
+}
+
+// samsim_b200_close_time_window: finalise the window in progress into its history slot, one thread per column
+__global__ void samsim_ts_close_kernel(const double* acc, double* out, int Q, long long ncol, long long ncol_pad) {
+  const long long c = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= ncol) return;
+  const size_t ls = (size_t)ncol_pad;
+  for (int q = 0; q < Q; q++) {
+    const size_t base = (size_t)q * SAMSIM_TS_NSTAT * ls + c;
+    const TsAcc a{acc[base], acc[base + ls], acc[base + 2 * ls], acc[base + 3 * ls], acc[base + 4 * ls]};
+    double r[SAMSIM_TS_NSTAT];
+    ts_finish(a, r);
+    for (int s = 0; s < SAMSIM_TS_NSTAT; s++) out[base + s * ls] = r[s];
+  }
+}
+
+// samsim_b200_get_time_stats: one window's [Q][5][ncol_pad] history -> dst[(cc*Q + q)*5 + s] for columns col0..col0+n-1
+__global__ void samsim_ts_get_kernel(const double* win, double* dst, long long ncol_pad, int Q, long long col0, long long n) {
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n * Q * SAMSIM_TS_NSTAT) return;
+  const long long cc = t / ((long long)Q * SAMSIM_TS_NSTAT), qs = t % ((long long)Q * SAMSIM_TS_NSTAT);
+  dst[t] = win[(size_t)qs * ncol_pad + col0 + cc];
+}
+
 __global__ void samsim_count_failed_kernel(const int* in, long long ncol, long long ncol_pad, int* out) {
   const long long col = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (col < ncol && in[(size_t)IN_STATUS * ncol_pad + col] != 0) atomicAdd(out, 1);
@@ -655,6 +741,17 @@ struct samsim_b200_handle_s {
   double *gs_z = nullptr, *gs_vals = nullptr, *gs_reach = nullptr, *gs_part = nullptr, *gs_hist = nullptr;
   std::vector<double> gs_time;
   std::vector<int64_t> gs_i;
+  // time statistics (samsim_b200_set_time_stats): off while ts_Q == 0
+  int ts_Q = 0, ts_nsc = 0, ts_nz = 0, ts_nprof = 0, ts_rpw = 0, ts_max = 0, ts_held = 0;
+  int ts_cur = 0;  // records in the window in progress
+  int ts_sc[SAMSIM_SNAPSC_COUNT] = {0}, ts_prof[SAMSIM_SNAPARR_COUNT] = {0};
+  uint32_t ts_mask = 0;  // profile_mask
+  double *ts_z = nullptr, *ts_acc = nullptr, *ts_hist = nullptr;
+  std::vector<int32_t> ts_nrec;  // [max_windows]
+  // [max_windows + 1][2]: time and loop index of the first and last record of each held window, and of the window in
+  // progress in row max_windows
+  std::vector<double> ts_time;
+  std::vector<int64_t> ts_i;
 };
 
 // The step kernel reads its configuration from constant memory (samsim_dev_cfg, physics.cuh), one copy per device.
@@ -795,8 +892,54 @@ static int gs_record(samsim_handle_t h, double time) {
 
 // records that `nsteps` steps from the current clock write (output steps: i == 1 and every i_time_out+1 steps)
 static int64_t records_in(samsim_handle_t h, int64_t nsteps) {
-  const int64_t first = (h->i == 0) ? 1 : (int64_t)(h->cfg.i_time_out - h->n_time_out) + 1;
-  return (nsteps < first) ? 0 : 1 + (nsteps - first) / ((int64_t)h->cfg.i_time_out + 1);
+  return ts_records_in(h->i, h->n_time_out, h->cfg.i_time_out, nsteps);
+}
+
+static void ts_free(samsim_handle_t h) {
+  cudaFree(h->ts_z); cudaFree(h->ts_acc); cudaFree(h->ts_hist);
+  h->ts_z = h->ts_acc = h->ts_hist = nullptr;
+  h->ts_Q = h->ts_nsc = h->ts_nz = h->ts_nprof = h->ts_rpw = h->ts_max = h->ts_held = h->ts_cur = 0;
+  h->ts_mask = 0;
+  h->ts_nrec.clear();
+  h->ts_time.clear();
+  h->ts_i.clear();
+}
+
+// the window in progress becomes history slot ts_held (its statistics were written there by the kernels)
+static void ts_window_done(samsim_handle_t h) {
+  const size_t w = (size_t)h->ts_held, cur = (size_t)h->ts_max;
+  h->ts_nrec[w] = h->ts_cur;
+  for (int k = 0; k < 2; k++) {
+    h->ts_time[2 * w + k] = h->ts_time[2 * cur + k];
+    h->ts_i[2 * w + k] = h->ts_i[2 * cur + k];
+  }
+  h->ts_held++;
+  h->ts_cur = 0;
+}
+
+// Queue the record just written by the last step kernel (loop index h->i, model time `time`) into the window in
+// progress; on its closing record the same kernel writes history slot ts_held.  No host synchronisation.
+static int ts_record(samsim_handle_t h, double time) {
+  TsParams p;
+  memset(&p, 0, sizeof p);
+  p.snap_sc = h->snap_sc; p.snap_arr = h->snap_arr; p.in = h->in; p.end_of_col = h->end_of_col; p.map = h->slot_of_col;
+  p.ncol = h->ncol; p.ncol_pad = h->ncol_pad; p.LS = h->LS; p.i = h->i;
+  p.z = h->ts_z; p.nz = h->ts_nz; p.nsc = h->ts_nsc; p.nprof = h->ts_nprof;
+  for (int q = 0; q < h->ts_nsc; q++) p.sc[q] = h->ts_sc[q];
+  for (int a = 0; a < h->ts_nprof; a++) p.prof[a] = h->ts_prof[a];
+  p.acc = h->ts_acc;
+  p.first = (h->ts_cur == 0);
+  const bool closes = h->ts_rpw > 0 && h->ts_cur + 1 == h->ts_rpw;
+  p.out = closes ? h->ts_hist + (size_t)h->ts_held * h->ts_Q * SAMSIM_TS_NSTAT * h->ncol_pad : nullptr;
+  samsim_ts_record_kernel<<<(unsigned)((h->ncol + 255) / 256), 256, 0, h->stream>>>(p);
+  CU(cudaGetLastError());
+  const size_t cur = (size_t)h->ts_max;
+  if (p.first) { h->ts_time[2 * cur] = time; h->ts_i[2 * cur] = h->i; }
+  h->ts_time[2 * cur + 1] = time;
+  h->ts_i[2 * cur + 1] = h->i;
+  h->ts_cur++;
+  if (closes) ts_window_done(h);
+  return 0;
 }
 
 extern "C" {
@@ -892,6 +1035,7 @@ void samsim_b200_destroy(samsim_handle_t h) {
   cudaFree(h->fscale); cudaFree(h->foffset); cudaFree(h->lab); cudaFree(h->set_of_col); cudaFree(h->snap_sc);
   cudaFree(h->snap_arr); cudaFree(h->stage); cudaFree(h->slot_of_col); cudaFree(h->col_of_slot); cudaFree(h->end_of_col);
   gs_free(h);
+  ts_free(h);
   if (h->ev0) cudaEventDestroy(h->ev0);
   if (h->ev1) cudaEventDestroy(h->ev1);
   if (h->stream) cudaStreamDestroy(h->stream);
@@ -1207,6 +1351,9 @@ int samsim_b200_step(samsim_handle_t h, int64_t nsteps) {
   if (h->gs_ngroup > 0 && (int64_t)h->gs_held + records_in(h, nsteps) > h->gs_max)
     return fail(SAMSIM_ERR_STATE, "step: the call writes more output records than the group statistics history can hold "
                                   "(samsim_b200_get_group_stats / _clear_group_stats, or a larger max_records)");
+  if (h->ts_Q > 0 && ts_windows_completed(h->ts_rpw, h->ts_cur, records_in(h, nsteps)) > (int64_t)h->ts_max - h->ts_held)
+    return fail(SAMSIM_ERR_STATE, "step: the call completes more windows than the time statistics history can hold "
+                                  "(samsim_b200_get_time_stats / _clear_time_stats, or a larger max_windows)");
   CU(cudaSetDevice(h->device));
   {
     int rc = collect_divergence(h, /*may_rebin=*/true);  // the previous call's measurement decides about re-binning now
@@ -1225,8 +1372,10 @@ int samsim_b200_step(samsim_handle_t h, int64_t nsteps) {
     int64_t chunk = left;
     if (chunk > 1000000) chunk = 1000000;
     if (h->rebin_every > 0 && chunk > h->rebin_every - h->since_rebin) chunk = h->rebin_every - h->since_rebin;
-    // group statistics read the snapshot, status and end steps of each record: no launch runs past an output step
-    if (h->gs_ngroup > 0 && chunk > samsim_b200_steps_to_next_output(h)) chunk = samsim_b200_steps_to_next_output(h);
+    // group and time statistics read the snapshot, status and end steps of each record: no launch runs past an
+    // output step
+    if ((h->gs_ngroup > 0 || h->ts_Q > 0) && chunk > samsim_b200_steps_to_next_output(h))
+      chunk = samsim_b200_steps_to_next_output(h);
     if (need_forcing) {
       // simulate the clock to find the records the launch touches
       const int tc0 = h->time_counter;
@@ -1307,6 +1456,10 @@ int samsim_b200_step(samsim_handle_t h, int64_t nsteps) {
     }
     if (out && h->gs_ngroup > 0) {
       int rc = gs_record(h, out_time);
+      if (rc) return rc;
+    }
+    if (out && h->ts_Q > 0) {
+      int rc = ts_record(h, out_time);
       if (rc) return rc;
     }
     left -= chunk;
@@ -1540,6 +1693,8 @@ int samsim_b200_set_snapshot_mode(samsim_handle_t h, int32_t mode) {
   if (!h || mode < 0 || mode > 2) return fail(SAMSIM_ERR_ARG, "set_snapshot_mode: bad argument");
   if (h->gs_ngroup > 0 && mode < (h->gs_mask ? SAMSIM_SNAP_FULL : SAMSIM_SNAP_SCALARS))
     return fail(SAMSIM_ERR_STATE, "set_snapshot_mode: the group statistics read this snapshot (switch them off first)");
+  if (h->ts_Q > 0 && mode < (h->ts_mask ? SAMSIM_SNAP_FULL : SAMSIM_SNAP_SCALARS))
+    return fail(SAMSIM_ERR_STATE, "set_snapshot_mode: the time statistics read this snapshot (switch them off first)");
   CU(cudaSetDevice(h->device));
   if (mode >= SAMSIM_SNAP_SCALARS && !h->snap_sc) {
     CU(cudaMalloc(&h->snap_sc, (size_t)SAMSIM_SNAPSC_COUNT * h->ncol_pad * sizeof(double)));
@@ -1584,6 +1739,26 @@ int samsim_b200_get_snapshot(samsim_handle_t h, double* scalars, double* arrays,
   return 0;
 }
 
+// The depth grid and profiles of the group and time statistics, and the snapshot they need (SAMSIM_ERR_ARG /
+// SAMSIM_ERR_STATE with the caller's name)
+static int check_depth_grid(samsim_handle_t h, int32_t nz, const double* depth, uint32_t profile_mask, const char* who) {
+  const std::string w = std::string(who) + ": ";
+  if (nz < 0 || (nz > 0 && !depth)) return fail(SAMSIM_ERR_ARG, w + "bad depth grid");
+  for (int32_t j = 0; j < nz; j++)
+    if (!isfinite(depth[j]) || !(depth[j] > 0.0) || (j > 0 && !(depth[j] > depth[j - 1])))
+      return fail(SAMSIM_ERR_ARG, w + "depths must be finite, > 0 and strictly increasing");
+  if (profile_mask >> SAMSIM_SNAPARR_COUNT) return fail(SAMSIM_ERR_ARG, w + "unknown snapshot array in profile_mask");
+  if (profile_mask & (1u << SAMSIM_SNAPARR_RAY))
+    return fail(SAMSIM_ERR_ARG, w + "ray is an interface quantity (extent Nlayer-1), not a layer profile");
+  for (int a = SAMSIM_SNAPARR_BGC1_BU; a < SAMSIM_SNAPARR_COUNT; a++)
+    if ((profile_mask >> a & 1u) && (a - SAMSIM_SNAPARR_BGC1_BU) / 2 >= h->cfg.N_bgc)
+      return fail(SAMSIM_ERR_ARG, w + "tracer rows need N_bgc tracers");
+  if (profile_mask && nz == 0) return fail(SAMSIM_ERR_ARG, w + "profiles need a depth grid (nz > 0)");
+  if (h->snap_mode < (profile_mask ? SAMSIM_SNAP_FULL : SAMSIM_SNAP_SCALARS))
+    return fail(SAMSIM_ERR_STATE, w + "needs snapshot mode SCALARS, or FULL for profiles");
+  return 0;
+}
+
 int samsim_b200_set_group_stats(samsim_handle_t h, int32_t ngroup, const int32_t* group_of_col, int32_t nz,
                                 const double* depth, uint32_t profile_mask, int32_t max_records) {
   if (!h) return fail(SAMSIM_ERR_ARG, "null handle");
@@ -1599,19 +1774,10 @@ int samsim_b200_set_group_stats(samsim_handle_t h, int32_t ngroup, const int32_t
   if (group_of_col)
     for (long long c = 0; c < h->ncol; c++)
       if (group_of_col[c] < -1 || group_of_col[c] >= ngroup) return fail(SAMSIM_ERR_ARG, "set_group_stats: group index out of [-1, ngroup)");
-  if (nz < 0 || (nz > 0 && !depth)) return fail(SAMSIM_ERR_ARG, "set_group_stats: bad depth grid");
-  for (int32_t j = 0; j < nz; j++)
-    if (!isfinite(depth[j]) || !(depth[j] > 0.0) || (j > 0 && !(depth[j] > depth[j - 1])))
-      return fail(SAMSIM_ERR_ARG, "set_group_stats: depths must be finite, > 0 and strictly increasing");
-  if (profile_mask >> SAMSIM_SNAPARR_COUNT) return fail(SAMSIM_ERR_ARG, "set_group_stats: unknown snapshot array in profile_mask");
-  if (profile_mask & (1u << SAMSIM_SNAPARR_RAY))
-    return fail(SAMSIM_ERR_ARG, "set_group_stats: ray is an interface quantity (extent Nlayer-1), not a layer profile");
-  for (int a = SAMSIM_SNAPARR_BGC1_BU; a < SAMSIM_SNAPARR_COUNT; a++)
-    if ((profile_mask >> a & 1u) && (a - SAMSIM_SNAPARR_BGC1_BU) / 2 >= h->cfg.N_bgc)
-      return fail(SAMSIM_ERR_ARG, "set_group_stats: tracer rows need N_bgc tracers");
-  if (profile_mask && nz == 0) return fail(SAMSIM_ERR_ARG, "set_group_stats: profiles need a depth grid (nz > 0)");
-  if (h->snap_mode < (profile_mask ? SAMSIM_SNAP_FULL : SAMSIM_SNAP_SCALARS))
-    return fail(SAMSIM_ERR_STATE, "set_group_stats: needs snapshot mode SCALARS, or FULL for profiles");
+  {
+    int rc = check_depth_grid(h, nz, depth, profile_mask, "set_group_stats");
+    if (rc) return rc;
+  }
   int nprof = 0;
   int prof[SAMSIM_SNAPARR_COUNT];
   for (int a = 0; a < SAMSIM_SNAPARR_COUNT; a++)
@@ -1678,6 +1844,109 @@ int samsim_b200_get_group_stats(samsim_handle_t h, double* stats, double* rec_ti
 int samsim_b200_clear_group_stats(samsim_handle_t h) {
   if (!h) return fail(SAMSIM_ERR_ARG, "null handle");
   h->gs_held = 0;
+  return 0;
+}
+
+int samsim_b200_set_time_stats(samsim_handle_t h, int32_t records_per_window, uint32_t scalar_mask, int32_t nz,
+                               const double* depth, uint32_t profile_mask, int32_t max_windows) {
+  if (!h) return fail(SAMSIM_ERR_ARG, "null handle");
+  if (scalar_mask == 0 && profile_mask == 0) {  // off
+    CU(cudaSetDevice(h->device));
+    CU(cudaStreamSynchronize(h->stream));
+    ts_free(h);
+    return 0;
+  }
+  // every argument is checked before the previous setting is dropped
+  if (records_per_window < 0) return fail(SAMSIM_ERR_ARG, "set_time_stats: records_per_window must be >= 0");
+  if (max_windows < 1) return fail(SAMSIM_ERR_ARG, "set_time_stats: max_windows must be >= 1");
+  if (scalar_mask >> SAMSIM_SNAPSC_COUNT) return fail(SAMSIM_ERR_ARG, "set_time_stats: unknown snapshot scalar in scalar_mask");
+  {
+    int rc = check_depth_grid(h, nz, depth, profile_mask, "set_time_stats");
+    if (rc) return rc;
+  }
+  int nsc = 0, nprof = 0;
+  int sc[SAMSIM_SNAPSC_COUNT], prof[SAMSIM_SNAPARR_COUNT];
+  for (int q = 0; q < SAMSIM_SNAPSC_COUNT; q++)
+    if (scalar_mask >> q & 1u) sc[nsc++] = q;
+  for (int a = 0; a < SAMSIM_SNAPARR_COUNT; a++)
+    if (profile_mask >> a & 1u) prof[nprof++] = a;
+  const int Q = nsc + nprof * (profile_mask ? nz : 0);
+
+  CU(cudaSetDevice(h->device));
+  CU(cudaStreamSynchronize(h->stream));
+  ts_free(h);
+  const size_t per = (size_t)Q * SAMSIM_TS_NSTAT * h->ncol_pad;  // doubles of one window
+  cudaError_t e;
+  if ((e = cudaMalloc(&h->ts_z, ((size_t)nz + 1) * sizeof(double))) != cudaSuccess ||
+      (e = cudaMalloc(&h->ts_acc, per * sizeof(double))) != cudaSuccess ||
+      (e = cudaMalloc(&h->ts_hist, (size_t)max_windows * per * sizeof(double))) != cudaSuccess ||
+      (nz && (e = cudaMemcpy(h->ts_z, depth, (size_t)nz * sizeof(double), cudaMemcpyHostToDevice)) != cudaSuccess)) {
+    ts_free(h);
+    cudaGetLastError();
+    return fail(SAMSIM_ERR_CUDA, std::string("set_time_stats: ") + cudaGetErrorString(e));
+  }
+  h->ts_Q = Q; h->ts_nsc = nsc; h->ts_nz = profile_mask ? nz : 0; h->ts_nprof = nprof;
+  h->ts_rpw = records_per_window; h->ts_max = max_windows; h->ts_held = 0; h->ts_cur = 0;
+  for (int q = 0; q < nsc; q++) h->ts_sc[q] = sc[q];
+  for (int a = 0; a < nprof; a++) h->ts_prof[a] = prof[a];
+  h->ts_mask = profile_mask;
+  h->ts_nrec.assign((size_t)max_windows, 0);
+  h->ts_time.assign(2 * ((size_t)max_windows + 1), 0.0);
+  h->ts_i.assign(2 * ((size_t)max_windows + 1), 0);
+  return 0;
+}
+
+int32_t samsim_b200_time_stats_held(samsim_handle_t h) { return h ? h->ts_held : -1; }
+
+int samsim_b200_get_time_stats(samsim_handle_t h, double* stats, int32_t* win_nrec, double* win_time, int64_t* win_i,
+                               int32_t win0, int32_t nwin, int32_t col0, int32_t n) {
+  if (!h) return fail(SAMSIM_ERR_ARG, "null handle");
+  if (win0 < 0 || nwin < 0 || (int64_t)win0 + nwin > h->ts_held)
+    return fail(SAMSIM_ERR_ARG, "get_time_stats: windows win0 .. win0+nwin-1 must be held");
+  if (col0 < 0 || n < 0 || (int64_t)col0 + n > h->ncol) return fail(SAMSIM_ERR_ARG, "get_time_stats: column range out of bounds");
+  if (nwin == 0) return 0;
+  if (win_nrec) std::copy(h->ts_nrec.begin() + win0, h->ts_nrec.begin() + win0 + nwin, win_nrec);
+  if (win_time) std::copy(h->ts_time.begin() + 2 * (size_t)win0, h->ts_time.begin() + 2 * ((size_t)win0 + nwin), win_time);
+  if (win_i) std::copy(h->ts_i.begin() + 2 * (size_t)win0, h->ts_i.begin() + 2 * ((size_t)win0 + nwin), win_i);
+  if (stats && n > 0) {
+    CU(cudaSetDevice(h->device));
+    const size_t per_col = (size_t)h->ts_Q * SAMSIM_TS_NSTAT, per_win = per_col * h->ncol_pad;
+    // staged in pieces of at most 2^25 doubles (256 MB)
+    const int64_t cols = std::max<int64_t>(1, std::min<int64_t>(n, ((int64_t)1 << 25) / (int64_t)per_col));
+    int rc;
+    if ((rc = ensure_stage(h, (size_t)cols * per_col * sizeof(double)))) return rc;
+    for (int32_t w = 0; w < nwin; w++)
+      for (int64_t c0 = 0; c0 < n; c0 += cols) {
+        const int64_t m = std::min<int64_t>(cols, n - c0);
+        const long long total = m * (long long)per_col;
+        samsim_ts_get_kernel<<<(unsigned)((total + 255) / 256), 256, 0, h->stream>>>(
+            h->ts_hist + (size_t)(win0 + w) * per_win, h->stage, h->ncol_pad, h->ts_Q, col0 + c0, m);
+        CU(cudaGetLastError());
+        CU(cudaMemcpyAsync(stats + ((size_t)w * n + c0) * per_col, h->stage, (size_t)total * sizeof(double),
+                           cudaMemcpyDeviceToHost, h->stream));
+        CU(cudaStreamSynchronize(h->stream));
+      }
+  }
+  return 0;
+}
+
+int samsim_b200_close_time_window(samsim_handle_t h) {
+  if (!h) return fail(SAMSIM_ERR_ARG, "null handle");
+  if (h->ts_Q == 0) return fail(SAMSIM_ERR_STATE, "close_time_window: time statistics are off");
+  if (h->ts_cur == 0) return fail(SAMSIM_ERR_STATE, "close_time_window: the window in progress holds no record");
+  if (h->ts_held >= h->ts_max)
+    return fail(SAMSIM_ERR_STATE, "close_time_window: the history is full (samsim_b200_get_time_stats / _clear_time_stats)");
+  CU(cudaSetDevice(h->device));
+  samsim_ts_close_kernel<<<(unsigned)((h->ncol + 255) / 256), 256, 0, h->stream>>>(
+      h->ts_acc, h->ts_hist + (size_t)h->ts_held * h->ts_Q * SAMSIM_TS_NSTAT * h->ncol_pad, h->ts_Q, h->ncol, h->ncol_pad);
+  CU(cudaGetLastError());
+  ts_window_done(h);
+  return 0;
+}
+
+int samsim_b200_clear_time_stats(samsim_handle_t h) {
+  if (!h) return fail(SAMSIM_ERR_ARG, "null handle");
+  h->ts_held = 0;
   return 0;
 }
 

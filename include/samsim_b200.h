@@ -243,6 +243,36 @@ int samsim_b200_update_forcing(samsim_handle_t h, const double* series);
  * ordered with launches like samsim_b200_update_forcing (asynchronous when `series` is pinned host memory).
  * SAMSIM_ERR_STATE before set_forcing; SAMSIM_ERR_ARG for a NULL pointer, n < 1 or records outside 1..nrec. */
 int samsim_b200_update_forcing_records(samsim_handle_t h, int32_t rec0, int32_t n, const double* series);
+/* Stochastic forcing perturbations: per-column AR(1) red noise on the records of the table, generated on the device
+ * from a counter-based generator, so that a column's perturbation is a function of (seed, stream, kind, record) only
+ * and does not depend on launch lengths, re-binning, shards or restarts.  Per kind k (samsim_forcing_kind order):
+ * sigma[k] finite and >= 0 (0 leaves the kind untouched), phi[k] in [0, 1) (AR(1) coefficient per 3-hourly record),
+ * mode[k] 0 additive, 1 multiplicative, 2 lognormal.  stream_of_col[c] in the caller's column order: columns with equal
+ * ids get identical noise, -1 = unperturbed (control members); NULL = stream c.  All sigma 0 switches the feature off
+ * (the default).  A bad argument (NaN, infinite or negative sigma, phi outside [0, 1), an unknown mode, a stream below
+ * -1) is SAMSIM_ERR_ARG and keeps the previous setting; a config without atmoflux_flag 2 is SAMSIM_ERR_CONFIG; a failed
+ * device allocation is SAMSIM_ERR_CUDA and leaves the feature off.  A run input like the table: not saved in
+ * checkpoints.
+ *
+ * Bitwise contract.  For stream s >= 0, kind k and table record r >= 1:
+ *   (x0,x1,x2,x3) = Philox4x32-10(counter = (r, k, s, 0), key = (seed & 0xffffffff, seed >> 32))   (Random123)
+ *   u1 = ((double)(x0 >> 6) * 2^26 + (double)(x1 >> 6) + 0.5) * 2^-52,  u2 likewise from x2, x3
+ *   z(r) = sqrt(-2.0 * det_log(u1)) * det_cos(6.283185307179586 * u2)
+ *   e(1) = sigma * z(1);  e(r) = phi * e(r-1) + c * z(r),  c = sigma * sqrt(1.0 - phi * phi)
+ * each operation rounded on its own; det_log / det_cos / det_exp are those of detmath.h.  The record value
+ * v = base * scale + offset becomes v + e (additive), v * fmax(1.0 + e, 0.0) (multiplicative) or
+ * v * det_exp(e - 0.5 * (sigma * sigma)) (lognormal, mean kept); stream -1 and sigma 0 read v unchanged.  Between
+ * records the step interpolates the perturbed records linearly, as it does the plain ones.
+ *
+ * Device memory while on: SAMSIM_MAXWIN (24) * 4 * ncol_pad doubles for the perturbed records of a launch's window
+ * (805 MB at 1,048,576 columns), 8 * ncol_pad doubles of recursion state and ncol int32 stream ids. */
+int samsim_b200_set_stochastic_forcing(samsim_handle_t h, uint64_t seed, const double sigma[4], const double phi[4],
+                                       const int32_t mode[4], const int32_t* stream_of_col);
+/* The perturbation applied: out[c*nrec + r] = e(rec0 + r) of kind `kind` for the stream of caller column col0 + c
+ * (records rec0 >= 1), 0 for stream -1, for sigma 0 and while the feature is off.  Computed on the device from the
+ * definition, independent of the run. */
+int samsim_b200_get_forcing_noise(samsim_handle_t h, int32_t kind, int32_t rec0, int32_t nrec, int32_t col0, int32_t n,
+                                  double* out);
 /* lab series (mo_grotz.f90:138-169): nset record sets of nrec per-dt values, kinds
  * 0 Tice->T2m, 1 snowfall->solid_precip, 2 heat->fl_q_bottom, 3 styropor; series[(set*4+kind)*nrec + r];
  * set_of_col NULL = set 0.  snow_precip_flag 0 zeroes the snowfall like the reference. */

@@ -166,6 +166,8 @@ def load_library() -> C.CDLL:
         "samsim_b200_set_forcing": (C.c_int, [H, C.c_int32, C.c_int32, dp, ip, dp, dp]),
         "samsim_b200_update_forcing": (C.c_int, [H, dp]),
         "samsim_b200_update_forcing_records": (C.c_int, [H, C.c_int32, C.c_int32, dp]),
+        "samsim_b200_set_stochastic_forcing": (C.c_int, [H, C.c_uint64, dp, dp, ip, ip]),
+        "samsim_b200_get_forcing_noise": (C.c_int, [H, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, dp]),
         "samsim_b200_set_lab_forcing": (C.c_int, [H, C.c_int32, C.c_int64, dp, ip]),
         "samsim_b200_set_lab_lengths": (C.c_int, [H, C.c_int32, C.POINTER(C.c_int64)]),
         "samsim_b200_step": (C.c_int, [H, C.c_int64]),
@@ -216,7 +218,7 @@ EXPORTED_SYMBOLS = [
     "samsim_b200_array_extent", "samsim_b200_set_array", "samsim_b200_get_array", "samsim_b200_set_scalar",
     "samsim_b200_get_scalar", "samsim_b200_set_int", "samsim_b200_get_int", "samsim_b200_broadcast_column",
     "samsim_b200_set_clock", "samsim_b200_get_clock", "samsim_b200_set_forcing", "samsim_b200_update_forcing",
-    "samsim_b200_update_forcing_records",
+    "samsim_b200_update_forcing_records", "samsim_b200_set_stochastic_forcing", "samsim_b200_get_forcing_noise",
     "samsim_b200_set_lab_forcing", "samsim_b200_set_lab_lengths", "samsim_b200_set_end_step",
     "samsim_b200_step", "samsim_b200_synchronize", "samsim_b200_steps_to_next_output",
     "samsim_b200_set_snapshot_mode", "samsim_b200_get_snapshot", "samsim_b200_set_group_stats",
@@ -384,6 +386,28 @@ class Engine:
             s = s[None]
         assert s.ndim == 3 and s.shape[1] == 4
         _check(self.L, self.L.samsim_b200_update_forcing_records(self.h, int(rec0), s.shape[2], _dp(s)))
+
+    def set_stochastic_forcing(self, seed: int, sigma, phi, mode, stream_of_col=None):
+        """Per-column AR(1) red noise on the forcing records, generated on the device (include/samsim_b200.h).
+        sigma, phi, mode: 4 values each in kind order fl_sw, fl_lw, T2m, precip; mode 0 additive, 1 multiplicative,
+        2 lognormal.  stream_of_col[ncol]: columns with equal ids get identical noise, -1 = unperturbed; None = the
+        column index (distributed.noise_streams gives a shard its global ids).  All sigma 0 switches it off."""
+        sg = np.ascontiguousarray(sigma, dtype=np.float64).reshape(4)
+        ph = np.ascontiguousarray(phi, dtype=np.float64).reshape(4)
+        md = np.ascontiguousarray(mode, dtype=np.int32).reshape(4)
+        soc = None if stream_of_col is None else np.ascontiguousarray(stream_of_col, dtype=np.int32)
+        assert soc is None or soc.shape == (self.ncol,)
+        _check(self.L, self.L.samsim_b200_set_stochastic_forcing(self.h, int(seed) & 0xFFFFFFFFFFFFFFFF, _dp(sg), _dp(ph),
+                                                                 _ip(md), _ip(soc)))
+
+    def forcing_noise(self, kind: int, rec0: int, nrec: int, col0: int = 0, n: int | None = None) -> np.ndarray:
+        """e(rec0 .. rec0+nrec-1) of forcing kind `kind` for caller columns col0 .. col0+n-1, shape [n, nrec]: the
+        perturbation applied (0 for stream -1, sigma 0, or with the feature off)"""
+        n = self.ncol - col0 if n is None else n
+        out = np.empty((n, nrec), dtype=np.float64)
+        _check(self.L, self.L.samsim_b200_get_forcing_noise(self.h, int(kind), int(rec0), int(nrec), int(col0), int(n),
+                                                            _dp(out)))
+        return out
 
     def set_lab_forcing(self, series, set_of_col=None, nrec_of_set=None):
         """series[nset, 4, nrec] in kind order Tice, snowfall, heat, styropor.  nrec_of_set[nset]: the real length of

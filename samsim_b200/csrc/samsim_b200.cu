@@ -16,6 +16,7 @@
 
 #include "../../include/samsim_b200.h"
 #include "group_stats.cuh"
+#include "noise.cuh"
 #include "step.cuh"
 #include "time_stats.cuh"
 
@@ -65,6 +66,9 @@ struct KParams {
   const int* site_of_col; // [ncol_pad] or nullptr
   const double* fscale;   // [4][ncol_pad] or nullptr
   const double* foffset;  // [4][ncol_pad] or nullptr
+  // stochastic forcing: the perturbed records win_first .. win_first+win_len-1 of every column, [win_len][4][ncol_pad] in
+  // slot order (samsim_noise_kernel); nullptr = read the table
+  const double* colwin;
   const double* lab;      // [nset][4][lab_nrec]
   long long lab_nrec;
   const int* set_of_col;
@@ -92,7 +96,7 @@ __global__ void __launch_bounds__(SAMSIM_BLOCK, SAMSIM_MINBLOCKS) samsim_step_ke
   __shared__ double s_win[SAMSIM_MAXSITE * 4 * SAMSIM_MAXWIN];
   const bool staged = (p.nsite <= SAMSIM_MAXSITE);
   // stage the forcing window: records win_first .. win_first+win_len-1 of every site/kind (cp.async)
-  if (p.series != nullptr && staged) {
+  if (p.series != nullptr && staged && p.colwin == nullptr) {
     const int n = p.nsite * 4 * p.win_len;
     for (int e = threadIdx.x; e < n; e += blockDim.x) {
       const int sk = e / p.win_len, r = e - sk * p.win_len;
@@ -129,7 +133,9 @@ __global__ void __launch_bounds__(SAMSIM_BLOCK, SAMSIM_MINBLOCKS) samsim_step_ke
   c.fb_x = 0.0;
 
   Forcing f;
-  if (staged) {
+  if (p.colwin) {
+    f.cw = p.colwin + col; f.cw_ld = p.ncol_pad; f.win_first = p.win_first;
+  } else if (staged) {
     f.win = s_win; f.win_len = p.win_len; f.win_first = p.win_first;
   } else {  // the table as samsim_b200_set_forcing stored it
     f.win = p.series; f.win_len = p.nrec; f.win_first = 1; f.global = true;
@@ -608,6 +614,69 @@ __global__ void samsim_ts_get_kernel(const double* win, double* dst, long long n
   dst[t] = win[(size_t)qs * ncol_pad + col0 + cc];
 }
 
+// ---- stochastic forcing (samsim_b200_set_stochastic_forcing; the rules are in noise.cuh) ----------------------------
+struct NzParams {
+  const double* series;       // [nsite][4][nrec]
+  int nrec;
+  const int* site_of_col;     // [ncol_pad] slot order or nullptr
+  const double* fscale;       // [4][ncol_pad] slot order or nullptr
+  const double* foffset;
+  const int* col_of_slot;     // nullptr = identity
+  const int* stream_of_col;   // [ncol] caller order, nullptr = the caller column
+  double* state;              // [4][2][ncol_pad] caller order: e(cursor-1), e(cursor) of every kind
+  double* win;                // [len][4][ncol_pad] slot order: what the step kernel reads (KParams::colwin)
+  long long ncol, ncol_pad;
+  uint64_t seed;
+  NoiseKind nk[4];
+  int cursor, first, len;     // batch-wide cursor; the launch's window of records first .. first+len-1
+};
+
+// One thread per slot, before a step launch: base * scale + offset of every record of the window, perturbed unless the
+// column's stream is -1 or the kind's sigma is 0.  Stream and state are read in caller order, so re-binning moves
+// nothing here.
+__global__ void samsim_noise_kernel(const NzParams p) {
+  const long long s = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= p.ncol) return;
+  const size_t ls = (size_t)p.ncol_pad;
+  const long long c = p.col_of_slot ? (long long)p.col_of_slot[s] : s;
+  const int32_t stream = p.stream_of_col ? p.stream_of_col[c] : (int32_t)c;
+  const int site = p.site_of_col ? p.site_of_col[s] : 0;
+  for (int k = 0; k < 4; k++) {
+    const double scale = p.fscale ? p.fscale[k * ls + s] : 1.0;
+    const double offset = p.foffset ? p.foffset[k * ls + s] : 0.0;
+    const double* base = p.series + ((size_t)site * 4 + k) * p.nrec + (p.first - 1);
+    double* out = p.win + k * ls + s;
+    if (stream < 0 || p.nk[k].sigma == 0.0) {
+      for (int j = 0; j < p.len; j++) out[(size_t)j * 4 * ls] = base[j] * scale + offset;
+      continue;
+    }
+    double* st = p.state + 2 * k * ls + c;
+    double ep = st[0], ec = st[ls];
+    noise_window(p.nk[k], p.seed, k, stream, p.cursor, p.first, p.first + p.len - 1, ep, ec, [&](int32_t r, double e) {
+      const int j = r - p.first;
+      out[(size_t)j * 4 * ls] = noise_apply(p.nk[k], base[j] * scale + offset, e);
+    });
+    st[0] = ep;
+    st[ls] = ec;
+  }
+}
+
+// samsim_b200_get_forcing_noise: dst[t*nrec + r] = e(rec0 + r) of caller column col0 + t, from record 1 (0 for stream
+// -1 and for sigma 0)
+__global__ void samsim_noise_get_kernel(const int* stream_of_col, uint64_t seed, NoiseKind nk, int kind, int rec0, int nrec,
+                                        long long col0, long long n, double* dst) {
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n) return;
+  double* o = dst + (size_t)t * nrec;
+  const int32_t stream = stream_of_col ? stream_of_col[col0 + t] : (int32_t)(col0 + t);
+  if (stream < 0 || nk.sigma == 0.0) {
+    for (int r = 0; r < nrec; r++) o[r] = 0.0;
+    return;
+  }
+  double ep = 0.0, ec = 0.0;
+  noise_window(nk, seed, kind, stream, 0, rec0, rec0 + nrec - 1, ep, ec, [&](int32_t r, double e) { o[r - rec0] = e; });
+}
+
 __global__ void samsim_count_failed_kernel(const int* in, long long ncol, long long ncol_pad, int* out) {
   const long long col = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (col < ncol && in[(size_t)IN_STATUS * ncol_pad + col] != 0) atomicAdd(out, 1);
@@ -752,6 +821,13 @@ struct samsim_b200_handle_s {
   // progress in row max_windows
   std::vector<double> ts_time;
   std::vector<int64_t> ts_i;
+  // stochastic forcing (samsim_b200_set_stochastic_forcing): off while nz_on is false
+  bool nz_on = false;
+  uint64_t nz_seed = 0;
+  NoiseKind nz_kind[4];
+  int nz_cursor = 0;           // batch-wide: nz_state holds e(cursor-1), e(cursor); 0 = nothing held
+  int* nz_stream = nullptr;    // [ncol] caller order, nullptr = the caller column
+  double *nz_state = nullptr, *nz_win = nullptr;  // [4][2][ncol_pad] caller order, [SAMSIM_MAXWIN][4][ncol_pad] slot order
 };
 
 // The step kernel reads its configuration from constant memory (samsim_dev_cfg, physics.cuh), one copy per device.
@@ -942,6 +1018,29 @@ static int ts_record(samsim_handle_t h, double time) {
   return 0;
 }
 
+static void nz_free(samsim_handle_t h) {
+  cudaFree(h->nz_stream); cudaFree(h->nz_state); cudaFree(h->nz_win);
+  h->nz_stream = nullptr;
+  h->nz_state = h->nz_win = nullptr;
+  h->nz_on = false;
+  h->nz_cursor = 0;
+}
+
+// Queue the window kernel of a launch reading records first .. first+len-1 (no host synchronisation) and move the cursor
+static int nz_window(samsim_handle_t h, int first, int len) {
+  NzParams p;
+  memset(&p, 0, sizeof p);
+  p.series = h->series; p.nrec = h->nrec; p.site_of_col = h->site_of_col; p.fscale = h->fscale; p.foffset = h->foffset;
+  p.col_of_slot = h->col_of_slot; p.stream_of_col = h->nz_stream; p.state = h->nz_state; p.win = h->nz_win;
+  p.ncol = h->ncol; p.ncol_pad = h->ncol_pad; p.seed = h->nz_seed;
+  for (int k = 0; k < 4; k++) p.nk[k] = h->nz_kind[k];
+  p.cursor = h->nz_cursor; p.first = first; p.len = len;
+  samsim_noise_kernel<<<(unsigned)((h->ncol + 255) / 256), 256, 0, h->stream>>>(p);
+  CU(cudaGetLastError());
+  h->nz_cursor = noise_cursor_after(h->nz_cursor, first, first + len - 1);
+  return 0;
+}
+
 extern "C" {
 
 const char* samsim_b200_last_error(void) { return g_err.c_str(); }
@@ -1036,6 +1135,7 @@ void samsim_b200_destroy(samsim_handle_t h) {
   cudaFree(h->snap_arr); cudaFree(h->stage); cudaFree(h->slot_of_col); cudaFree(h->col_of_slot); cudaFree(h->end_of_col);
   gs_free(h);
   ts_free(h);
+  nz_free(h);
   if (h->ev0) cudaEventDestroy(h->ev0);
   if (h->ev1) cudaEventDestroy(h->ev1);
   if (h->stream) cudaStreamDestroy(h->stream);
@@ -1220,6 +1320,73 @@ int samsim_b200_update_forcing_records(samsim_handle_t h, int32_t rec0, int32_t 
   return 0;
 }
 
+int samsim_b200_set_stochastic_forcing(samsim_handle_t h, uint64_t seed, const double sigma[4], const double phi[4],
+                                       const int32_t mode[4], const int32_t* stream_of_col) {
+  if (!h || !sigma || !phi || !mode) return fail(SAMSIM_ERR_ARG, "set_stochastic_forcing: bad argument");
+  if (h->cfg.atmoflux_flag != 2) return fail(SAMSIM_ERR_CONFIG, "set_stochastic_forcing: needs atmoflux_flag 2");
+  bool on = false;
+  for (int k = 0; k < 4; k++) {
+    if (!(sigma[k] >= 0.0 && std::isfinite(sigma[k])))
+      return fail(SAMSIM_ERR_ARG, "set_stochastic_forcing: sigma must be finite and >= 0");
+    if (!(phi[k] >= 0.0 && phi[k] < 1.0)) return fail(SAMSIM_ERR_ARG, "set_stochastic_forcing: phi must lie in [0, 1)");
+    if (mode[k] < SAMSIM_NOISE_ADDITIVE || mode[k] > SAMSIM_NOISE_LOGNORMAL)
+      return fail(SAMSIM_ERR_ARG, "set_stochastic_forcing: mode must be 0 (additive), 1 (multiplicative) or 2 (lognormal)");
+    on = on || sigma[k] > 0.0;
+  }
+  if (stream_of_col)
+    for (long long c = 0; c < h->ncol; c++)
+      if (stream_of_col[c] < -1) return fail(SAMSIM_ERR_ARG, "set_stochastic_forcing: stream ids must be >= -1");
+  CU(cudaSetDevice(h->device));
+  CU(cudaStreamSynchronize(h->stream));  // a launch in flight may still read the window
+  if (!on) {
+    nz_free(h);
+    return 0;
+  }
+  h->nz_on = false;
+  cudaError_t e = cudaSuccess;
+  if (!h->nz_win) e = cudaMalloc(&h->nz_win, (size_t)SAMSIM_MAXWIN * 4 * h->ncol_pad * sizeof(double));
+  if (e == cudaSuccess && !h->nz_state) e = cudaMalloc(&h->nz_state, (size_t)8 * h->ncol_pad * sizeof(double));
+  if (e == cudaSuccess && stream_of_col) {
+    if (!h->nz_stream) e = cudaMalloc(&h->nz_stream, (size_t)h->ncol * sizeof(int));
+    if (e == cudaSuccess) e = cudaMemcpy(h->nz_stream, stream_of_col, (size_t)h->ncol * sizeof(int), cudaMemcpyHostToDevice);
+  } else if (e == cudaSuccess) {
+    cudaFree(h->nz_stream);
+    h->nz_stream = nullptr;
+  }
+  if (e != cudaSuccess) {
+    nz_free(h);
+    cudaGetLastError();  // an allocation failure is not sticky; keep it from surfacing at the next launch check
+    return fail(SAMSIM_ERR_CUDA, std::string("set_stochastic_forcing: ") + cudaGetErrorString(e));
+  }
+  h->nz_seed = seed;
+  for (int k = 0; k < 4; k++) h->nz_kind[k] = noise_kind(sigma[k], phi[k], mode[k]);
+  h->nz_cursor = 0;  // the next window restarts from record 1
+  h->nz_on = true;
+  return 0;
+}
+
+int samsim_b200_get_forcing_noise(samsim_handle_t h, int32_t kind, int32_t rec0, int32_t nrec, int32_t col0, int32_t n,
+                                  double* out) {
+  int rc = check_cols(h, col0, n);
+  if (rc) return rc;
+  if (!out || kind < 0 || kind >= SAMSIM_F_COUNT || rec0 < 1 || nrec < 0 || (int64_t)rec0 + nrec - 1 > INT32_MAX)
+    return fail(SAMSIM_ERR_ARG, "get_forcing_noise: bad argument");
+  if (n == 0 || nrec == 0) return 0;
+  const size_t bytes = (size_t)n * nrec * sizeof(double);
+  if (!h->nz_on) {
+    memset(out, 0, bytes);
+    return 0;
+  }
+  CU(cudaSetDevice(h->device));
+  if ((rc = ensure_stage(h, bytes))) return rc;
+  samsim_noise_get_kernel<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>(h->nz_stream, h->nz_seed, h->nz_kind[kind], kind,
+                                                                              rec0, nrec, col0, n, h->stage);
+  CU(cudaGetLastError());
+  CU(cudaMemcpyAsync(out, h->stage, bytes, cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  return 0;
+}
+
 // latest end step of the columns of each lab set: only the sets of running columns bound a launch (samsim_b200_step)
 static void update_lab_end(samsim_handle_t h) {
   h->lab_end.assign(h->lab_len.size(), INT64_MIN);
@@ -1401,6 +1568,11 @@ int samsim_b200_step(samsim_handle_t h, int64_t nsteps) {
       if (p.win_len < 1) p.win_len = 1;
       if (p.win_first + p.win_len - 1 > h->nrec) p.win_len = h->nrec - p.win_first + 1;
       p.site_of_col = h->site_of_col; p.fscale = h->fscale; p.foffset = h->foffset;
+      if (h->nz_on) {
+        int rc = nz_window(h, p.win_first, p.win_len);
+        if (rc) return rc;
+        p.colwin = h->nz_win;
+      }
     }
     if (need_lab) {
       // Records FLOOR(1 + time/dt) of every step a column runs in the chunk must exist in its set.  The device

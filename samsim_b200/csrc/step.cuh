@@ -21,14 +21,20 @@ struct Forcing {
   long long lab_nrec;
   int lab_set;
   bool global = false;    // win is the device table in global memory: read-only loads, 64-bit index
+  // stochastic forcing (samsim_b200_set_stochastic_forcing): this column's perturbed record values of the launch's
+  // window, cw[((rec - win_first)*4 + kind)*cw_ld], written by samsim_noise_kernel; nullptr = read the table
+  const double* cw = nullptr;
+  long long cw_ld;
 };
 
 __device__ __forceinline__ double forcing_rec(const Forcing& f, int kind, int rec /*1-based*/) {
 #ifdef __CUDA_ARCH__
+  if (f.cw) return __ldg(f.cw + ((long long)(rec - f.win_first) * 4 + kind) * f.cw_ld);
   // (site*4 + kind)*nrec passes 2^31 at about 183,000 sites of a year of 3-hourly records
   const double base = f.global ? __ldg(f.win + (((long long)f.site * 4 + kind) * f.win_len + (rec - f.win_first)))
                                : f.win[(f.site * 4 + kind) * f.win_len + (rec - f.win_first)];
 #else
+  if (f.cw) return f.cw[((long long)(rec - f.win_first) * 4 + kind) * f.cw_ld];
   const double base = f.win[((long long)f.site * 4 + kind) * f.win_len + (rec - f.win_first)];
 #endif
   return base * f.scale[kind] + f.offset[kind];

@@ -30,6 +30,13 @@ def local_sites(site_of_col, col0: int, n: int) -> tuple[np.ndarray, np.ndarray]
     return sites, local.astype(np.int32).reshape(-1)
 
 
+def noise_streams(total: int, rank: int, world: int) -> np.ndarray:
+    """Stochastic-forcing stream ids of the block of `rank` (Engine.set_stochastic_forcing): the global column indices
+    col0 + arange(n) of shard(), so that a sharded ensemble draws the same noise as one handle holding every column."""
+    col0, n = shard(total, rank, world)
+    return np.arange(col0, col0 + n, dtype=np.int32)
+
+
 def reduce_ensemble(local: dict, ncol_local: int, group=None, device=None) -> dict:
     """local = Engine.reduce_diag() of this rank; returns the ensemble-wide mean/min/max per diagnostic."""
     import torch

@@ -273,6 +273,30 @@ int samsim_b200_set_stochastic_forcing(samsim_handle_t h, uint64_t seed, const d
  * definition, independent of the run. */
 int samsim_b200_get_forcing_noise(samsim_handle_t h, int32_t kind, int32_t rec0, int32_t nrec, int32_t col0, int32_t n,
                                   double* out);
+/* Correlated stochastic forcing: the four kinds drawn together and spatially coherent noise from shared basis streams.
+ * A generalisation of samsim_b200_set_stochastic_forcing, which it replaces (and which replaces it): one setting, one
+ * state.  sigma, phi, mode as there.  corr[16] (row-major, NULL = the identity) correlates the kinds' innovations: finite,
+ * exactly symmetric, unit diagonal, positive definite.  Column c mixes nmix (1..8) basis streams:
+ * basis_of_col[c*nmix + m] ids >= 0, distinct within the column, or -1 for an empty entry;
+ * weight_of_col[c*nmix + m] finite weights (NULL = 1.0).  A column whose entries are all empty is unperturbed.
+ *
+ * Bitwise contract.  For basis stream b and record r, z_k(r; b) is z(r) of the single-stream contract with s = b, for
+ * all four kinds.  w_k = z_k when corr is NULL or the identity, else w_k = ((L[k][0]*z_0 + L[k][1]*z_1) + ...) +
+ * L[k][k]*z_k, L the Cholesky factor of corr by Cholesky-Banachiewicz in double (s = corr[i][j]; s = s - L[i][m]*L[j][m]
+ * for m = 0..j-1; L[i][i] = sqrt(s), L[i][j] = s / L[j][j]).  E_k(1) = sigma_k * w_k(1), E_k(r) = phi_k * E_k(r-1) +
+ * c_k * w_k(r).  Over a column's non-empty entries in m order, e = w * E(b) of the first, then e = e + w * E(b); the
+ * modes read e, with h * q for the lognormal one, q = w*w of the first entry, then q = q + w*w.  So the lognormal mean is
+ * kept, and nmix 1, weight 1.0 and the identity give the bits of samsim_b200_set_stochastic_forcing.  The lag-0
+ * correlation of kinds i, j is corr[i][j] * sqrt((1-phi_i^2)(1-phi_j^2)) / (1 - phi_i*phi_j); two columns with unit-norm
+ * weights correlate by the sum of w_a*w_b over their shared ids.  samsim_b200_get_forcing_noise returns the column's e.
+ *
+ * Errors as samsim_b200_set_stochastic_forcing; SAMSIM_ERR_ARG also for nmix outside 1..8, an id below -1, a repeated
+ * id within a column, a non-finite weight, a bad corr or basis_of_col NULL.  Device memory while on: the window of
+ * SAMSIM_MAXWIN * 4 * ncol_pad doubles, and, unless the setting is the single-stream case, SAMSIM_MAXWIN * 4 * nbasis +
+ * 8 * nbasis doubles and 12 * nmix bytes per column (nbasis = the distinct ids) in place of the per-column state. */
+int samsim_b200_set_stochastic_forcing_correlated(samsim_handle_t h, uint64_t seed, const double sigma[4],
+                                                  const double phi[4], const int32_t mode[4], const double corr[16],
+                                                  int32_t nmix, const int32_t* basis_of_col, const double* weight_of_col);
 /* lab series (mo_grotz.f90:138-169): nset record sets of nrec per-dt values, kinds
  * 0 Tice->T2m, 1 snowfall->solid_precip, 2 heat->fl_q_bottom, 3 styropor; series[(set*4+kind)*nrec + r];
  * set_of_col NULL = set 0.  snow_precip_flag 0 zeroes the snowfall like the reference. */

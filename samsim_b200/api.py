@@ -168,6 +168,7 @@ def load_library() -> C.CDLL:
         "samsim_b200_update_forcing_records": (C.c_int, [H, C.c_int32, C.c_int32, dp]),
         "samsim_b200_set_stochastic_forcing": (C.c_int, [H, C.c_uint64, dp, dp, ip, ip]),
         "samsim_b200_get_forcing_noise": (C.c_int, [H, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, dp]),
+        "samsim_b200_set_stochastic_forcing_correlated": (C.c_int, [H, C.c_uint64, dp, dp, ip, dp, C.c_int32, ip, dp]),
         "samsim_b200_set_lab_forcing": (C.c_int, [H, C.c_int32, C.c_int64, dp, ip]),
         "samsim_b200_set_lab_lengths": (C.c_int, [H, C.c_int32, C.POINTER(C.c_int64)]),
         "samsim_b200_step": (C.c_int, [H, C.c_int64]),
@@ -219,6 +220,7 @@ EXPORTED_SYMBOLS = [
     "samsim_b200_get_scalar", "samsim_b200_set_int", "samsim_b200_get_int", "samsim_b200_broadcast_column",
     "samsim_b200_set_clock", "samsim_b200_get_clock", "samsim_b200_set_forcing", "samsim_b200_update_forcing",
     "samsim_b200_update_forcing_records", "samsim_b200_set_stochastic_forcing", "samsim_b200_get_forcing_noise",
+    "samsim_b200_set_stochastic_forcing_correlated",
     "samsim_b200_set_lab_forcing", "samsim_b200_set_lab_lengths", "samsim_b200_set_end_step",
     "samsim_b200_step", "samsim_b200_synchronize", "samsim_b200_steps_to_next_output",
     "samsim_b200_set_snapshot_mode", "samsim_b200_get_snapshot", "samsim_b200_set_group_stats",
@@ -387,18 +389,35 @@ class Engine:
         assert s.ndim == 3 and s.shape[1] == 4
         _check(self.L, self.L.samsim_b200_update_forcing_records(self.h, int(rec0), s.shape[2], _dp(s)))
 
-    def set_stochastic_forcing(self, seed: int, sigma, phi, mode, stream_of_col=None):
+    def set_stochastic_forcing(self, seed: int, sigma, phi, mode, stream_of_col=None, *, corr=None, basis=None,
+                               weights=None):
         """Per-column AR(1) red noise on the forcing records, generated on the device (include/samsim_b200.h).
         sigma, phi, mode: 4 values each in kind order fl_sw, fl_lw, T2m, precip; mode 0 additive, 1 multiplicative,
         2 lognormal.  stream_of_col[ncol]: columns with equal ids get identical noise, -1 = unperturbed; None = the
-        column index (distributed.noise_streams gives a shard its global ids).  All sigma 0 switches it off."""
+        column index (distributed.noise_streams gives a shard its global ids).  All sigma 0 switches it off.
+
+        Correlated noise (samsim_b200_set_stochastic_forcing_correlated, DESIGN 7.4): corr[4, 4] correlates the kinds'
+        innovations (None = the identity); basis[ncol, nmix] gives each column up to 8 basis streams (-1 = empty entry,
+        ids distinct within a column) and weights[ncol, nmix] their weights (None = 1.0); bilinear_noise_basis builds
+        both for a grid.  basis replaces stream_of_col; without it a column mixes its stream_of_col (or its index)."""
         sg = np.ascontiguousarray(sigma, dtype=np.float64).reshape(4)
         ph = np.ascontiguousarray(phi, dtype=np.float64).reshape(4)
         md = np.ascontiguousarray(mode, dtype=np.int32).reshape(4)
-        soc = None if stream_of_col is None else np.ascontiguousarray(stream_of_col, dtype=np.int32)
-        assert soc is None or soc.shape == (self.ncol,)
-        _check(self.L, self.L.samsim_b200_set_stochastic_forcing(self.h, int(seed) & 0xFFFFFFFFFFFFFFFF, _dp(sg), _dp(ph),
-                                                                 _ip(md), _ip(soc)))
+        seed = int(seed) & 0xFFFFFFFFFFFFFFFF
+        if corr is None and basis is None and weights is None:
+            soc = None if stream_of_col is None else np.ascontiguousarray(stream_of_col, dtype=np.int32)
+            assert soc is None or soc.shape == (self.ncol,)
+            _check(self.L, self.L.samsim_b200_set_stochastic_forcing(self.h, seed, _dp(sg), _dp(ph), _ip(md), _ip(soc)))
+            return
+        if basis is not None and stream_of_col is not None:
+            raise ValueError("set_stochastic_forcing: pass basis or stream_of_col, not both")
+        if basis is None:
+            basis = np.arange(self.ncol) if stream_of_col is None else stream_of_col
+        b = np.ascontiguousarray(basis, dtype=np.int32).reshape(self.ncol, -1)
+        w = None if weights is None else np.ascontiguousarray(weights, dtype=np.float64).reshape(b.shape)
+        cr = None if corr is None else np.ascontiguousarray(corr, dtype=np.float64).reshape(16)
+        _check(self.L, self.L.samsim_b200_set_stochastic_forcing_correlated(
+            self.h, seed, _dp(sg), _dp(ph), _ip(md), _dp(cr), b.shape[1], _ip(b), _dp(w)))
 
     def forcing_noise(self, kind: int, rec0: int, nrec: int, col0: int = 0, n: int | None = None) -> np.ndarray:
         """e(rec0 .. rec0+nrec-1) of forcing kind `kind` for caller columns col0 .. col0+n-1, shape [n, nrec]: the
@@ -610,6 +629,29 @@ class Engine:
         v = C.c_float()
         _check(self.L, self.L.samsim_b200_last_step_ms(self.h, C.byref(v)))
         return v.value
+
+
+def bilinear_noise_basis(ny: int, nx: int, spacing: int) -> tuple[np.ndarray, np.ndarray]:
+    """Spatially coherent stochastic forcing on a row-major ny x nx grid with one column per cell
+    (Engine.set_stochastic_forcing(basis=, weights=)).  The basis streams sit on a coarse lattice every `spacing` cells,
+    (ny - 1) // spacing + 2 rows of (nx - 1) // spacing + 2 nodes, id = row * nodes_per_row + node.  Cell (y, x) mixes
+    the four nodes around it with bilinear weights divided by sqrt(sum w^2), so every cell has unit variance and the
+    noise varies smoothly over about `spacing` cells.  Returns basis[ny*nx, 4] (int32) and weights[ny*nx, 4].  The ids
+    are global lattice indices: a shard holding cells col0 .. col0+n-1 passes basis[col0:col0+n] and weights[col0:col0+n]
+    and draws the same noise as one handle holding the grid."""
+    ny, nx, sp = int(ny), int(nx), int(spacing)
+    if ny < 1 or nx < 1 or sp < 1:
+        raise ValueError("bilinear_noise_basis: ny, nx and spacing must be >= 1")
+    nxl = (nx - 1) // sp + 2
+    if ((ny - 1) // sp + 2) * nxl > 2 ** 31 - 1:
+        raise ValueError("bilinear_noise_basis: the lattice has more nodes than int32 ids")
+    y, x = np.divmod(np.arange(ny * nx, dtype=np.int64), nx)
+    iy, ix = y // sp, x // sp
+    ty, tx = (y - iy * sp) / sp, (x - ix * sp) / sp
+    node = iy * nxl + ix
+    basis = np.stack([node, node + 1, node + nxl, node + nxl + 1], axis=1).astype(np.int32)
+    w = np.stack([(1 - ty) * (1 - tx), (1 - ty) * tx, ty * (1 - tx), ty * tx], axis=1)
+    return basis, w / np.sqrt((w * w).sum(axis=1))[:, None]
 
 
 # ---- unit KAT entry points ---------------------------------------------------------------------

@@ -20,6 +20,19 @@
 //   mode 2, lognormal:       v * det_exp(e - h),  h = 0.5 * (sigma * sigma)   (the mean of v is kept)
 // A kind with sigma 0 and a column with stream -1 read v unchanged.  The noise is keyed on the table record, not on
 // the step or the launch, so it does not depend on launch lengths, re-binning, shards or restarts.
+//
+// Correlated noise (samsim_b200_set_stochastic_forcing_correlated, DESIGN §7.4) generalises this.  A column mixes up to
+// SAMSIM_NOISE_MAXMIX basis streams, and the kinds' innovations are correlated through a 4x4 matrix corr.  For basis
+// stream b >= 0 and record r, z_k(r; b) is z(r) above with s = b, drawn for all four kinds whatever their sigma, and
+//   w_k = z_k                                                   corr NULL or the identity: no arithmetic
+//   w_k = ((L[k][0]*z_0 + L[k][1]*z_1) + ...) + L[k][k]*z_k     otherwise, left to right
+// with L the Cholesky factor of corr (noise_cholesky, in double, at set time).  E_k(1) = sigma_k * w_k(1) and
+// E_k(r) = phi_k * E_k(r-1) + c_k * w_k(r).  Column c holds entries m = 0..nmix-1, a basis id (-1 = empty) and a
+// finite weight; over its non-empty entries in m order
+//   e = w * E(b) of the first, then e = e + w * E(b)        (from the first term, not from 0.0: -0.0 is kept)
+//   q = w * w of the first, then q = q + w * w
+// and the modes read e, with h * q in place of h for the lognormal one.  A column with no entry reads v unchanged.
+// One entry of weight 1.0 with corr the identity gives the bits of the single-stream contract above.
 #pragma once
 
 #include <math.h>
@@ -30,6 +43,7 @@
 #define SAMSIM_NOISE_ADDITIVE 0
 #define SAMSIM_NOISE_MULTIPLICATIVE 1
 #define SAMSIM_NOISE_LOGNORMAL 2
+#define SAMSIM_NOISE_MAXMIX 8
 
 namespace samsim {
 
@@ -119,6 +133,140 @@ __host__ __device__ inline void noise_window(const NoiseKind& nk, uint64_t seed,
     }
     emit(r, (r == at) ? ec : ep);
   }
+}
+
+// ---- correlated noise --------------------------------------------------------------------------------------------
+
+// The Cholesky factor of the kinds' correlation: on == 0 for the identity (w = z, no arithmetic), else L row-major
+struct NoiseCorr {
+  double L[16];
+  int on;
+};
+
+// Cholesky-Banachiewicz of the symmetric 4x4 corr (row-major) into L, zero above the diagonal, each operation rounded
+// on its own.  False when a pivot is not > 0 (corr not positive definite, or not finite).
+__host__ __device__ inline bool noise_cholesky(const double corr[16], double L[16]) {
+  for (int q = 0; q < 16; q++) L[q] = 0.0;
+  for (int i = 0; i < 4; i++)
+    for (int j = 0; j <= i; j++) {
+      double s = corr[i * 4 + j];
+      for (int m = 0; m < j; m++) s = s - L[i * 4 + m] * L[j * 4 + m];
+      if (i == j) {
+        if (!(s > 0.0)) return false;
+        L[i * 4 + i] = sqrt(s);
+      } else {
+        L[i * 4 + j] = s / L[j * 4 + j];
+      }
+    }
+  return true;
+}
+
+// the four kinds' innovations w of basis stream b at record rec
+__host__ __device__ inline void noise_innovations(const NoiseCorr& nc, uint64_t seed, int32_t b, int32_t rec, double w[4]) {
+  double z[4];
+#pragma unroll
+  for (int k = 0; k < 4; k++) z[k] = noise_normal(seed, k, b, rec);
+#pragma unroll
+  for (int k = 0; k < 4; k++) {
+    if (!nc.on) {
+      w[k] = z[k];
+      continue;
+    }
+    double s = nc.L[k * 4] * z[0];
+#pragma unroll
+    for (int j = 1; j <= k; j++) s = s + nc.L[k * 4 + j] * z[j];
+    w[k] = s;
+  }
+}
+
+// noise_window for the four kinds of basis stream b at once: E_k(r) for r = first..last passed to emit(r, E) in record
+// order; ep[k], ec[k] hold E_k(cursor-1), E_k(cursor) on entry and on return, under the same cursor rule
+template <class Emit>
+__host__ __device__ inline void noise_basis_window(const NoiseKind* nk, const NoiseCorr& nc, uint64_t seed, int32_t b,
+                                                   int32_t cursor, int32_t first, int32_t last, double ep[4],
+                                                   double ec[4], Emit emit) {
+  int32_t at = cursor;  // ep = E(at-1), ec = E(at)
+  if (!noise_resumes(cursor, first)) {
+    at = 0;
+#pragma unroll
+    for (int k = 0; k < 4; k++) ep[k] = ec[k] = 0.0;
+  }
+  for (int32_t r = first; r <= last; r++) {
+    while (at < r) {
+      at++;
+      double w[4];
+      noise_innovations(nc, seed, b, at, w);
+#pragma unroll
+      for (int k = 0; k < 4; k++) {
+        ep[k] = ec[k];
+        ec[k] = noise_next(nk[k], ec[k], w[k], at);
+      }
+    }
+    double E[4];
+#pragma unroll
+    for (int k = 0; k < 4; k++) E[k] = (r == at) ? ec[k] : ep[k];
+    emit(r, E);
+  }
+}
+
+// One term of a column's mix, in m order over its non-empty entries: acc = w * x for the first (any false on entry),
+// acc = acc + w * x after.  x = E(b) gives e, x = w gives q.
+__host__ __device__ inline void noise_accumulate(double& acc, bool& any, double w, double x) {
+  const double t = w * x;
+  acc = any ? acc + t : t;
+  any = true;
+}
+
+// the record value v perturbed by the column's mixed e, q its sum of squared weights (lognormal: h * q in place of h)
+__host__ __device__ inline double noise_apply_mixed(const NoiseKind& nk, double v, double e, double q) {
+  if (nk.mode == SAMSIM_NOISE_LOGNORMAL) return v * det_exp(e - nk.h * q);
+  return noise_apply(nk, v, e);
+}
+
+// The argument rules of both setters, on the host: nullptr for a valid setting, else what is wrong.  basis[c*nmix + m]
+// (nullptr = stream c, nmix 1), weight likewise (nullptr = 1.0), corr row-major (nullptr = the identity).  On success
+// `on` tells whether a sigma is > 0, `single` whether the setting is the single-stream case (nmix 1, every weight 1.0,
+// corr the identity) and nc holds the Cholesky factor (nc.on = 0 for the identity).
+inline const char* noise_check(const double sigma[4], const double phi[4], const int32_t mode[4], const double* corr,
+                               int32_t nmix, int64_t ncol, const int32_t* basis, const double* weight, bool& on,
+                               bool& single, NoiseCorr& nc) {
+  on = false;
+  for (int k = 0; k < 4; k++) {
+    if (!(sigma[k] >= 0.0 && isfinite(sigma[k]))) return "sigma must be finite and >= 0";
+    if (!(phi[k] >= 0.0 && phi[k] < 1.0)) return "phi must lie in [0, 1)";
+    if (mode[k] < SAMSIM_NOISE_ADDITIVE || mode[k] > SAMSIM_NOISE_LOGNORMAL)
+      return "mode must be 0 (additive), 1 (multiplicative) or 2 (lognormal)";
+    on = on || sigma[k] > 0.0;
+  }
+  if (nmix < 1 || nmix > SAMSIM_NOISE_MAXMIX) return "nmix must lie in 1..8";
+  if (basis)
+    for (int64_t c = 0; c < ncol; c++)
+      for (int m = 0; m < nmix; m++) {
+        const int32_t b = basis[c * nmix + m];
+        if (b < -1) return "stream ids must be >= -1";
+        for (int m2 = 0; m2 < m && b >= 0; m2++)
+          if (basis[c * nmix + m2] == b) return "basis ids must be distinct within a column";
+      }
+  bool unit = true;
+  if (weight)
+    for (int64_t q = 0; q < ncol * nmix; q++) {
+      if (!isfinite(weight[q])) return "weights must be finite";
+      unit = unit && weight[q] == 1.0;
+    }
+  for (int q = 0; q < 16; q++) nc.L[q] = 0.0;
+  nc.on = 0;
+  if (corr) {
+    for (int i = 0; i < 4; i++)
+      for (int j = 0; j < 4; j++) {
+        const double x = corr[i * 4 + j];
+        if (!isfinite(x) || x != corr[j * 4 + i] || (i == j && x != 1.0))
+          return "corr must be finite, exactly symmetric and have a unit diagonal";
+        nc.on = nc.on || (i != j && x != 0.0);
+      }
+    if (!noise_cholesky(corr, nc.L)) return "corr must be positive definite";
+  }
+  single = nmix == 1 && unit && !nc.on;
+  return nullptr;
 }
 
 }  // namespace samsim

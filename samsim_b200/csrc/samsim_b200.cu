@@ -629,6 +629,15 @@ struct NzParams {
   uint64_t seed;
   NoiseKind nk[4];
   int cursor, first, len;     // batch-wide cursor; the launch's window of records first .. first+len-1
+  // correlated noise (samsim_b200_set_stochastic_forcing_correlated): basis streams mixed per column
+  NoiseCorr corr;
+  int nmix;
+  long long nbasis;
+  const int* basis_id;        // [nbasis] the distinct basis ids, ascending
+  const int* bidx;            // [nmix][ncol] caller order: index into basis_id, -1 = empty entry
+  const double* bweight;      // [nmix][ncol] caller order
+  double* bstate;             // [4][2][nbasis]: E(cursor-1), E(cursor) of every basis stream and kind
+  double* bwin;               // [len][4][nbasis]: E of the window's records (samsim_noise_basis_kernel)
 };
 
 // One thread per slot, before a step launch: base * scale + offset of every record of the window, perturbed unless the
@@ -675,6 +684,104 @@ __global__ void samsim_noise_get_kernel(const int* stream_of_col, uint64_t seed,
   }
   double ep = 0.0, ec = 0.0;
   noise_window(nk, seed, kind, stream, 0, rec0, rec0 + nrec - 1, ep, ec, [&](int32_t r, double e) { o[r - rec0] = e; });
+}
+
+// Correlated noise, first of the two kernels before a step launch: one thread per distinct basis stream draws the four
+// kinds' innovations of the window's records, mixes them through L and advances the four AR(1) states under the
+// batch-wide cursor.  Writes E[len][4][nbasis].
+__global__ void samsim_noise_basis_kernel(const NzParams p) {
+  const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= p.nbasis) return;
+  const size_t lb = (size_t)p.nbasis;
+  double ep[4], ec[4];
+#pragma unroll
+  for (int k = 0; k < 4; k++) {
+    ep[k] = p.bstate[2 * k * lb + j];
+    ec[k] = p.bstate[(2 * k + 1) * lb + j];
+  }
+  noise_basis_window(p.nk, p.corr, p.seed, p.basis_id[j], p.cursor, p.first, p.first + p.len - 1, ep, ec,
+                     [&](int32_t r, const double* E) {
+                       double* o = p.bwin + (size_t)(r - p.first) * 4 * lb + j;
+#pragma unroll
+                       for (int k = 0; k < 4; k++) o[k * lb] = E[k];
+                     });
+#pragma unroll
+  for (int k = 0; k < 4; k++) {
+    p.bstate[2 * k * lb + j] = ep[k];
+    p.bstate[(2 * k + 1) * lb + j] = ec[k];
+  }
+}
+
+// Second kernel: one thread per slot gathers its column's basis values per record and kind, mixes them and writes the
+// perturbed records in the layout samsim_noise_kernel writes (KParams::colwin).  Columns with no entry and kinds with
+// sigma 0 get base * scale + offset.
+__global__ void samsim_noise_mix_kernel(const NzParams p) {
+  const long long s = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= p.ncol) return;
+  const size_t ls = (size_t)p.ncol_pad, lb = (size_t)p.nbasis;
+  const long long c = p.col_of_slot ? (long long)p.col_of_slot[s] : s;
+  int32_t bi[SAMSIM_NOISE_MAXMIX];
+  double bw[SAMSIM_NOISE_MAXMIX];
+  double q = 0.0;
+  bool any = false;
+#pragma unroll
+  for (int m = 0; m < SAMSIM_NOISE_MAXMIX; m++) {
+    bi[m] = -1;
+    bw[m] = 0.0;
+    if (m < p.nmix) {
+      bi[m] = p.bidx[(size_t)m * p.ncol + c];
+      bw[m] = p.bweight[(size_t)m * p.ncol + c];
+      if (bi[m] >= 0) noise_accumulate(q, any, bw[m], bw[m]);
+    }
+  }
+  const int site = p.site_of_col ? p.site_of_col[s] : 0;
+  for (int k = 0; k < 4; k++) {
+    const double scale = p.fscale ? p.fscale[k * ls + s] : 1.0;
+    const double offset = p.foffset ? p.foffset[k * ls + s] : 0.0;
+    const double* base = p.series + ((size_t)site * 4 + k) * p.nrec + (p.first - 1);
+    double* out = p.win + k * ls + s;
+    if (!any || p.nk[k].sigma == 0.0) {
+      for (int j = 0; j < p.len; j++) out[(size_t)j * 4 * ls] = base[j] * scale + offset;
+      continue;
+    }
+    for (int j = 0; j < p.len; j++) {
+      const double* E = p.bwin + ((size_t)j * 4 + k) * lb;
+      double e = 0.0;
+      bool got = false;
+#pragma unroll
+      for (int m = 0; m < SAMSIM_NOISE_MAXMIX; m++)
+        if (bi[m] >= 0) noise_accumulate(e, got, bw[m], E[bi[m]]);
+      out[(size_t)j * 4 * ls] = noise_apply_mixed(p.nk[k], base[j] * scale + offset, e, q);
+    }
+  }
+}
+
+// samsim_b200_get_forcing_noise with basis streams: dst[t*nrec + r] = the mixed e(rec0 + r) of caller column col0 + t,
+// every basis stream from record 1 (0 for a column with no entry and for sigma 0)
+__global__ void samsim_noise_get_mixed_kernel(const NzParams p, int kind, int rec0, int nrec, long long col0, long long n,
+                                              double* dst) {
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n) return;
+  double* o = dst + (size_t)t * nrec;
+  bool any = false;
+  for (int m = 0; m < p.nmix && p.nk[kind].sigma != 0.0; m++) {
+    const int32_t b = p.bidx[(size_t)m * p.ncol + col0 + t];
+    if (b < 0) continue;
+    const double w = p.bweight[(size_t)m * p.ncol + col0 + t];
+    double ep[4], ec[4];
+    noise_basis_window(p.nk, p.corr, p.seed, p.basis_id[b], 0, rec0, rec0 + nrec - 1, ep, ec,
+                       [&](int32_t r, const double* E) {
+                         double x = E[0];
+#pragma unroll
+                         for (int k = 1; k < 4; k++)
+                           if (kind == k) x = E[k];
+                         bool got = any;
+                         noise_accumulate(o[r - rec0], got, w, x);
+                       });
+    any = true;
+  }
+  if (!any)
+    for (int r = 0; r < nrec; r++) o[r] = 0.0;
 }
 
 __global__ void samsim_count_failed_kernel(const int* in, long long ncol, long long ncol_pad, int* out) {
@@ -828,6 +935,13 @@ struct samsim_b200_handle_s {
   int nz_cursor = 0;           // batch-wide: nz_state holds e(cursor-1), e(cursor); 0 = nothing held
   int* nz_stream = nullptr;    // [ncol] caller order, nullptr = the caller column
   double *nz_state = nullptr, *nz_win = nullptr;  // [4][2][ncol_pad] caller order, [SAMSIM_MAXWIN][4][ncol_pad] slot order
+  // basis streams mixed per column (samsim_b200_set_stochastic_forcing_correlated): nz_nmix 0 = the per-column path
+  // above (nz_stream, nz_state); otherwise NzParams' basis fields, and nz_state is not held
+  int nz_nmix = 0;
+  long long nz_nbasis = 0;
+  NoiseCorr nz_corr;
+  int *nz_basis_id = nullptr, *nz_bidx = nullptr;       // [nbasis], [nmix][ncol]
+  double *nz_bweight = nullptr, *nz_bstate = nullptr, *nz_bwin = nullptr;  // [nmix][ncol], [4][2][nbasis], [MAXWIN][4][nbasis]
 };
 
 // The step kernel reads its configuration from constant memory (samsim_dev_cfg, physics.cuh), one copy per device.
@@ -1018,24 +1132,51 @@ static int ts_record(samsim_handle_t h, double time) {
   return 0;
 }
 
+// the basis-stream buffers of the correlated path
+static void nz_free_basis(samsim_handle_t h) {
+  cudaFree(h->nz_basis_id); cudaFree(h->nz_bidx); cudaFree(h->nz_bweight); cudaFree(h->nz_bstate); cudaFree(h->nz_bwin);
+  h->nz_basis_id = h->nz_bidx = nullptr;
+  h->nz_bweight = h->nz_bstate = h->nz_bwin = nullptr;
+  h->nz_nmix = 0;
+  h->nz_nbasis = 0;
+}
+
 static void nz_free(samsim_handle_t h) {
   cudaFree(h->nz_stream); cudaFree(h->nz_state); cudaFree(h->nz_win);
   h->nz_stream = nullptr;
   h->nz_state = h->nz_win = nullptr;
+  nz_free_basis(h);
   h->nz_on = false;
   h->nz_cursor = 0;
 }
 
-// Queue the window kernel of a launch reading records first .. first+len-1 (no host synchronisation) and move the cursor
-static int nz_window(samsim_handle_t h, int first, int len) {
+static NzParams nz_params(samsim_handle_t h) {
   NzParams p;
   memset(&p, 0, sizeof p);
   p.series = h->series; p.nrec = h->nrec; p.site_of_col = h->site_of_col; p.fscale = h->fscale; p.foffset = h->foffset;
   p.col_of_slot = h->col_of_slot; p.stream_of_col = h->nz_stream; p.state = h->nz_state; p.win = h->nz_win;
   p.ncol = h->ncol; p.ncol_pad = h->ncol_pad; p.seed = h->nz_seed;
   for (int k = 0; k < 4; k++) p.nk[k] = h->nz_kind[k];
-  p.cursor = h->nz_cursor; p.first = first; p.len = len;
-  samsim_noise_kernel<<<(unsigned)((h->ncol + 255) / 256), 256, 0, h->stream>>>(p);
+  p.cursor = h->nz_cursor;
+  p.corr = h->nz_corr; p.nmix = h->nz_nmix; p.nbasis = h->nz_nbasis; p.basis_id = h->nz_basis_id; p.bidx = h->nz_bidx;
+  p.bweight = h->nz_bweight; p.bstate = h->nz_bstate; p.bwin = h->nz_bwin;
+  return p;
+}
+
+// Queue the window kernels of a launch reading records first .. first+len-1 (no host synchronisation) and move the
+// cursor
+static int nz_window(samsim_handle_t h, int first, int len) {
+  NzParams p = nz_params(h);
+  p.first = first; p.len = len;
+  if (h->nz_nmix == 0) {
+    samsim_noise_kernel<<<(unsigned)((h->ncol + 255) / 256), 256, 0, h->stream>>>(p);
+  } else {
+    if (h->nz_nbasis > 0) {  // none when every column's entries are empty
+      samsim_noise_basis_kernel<<<(unsigned)((h->nz_nbasis + 255) / 256), 256, 0, h->stream>>>(p);
+      CU(cudaGetLastError());
+    }
+    samsim_noise_mix_kernel<<<(unsigned)((h->ncol + 255) / 256), 256, 0, h->stream>>>(p);
+  }
   CU(cudaGetLastError());
   h->nz_cursor = noise_cursor_after(h->nz_cursor, first, first + len - 1);
   return 0;
@@ -1320,22 +1461,33 @@ int samsim_b200_update_forcing_records(samsim_handle_t h, int32_t rec0, int32_t 
   return 0;
 }
 
-int samsim_b200_set_stochastic_forcing(samsim_handle_t h, uint64_t seed, const double sigma[4], const double phi[4],
-                                       const int32_t mode[4], const int32_t* stream_of_col) {
-  if (!h || !sigma || !phi || !mode) return fail(SAMSIM_ERR_ARG, "set_stochastic_forcing: bad argument");
-  if (h->cfg.atmoflux_flag != 2) return fail(SAMSIM_ERR_CONFIG, "set_stochastic_forcing: needs atmoflux_flag 2");
-  bool on = false;
-  for (int k = 0; k < 4; k++) {
-    if (!(sigma[k] >= 0.0 && std::isfinite(sigma[k])))
-      return fail(SAMSIM_ERR_ARG, "set_stochastic_forcing: sigma must be finite and >= 0");
-    if (!(phi[k] >= 0.0 && phi[k] < 1.0)) return fail(SAMSIM_ERR_ARG, "set_stochastic_forcing: phi must lie in [0, 1)");
-    if (mode[k] < SAMSIM_NOISE_ADDITIVE || mode[k] > SAMSIM_NOISE_LOGNORMAL)
-      return fail(SAMSIM_ERR_ARG, "set_stochastic_forcing: mode must be 0 (additive), 1 (multiplicative) or 2 (lognormal)");
-    on = on || sigma[k] > 0.0;
-  }
-  if (stream_of_col)
+// Both stochastic forcing setters.  basis NULL (only from samsim_b200_set_stochastic_forcing) means stream c for column c.
+// The single-stream case (nmix 1, weights 1.0, corr the identity) keeps the per-column path of samsim_noise_kernel.
+static int nz_set(samsim_handle_t h, const char* who, uint64_t seed, const double sigma[4], const double phi[4],
+                  const int32_t mode[4], const double corr[16], int32_t nmix, const int32_t* basis, const double* weight) {
+  const std::string w = std::string(who) + ": ";
+  if (!h || !sigma || !phi || !mode) return fail(SAMSIM_ERR_ARG, w + "bad argument");
+  if (h->cfg.atmoflux_flag != 2) return fail(SAMSIM_ERR_CONFIG, w + "needs atmoflux_flag 2");
+  bool on, single;
+  NoiseCorr nc;
+  if (const char* bad = noise_check(sigma, phi, mode, corr, nmix, h->ncol, basis, weight, on, single, nc))
+    return fail(SAMSIM_ERR_ARG, w + bad);
+  const size_t nent = (size_t)h->ncol * nmix;
+  // the distinct basis ids, ascending, and every entry's index among them
+  std::vector<int32_t> ids, idx;
+  if (on && !single) {
+    ids.reserve(nent);
+    for (size_t q = 0; q < nent; q++)
+      if (basis[q] >= 0) ids.push_back(basis[q]);
+    std::sort(ids.begin(), ids.end());
+    ids.erase(std::unique(ids.begin(), ids.end()), ids.end());
+    idx.resize(nent);  // [nmix][ncol]
     for (long long c = 0; c < h->ncol; c++)
-      if (stream_of_col[c] < -1) return fail(SAMSIM_ERR_ARG, "set_stochastic_forcing: stream ids must be >= -1");
+      for (int m = 0; m < nmix; m++) {
+        const int32_t b = basis[(size_t)c * nmix + m];
+        idx[(size_t)m * h->ncol + c] = b < 0 ? -1 : (int32_t)(std::lower_bound(ids.begin(), ids.end(), b) - ids.begin());
+      }
+  }
   CU(cudaSetDevice(h->device));
   CU(cudaStreamSynchronize(h->stream));  // a launch in flight may still read the window
   if (!on) {
@@ -1343,26 +1495,61 @@ int samsim_b200_set_stochastic_forcing(samsim_handle_t h, uint64_t seed, const d
     return 0;
   }
   h->nz_on = false;
+  nz_free_basis(h);
   cudaError_t e = cudaSuccess;
   if (!h->nz_win) e = cudaMalloc(&h->nz_win, (size_t)SAMSIM_MAXWIN * 4 * h->ncol_pad * sizeof(double));
-  if (e == cudaSuccess && !h->nz_state) e = cudaMalloc(&h->nz_state, (size_t)8 * h->ncol_pad * sizeof(double));
-  if (e == cudaSuccess && stream_of_col) {
-    if (!h->nz_stream) e = cudaMalloc(&h->nz_stream, (size_t)h->ncol * sizeof(int));
-    if (e == cudaSuccess) e = cudaMemcpy(h->nz_stream, stream_of_col, (size_t)h->ncol * sizeof(int), cudaMemcpyHostToDevice);
-  } else if (e == cudaSuccess) {
-    cudaFree(h->nz_stream);
+  if (single) {
+    if (e == cudaSuccess && !h->nz_state) e = cudaMalloc(&h->nz_state, (size_t)8 * h->ncol_pad * sizeof(double));
+    if (e == cudaSuccess && basis) {
+      if (!h->nz_stream) e = cudaMalloc(&h->nz_stream, (size_t)h->ncol * sizeof(int));
+      if (e == cudaSuccess) e = cudaMemcpy(h->nz_stream, basis, (size_t)h->ncol * sizeof(int), cudaMemcpyHostToDevice);
+    } else if (e == cudaSuccess) {
+      cudaFree(h->nz_stream);
+      h->nz_stream = nullptr;
+    }
+  } else {
+    cudaFree(h->nz_state); cudaFree(h->nz_stream);
+    h->nz_state = nullptr;
     h->nz_stream = nullptr;
+    const size_t nb = ids.size();
+    std::vector<double> wt(nent, 1.0);  // [nmix][ncol]
+    if (weight)
+      for (long long c = 0; c < h->ncol; c++)
+        for (int m = 0; m < nmix; m++) wt[(size_t)m * h->ncol + c] = weight[(size_t)c * nmix + m];
+    if (e == cudaSuccess) e = cudaMalloc(&h->nz_bidx, nent * sizeof(int));
+    if (e == cudaSuccess) e = cudaMalloc(&h->nz_bweight, nent * sizeof(double));
+    if (e == cudaSuccess && nb) e = cudaMalloc(&h->nz_basis_id, nb * sizeof(int));
+    if (e == cudaSuccess && nb) e = cudaMalloc(&h->nz_bstate, 8 * nb * sizeof(double));
+    if (e == cudaSuccess && nb) e = cudaMalloc(&h->nz_bwin, (size_t)SAMSIM_MAXWIN * 4 * nb * sizeof(double));
+    if (e == cudaSuccess) e = cudaMemcpy(h->nz_bidx, idx.data(), nent * sizeof(int), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) e = cudaMemcpy(h->nz_bweight, wt.data(), nent * sizeof(double), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess && nb) e = cudaMemcpy(h->nz_basis_id, ids.data(), nb * sizeof(int), cudaMemcpyHostToDevice);
+    h->nz_nmix = nmix;
+    h->nz_nbasis = (long long)nb;
+    h->nz_corr = nc;
   }
   if (e != cudaSuccess) {
     nz_free(h);
     cudaGetLastError();  // an allocation failure is not sticky; keep it from surfacing at the next launch check
-    return fail(SAMSIM_ERR_CUDA, std::string("set_stochastic_forcing: ") + cudaGetErrorString(e));
+    return fail(SAMSIM_ERR_CUDA, w + cudaGetErrorString(e));
   }
   h->nz_seed = seed;
   for (int k = 0; k < 4; k++) h->nz_kind[k] = noise_kind(sigma[k], phi[k], mode[k]);
   h->nz_cursor = 0;  // the next window restarts from record 1
   h->nz_on = true;
   return 0;
+}
+
+int samsim_b200_set_stochastic_forcing(samsim_handle_t h, uint64_t seed, const double sigma[4], const double phi[4],
+                                       const int32_t mode[4], const int32_t* stream_of_col) {
+  return nz_set(h, "set_stochastic_forcing", seed, sigma, phi, mode, nullptr, 1, stream_of_col, nullptr);
+}
+
+int samsim_b200_set_stochastic_forcing_correlated(samsim_handle_t h, uint64_t seed, const double sigma[4],
+                                                  const double phi[4], const int32_t mode[4], const double corr[16],
+                                                  int32_t nmix, const int32_t* basis_of_col, const double* weight_of_col) {
+  if (!basis_of_col) return fail(SAMSIM_ERR_ARG, "set_stochastic_forcing_correlated: bad argument");
+  return nz_set(h, "set_stochastic_forcing_correlated", seed, sigma, phi, mode, corr, nmix, basis_of_col, weight_of_col);
 }
 
 int samsim_b200_get_forcing_noise(samsim_handle_t h, int32_t kind, int32_t rec0, int32_t nrec, int32_t col0, int32_t n,
@@ -1379,8 +1566,12 @@ int samsim_b200_get_forcing_noise(samsim_handle_t h, int32_t kind, int32_t rec0,
   }
   CU(cudaSetDevice(h->device));
   if ((rc = ensure_stage(h, bytes))) return rc;
-  samsim_noise_get_kernel<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>(h->nz_stream, h->nz_seed, h->nz_kind[kind], kind,
-                                                                              rec0, nrec, col0, n, h->stage);
+  if (h->nz_nmix == 0)
+    samsim_noise_get_kernel<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>(h->nz_stream, h->nz_seed, h->nz_kind[kind],
+                                                                                kind, rec0, nrec, col0, n, h->stage);
+  else
+    samsim_noise_get_mixed_kernel<<<(unsigned)((n + 127) / 128), 128, 0, h->stream>>>(nz_params(h), kind, rec0, nrec, col0,
+                                                                                      n, h->stage);
   CU(cudaGetLastError());
   CU(cudaMemcpyAsync(out, h->stage, bytes, cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));

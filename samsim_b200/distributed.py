@@ -32,7 +32,9 @@ def local_sites(site_of_col, col0: int, n: int) -> tuple[np.ndarray, np.ndarray]
 
 def noise_streams(total: int, rank: int, world: int) -> np.ndarray:
     """Stochastic-forcing stream ids of the block of `rank` (Engine.set_stochastic_forcing): the global column indices
-    col0 + arange(n) of shard(), so that a sharded ensemble draws the same noise as one handle holding every column."""
+    col0 + arange(n) of shard(), so that a sharded ensemble draws the same noise as one handle holding every column.
+    Spatially coherent noise on a grid works the same way: api.bilinear_noise_basis gives global lattice ids, and a
+    shard passes basis[col0:col0 + n] and weights[col0:col0 + n] of the whole grid's arrays."""
     col0, n = shard(total, rank, world)
     return np.arange(col0, col0 + n, dtype=np.int32)
 

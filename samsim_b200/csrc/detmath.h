@@ -196,6 +196,50 @@ DM_API double det_pow(double x, double y) {
   return dm_exp2part(ph, pl);
 }
 
+// ---- inverse permeability, from below ----------------------------------------
+// A lower bound of 1 / perm with perm = 1e-17 * det_pow(1000*|psi_l|, 3.10) (mo_grav_drain.f90:104-106), for the
+// gravity-drainage bound that rules out layers without evaluating det_pow (physics.cuh, grav_drain).  No division:
+// log2 of the mantissa by a degree-8 polynomial in m-1 on [sqrt(1/2), sqrt(2)), 2^f by a degree-6 polynomial on
+// [-1/2, 1/2] (Chebyshev fits; together < 1e-7 relative, measured by tests/test_perm_bound_cpu.py), then the result
+// is lowered by DM_PERM_SLACK.  Where 1/perm is a normal double the result r satisfies
+//     (1 - 2*DM_PERM_SLACK) / perm  <=  r  <  (1 - DM_PERM_SLACK/2) / perm .
+// Ends: psi_l = 0 gives +inf (= 1/0); 1000|psi_l| < 2^-256 gives 2^790 (1/perm > 2^849 there); 1000|psi_l| > 2^256
+// gives 0; NaN and +-inf give NaN, which the caller treats like any non-finite bound (the layer is evaluated exactly).
+#define DM_PERM_SLACK 1.52587890625e-05  /* 2^-16 */
+DM_HD double dm_perm_inv_lo(double psi_l) {
+  const double x = 1000.0 * fabs(psi_l);
+  if (!(x <= 1.157920892373162e+77)) return (x != x || x > 1.7976931348623157e+308) ? dm_from_bits(0x7ff8000000000000LL) : 0.0;
+  if (x < 8.636168555094445e-78) return (x == 0.0) ? dm_from_bits(0x7ff0000000000000LL) : dm_pow2i(790);  // 2^-256
+  const int64_t b = dm_bits(x);
+  int e = (int)(b >> 52) - 1023;
+  double m = dm_from_bits((b & 0x000fffffffffffffLL) | 0x3ff0000000000000LL);  // [1, 2)
+  if (m > 1.4142135623730951) {
+    m = m * 0.5;
+    e += 1;
+  }
+  const double u = m - 1.0;                 // exact
+  double p = 0.12453901975427666;           // log2(1+u)/u
+  p = fma(p, u, -0.2048054494423592);
+  p = fma(p, u, 0.21508739257218026);
+  p = fma(p, u, -0.23924569897150472);
+  p = fma(p, u, 0.28800520316499323);
+  p = fma(p, u, -0.3606933098145126);
+  p = fma(p, u, 0.4809079378408423);
+  p = fma(p, u, -0.7213474398355846);
+  p = fma(p, u, 1.4426950148397704);
+  const double t = -3.10 * ((double)e + u * p);  // log2(1/x^3.10), |t| < 800
+  const double n = rint(t);
+  const double f = t - n;                   // exact, |f| <= 1/2
+  double q = 0.00015465312336038613;        // 2^f
+  q = fma(q, f, 0.001339527980035732);
+  q = fma(q, f, 0.00961803994572486);
+  q = fma(q, f, 0.05550340680745591);
+  q = fma(q, f, 0.24022651101313985);
+  q = fma(q, f, 0.6931472000626802);
+  q = fma(q, f, 0.9999999999718431);
+  return 1e17 * ((q * (1.0 - DM_PERM_SLACK)) * dm_pow2i((int)n));
+}
+
 // ---- sin / cos ------------------------------------------------------------
 #define DM_PIO2_1 1.57079632673412561417e+00 /* first 33 bits of pi/2 */
 #define DM_PIO2_2 6.07710050630396597660e-11 /* second 33 bits */

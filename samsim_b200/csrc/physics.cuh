@@ -889,9 +889,38 @@ __device__ __forceinline__ double fl_Q_0_snow(double m_snow, double thick_snow, 
 // relative deviation <= ~1e-14) and classifies every layer with them; the reference's forward sums are evaluated
 // only for layers whose estimate is above ray_crit*(1 - 1e-10) -- a margin four orders wider than the deviation --
 // so decisions and fluxes are the reference's, bit for bit, and layers that cannot drain cost O(1).
+// With harmonic_flag 2 and no tracers, a cheaper bound pass first rules out the layers above the topmost layer
+// whose estimate can come near ray_crit (in mid-winter the warm bottom fifth): they need no det_pow and no
+// division, and keep ray from an earlier step, which nothing reads before an exact_all step rewrites it.
 #ifndef SAMSIM_GB
 #define SAMSIM_GB 8   // layers per block of the blocked forward sums: 16 accumulators in registers
 #endif
+// Bound pass of grav_drain (harmonic_flag 2): the estimate with thick/perm from below (dm_perm_inv_lo) and no
+// division, est > thr tested as P*(st + bottom_h) > thr*(kappa_l*mu)*(sq + qb).  Every layer whose estimate exceeds
+// ray_crit*(1 - 1e-10) is flagged, and so is any comparison with a NaN (DESIGN §5.1).  Nothing is stored.  Returns
+// the first layer of the block of the blocked sums (SAMSIM_GB) that holds the topmost flagged layer, or Na when no
+// layer is flagged.  Out of line: its registers stay out of grav_drain's allocation.
+__device__ __noinline__ int grav_drain_bound(const Col& c, double bottom_h, double S_br_Na) {
+  const View v = c;
+  const int Na = c.N_active;
+  const double thr = (ray_crit * (1.0 - 1e-6)) * (kappa_l * mu);
+  double sq = 0.0, st = 0.0, qb = 0.0;
+  int ktop = 0;  // topmost flagged layer
+  SAMSIM_LOOP
+  for (int k = Na; k >= 1; k--) {
+    if (k - SAMSIM_PF >= 1) { v.psi_l().prefetch(k - SAMSIM_PF); v.thick().prefetch(k - SAMSIM_PF); v.S_br().prefetch(k - SAMSIM_PF); }
+    const double ip = dm_perm_inv_lo(v.psi_l()[k]);
+    if (k == Na) { qb = bottom_h * ip; continue; }
+    const double thk = v.thick()[k];
+    const double st_below = st;
+    sq = sq + thk * ip;
+    st = st + thk;
+    const double a = grav * rho_l * bbeta * (v.S_br()[k] - S_br_Na) * (st_below + bottom_h) * (st + bottom_h);
+    if (!(a <= thr * (sq + qb))) ktop = k;
+  }
+  return ktop ? ((ktop - 1) / SAMSIM_GB) * SAMSIM_GB + 1 : Na;
+}
+
 __device__ __noinline__ void grav_drain(Col& c, bool exact_all) {
   const View v = c;
   const int Na = c.N_active, N = CFG.Nlayer;
@@ -903,14 +932,16 @@ __device__ __noinline__ void grav_drain(Col& c, bool exact_all) {
   for (int k = Na; k <= N - 1; k++) v.ray()[k] = 0.0;  // :98 ray = 0 (entries below N_active are overwritten next)
   const double bottom_h = v.thick()[Na] * v.psi_s()[Na] / psi_s_min;  // thick(N_active)*psi_s(N_active)/psi_s_min
   const double S_br_Na = v.S_br()[Na];
+  // Layers K0..Na are evaluated below; layers 1..K0-1 are proven unable to drain by the bound pass (lean steps only)
+  const int K0 = (!exact_all && CFG.harmonic_flag == 2 && CFG.n_bgc == 0) ? grav_drain_bound(c, bottom_h, S_br_Na) : 1;
   // :104-106 permeability, thick/perm, and the order-independent suffix minimum of perm(k:Na-1), one backward pass
   double perm_Na = 0.0;
   int kmin_cand = 0, ncand = 0;  // candidates: layers whose estimate can exceed ray_crit
   {
     double mn = 0.0, sq = 0.0, st = 0.0, st_below = 0.0, qb_est = 0.0;  // suffix sums for the estimate
     SAMSIM_LOOP
-    for (int k = Na; k >= 1; k--) {
-      if (k - SAMSIM_PF >= 1) { v.psi_l().prefetch(k - SAMSIM_PF); v.thick().prefetch(k - SAMSIM_PF); v.S_br().prefetch(k - SAMSIM_PF); }
+    for (int k = Na; k >= K0; k--) {
+      if (k - SAMSIM_PF >= K0) { v.psi_l().prefetch(k - SAMSIM_PF); v.thick().prefetch(k - SAMSIM_PF); v.S_br().prefetch(k - SAMSIM_PF); }
       const double pk = 1e-17 * det_pow(1000.0 * fabs(v.psi_l()[k]), 3.10);
       if (k == Na) { perm_Na = pk; qb_est = bottom_h / pk; continue; }  // perm itself is not needed again
       const double thk = v.thick()[k];
@@ -1021,10 +1052,21 @@ __device__ __noinline__ void grav_drain(Col& c, bool exact_all) {
   double min_S = 1e300;  // minimum over the S_abs values this routine leaves behind (:198)
   int kfirst = 0;        // first draining layer: fl_m(1:kfirst) == 0
 
-  double run = 0.0;  // running sum = fl_up(kk) for every kk not yet clamped
-  double sbk = v.S_br()[1];
+  // Layers 1..K0-1 cannot drain (and kfirst == 0 there): each leaves S_abs as it is, so both sums take the same
+  // additions from 0.0 and get the same bits
   SAMSIM_LOOP
-  for (int k = 1; k <= Na - 1; k++) {  // :144-171
+  for (int k = 1; k <= K0 - 1; k++) {
+    if (k + SAMSIM_PF <= K0 - 1) v.S_abs().prefetch(k + SAMSIM_PF);
+    const double Sk = v.S_abs()[k];
+    sum_before = sum_before + Sk;
+    min_S = f_min(min_S, Sk);
+  }
+  sum_after = sum_before;
+
+  double run = 0.0;  // running sum = fl_up(kk) for every kk not yet clamped
+  double sbk = v.S_br()[K0];
+  SAMSIM_LOOP
+  for (int k = K0; k <= Na - 1; k++) {  // :144-171
     if (k + SAMSIM_PF <= Na) {
       // psi_s and m are only read for layers above ray_crit: prefetching them for every layer was 16 B of DRAM
       // traffic per layer and step for nothing
